@@ -5,6 +5,7 @@
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
         --master-port P bench.py --gpus N --steps K --warmup W
     python bench.py --impl reference ...      # CPU arm: the oracle port on the host cores
+    python bench.py ... --dump-outputs DIR    # also write what the last timed step computed as DIR/<name>.npy
 
 A step = forward + MSE+L1 loss + BPTT + gradient all-reduce + Adam (train.py:96-110) on one batch of
 synthetic N(0,1) data of the named shape.  Prints ONE JSON line (rank 0):
@@ -30,6 +31,7 @@ import threading
 import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
+sys.dont_write_bytecode = True                             # the benchmark leaves the source tree as it found it
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 
@@ -146,6 +148,22 @@ def run_reference(args):
 
 
 # ---------------------------------------------------------------------------------------------------------------------
+def dump_outputs(out_dir, model, loss):
+    """What Trainer.step, the timed path, hands its caller after the last timed step: the loss it returns, the
+    parameters it updated in place and the gradients it wrote into their .grad (all fp32, 0.8 MB each for parameters and
+    gradients at hidden 64, k3).  Inputs and initial weights come from fixed seeds, so two builds can be compared array
+    by array."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"loss": loss}
+    for name, p in model.named_parameters():
+        arrays["param." + name] = p
+        arrays["grad." + name] = p.grad
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().float().cpu().numpy())
+    return sorted(arrays)
+
+
 def cuda_timed(fn, n, dev):
     """ms per call of fn over n calls (CUDA events on the current stream, synchronised on both sides)"""
     torch.cuda.synchronize(dev)
@@ -185,6 +203,7 @@ def gpu_eager_baseline(B, T, k, dev, steps=3):
     opt = torch.optim.Adam(net.parameters(), lr=1e-3, betas=(0.5, 0.999), fused=True)
     x, y = torch.randn(B, T, C_IN, H, W, device=dev), torch.randn(B, H, W, device=dev)
     torch.backends.cudnn.benchmark = True
+    torch.backends.cudnn.deterministic = False             # cuDNN's fastest algorithms: the library kernels to beat
 
     def step():
         opt.zero_grad(set_to_none=True)
@@ -278,7 +297,11 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the sustained run, eager baseline, e2e variants and configs block")
     ap.add_argument("--sustained-seconds", type=float, default=2.0)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the loss, parameters and gradients of the last timed step as DIR/<name>.npy (rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -307,6 +330,10 @@ def main():
         B, global_batch, scaling = args.batch, args.batch * world, "weak"
 
     torch.manual_seed(0)                                   # identical init on every rank (utils.py:77-88)
+    # the reference trains under seed() (train.py:32 -> utils.py:87: cudnn.deterministic), which selects the fixed-order
+    # gradient reductions here: every run of the same arguments computes the same bits (--dump-outputs), instead of
+    # fp32-atomic sums whose order differences Adam carries from step to step
+    torch.backends.cudnn.deterministic = True
     model = ConvLSTM(C_IN, [HIDDEN], [k], 1, precision=args.precision).to(dev)
     trainer = Trainer(model, lr=1e-3, betas=(0.5, 0.999))
     torch.manual_seed(1 + rank)
@@ -350,6 +377,9 @@ def main():
     clocks = sampler.stop() if rank == 0 else None
     ms_step = max_over_ranks(e0.elapsed_time(e1)) / K_
     value = global_batch / (ms_step * 1e-3)
+    dumped = None
+    if args.dump_outputs and rank == 0:                    # before the runs below train the same model further
+        dumped = {"dir": os.path.abspath(args.dump_outputs), "arrays": dump_outputs(args.dump_outputs, model, loss)}
 
     # ---------------- the same over >= 2 s: the power cap bites after ~1 s, short runs read 3-8 % high
     sustained = None
@@ -507,7 +537,7 @@ def main():
             "config": {"workload": f"ConvLSTM train step (fwd+MSE/L1+BPTT+allreduce+Adam), 90x144 grid, 20 levels + BCB "
                                    f"= 21 ch, hidden 64, k{k}, T={T}, batch {B}/GPU (global {global_batch})",
                        "parallelism": f"dp{world}", "l2_policy": "inputs (418 MB/step at B=32) larger than the 126 MB L2",
-                       "loss_at_end": round(float(loss), 5), "numa_node": numa,
+                       "loss_at_end": round(float(loss), 5), "numa_node": numa, "deterministic": True,
                        "sub_batch": int(os.environ.get("NINT_SUB_BATCH", "0") or 0),
                        "pdl": int(os.environ.get("NINT_PDL", "0") or 0),
                        "time_fused_launches": os.environ.get("NINT_FUSE_STEPS", "auto (BPTT launches fused when short)")},
@@ -519,6 +549,7 @@ def main():
             "clocks": clocks,
             "roofline": roof,
             "kernels": kernels,
+            "dumped_outputs": dumped,
             "gate_conv_fwd_bwd": {"tflops": round(total_tf, 1), "frac": round(total_tf / peak_sus, 4),
                                   "frac_burst": round(total_tf / peak_burst, 4), "peak_sustained": peak_sus,
                                   "peak_burst": peak_burst, "target": "60 % of bf16 dense peak (BASELINE.md: <= 5.13 ms of conv time at cfg 2)",

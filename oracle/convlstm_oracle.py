@@ -7,8 +7,8 @@ reference`` legs of ``bench.py``; the product package never imports it and has
 no CPU fallback.
 
 Parity status: PINNED.  ``oracle/make_golden.py`` imports the unmodified
-reference ``/root/reference/model.py`` in the build container, runs it on seeded
-inputs and writes ``tests/golden/*.npz``; ``tests/test_oracle.py`` checks every
+reference ``model.py`` from an upstream checkout, runs it on seeded inputs and
+writes ``tests/golden/*.npz`` (``oracle/golden.py``); ``tests/test_oracle.py`` checks every
 function here against those vectors and against the structural known answers
 the reference's notebooks print (param counts ``test.ipynb:4698-4699``, padding
 print ``dataset_config.ipynb:484-496``).  The arithmetic itself lives in a

@@ -1,16 +1,18 @@
 """Generate tests/golden/*.npz by running the UNMODIFIED reference.
 
-Run in the build container only (needs /root/reference):
+Needs a checkout of the upstream repository (smhassanerfani/nasa-niswan):
 
-    PYTHONDONTWRITEBYTECODE=1 python oracle/make_golden.py
+    PYTHONDONTWRITEBYTECODE=1 python oracle/make_golden.py <path of the upstream checkout>
 
-* ConvLSTM vectors: imports ``/root/reference/model.py`` as-is, seeds torch,
+* ConvLSTM vectors: imports the upstream ``model.py`` as-is, seeds torch,
   runs forward + ``MSELoss+L1Loss`` + backward (train.py:96-109) on CPU fp32
-  and stores inputs, state_dict, prediction, loss and every parameter gradient.
+  and stores prediction, loss and every parameter gradient; the inputs
+  (x, y, state_dict, cell-step inputs) are stored as their seed and digest
+  (oracle/golden.py).
 * Padding vectors: ``dataset.py`` cannot be imported here (xarray missing), so
   the two padding classes (dataset.py:13-98) are pulled out of the source with
   ``ast`` and executed against numpy only, exactly as written upstream.
-The files are small and committed; nothing on the GPU box reads /root/reference.
+The files are small and committed; the tests never read the upstream checkout.
 """
 import ast
 import os
@@ -19,7 +21,10 @@ import sys
 import numpy as np
 import torch
 
-REF = "/root/reference"
+sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), ".."))
+from oracle import golden  # noqa: E402
+
+REF = None                # the upstream checkout, from the command line
 OUT = os.path.join(os.path.dirname(os.path.abspath(__file__)), "..", "tests", "golden")
 
 
@@ -76,7 +81,7 @@ def convlstm_case(name, B, T, cin, hidden, ks, H, W, seed, crop=None, with_seque
         h1, c1 = cell(xs, (h0, c0))
     out.update({"cell/x": xs.numpy(), "cell/h0": h0.numpy(), "cell/c0": c0.numpy(),
                 "cell/h1": h1.numpy(), "cell/c1": c1.numpy()})
-    np.savez(os.path.join(OUT, name + ".npz"), **out)
+    golden.save_case(os.path.join(OUT, name + ".npz"), out, seed)
     print(name, "loss", float(loss), "pred", tuple(pred.shape))
 
 
@@ -105,6 +110,10 @@ def padding_case():
 
 
 def main():
+    global REF
+    if len(sys.argv) != 2:
+        raise SystemExit(__doc__)
+    REF = os.path.abspath(sys.argv[1])
     os.makedirs(OUT, exist_ok=True)
     torch.set_num_threads(1)  # bit-reproducible reductions
     # single layer, BASELINE channel geometry (20 levels + emission), small grid; GPU-tile friendly

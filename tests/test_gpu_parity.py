@@ -9,6 +9,7 @@ import torch
 import torch.nn.functional as F
 
 from oracle import convlstm_oracle as O
+from oracle.golden import load_case
 
 pytestmark = pytest.mark.gpu
 
@@ -25,7 +26,7 @@ def _need_gpu():
 
 
 def _load(golden_dir, name):
-    z = np.load(os.path.join(golden_dir, name + ".npz"))
+    z = load_case(golden_dir, name)
     meta = z["meta"].tolist()
     B, T, cin, H, W, L = meta[:6]
     hidden, ks = meta[6:6 + L], meta[6 + L:6 + 2 * L]
@@ -36,7 +37,7 @@ def _load(golden_dir, name):
 def _net(z, m, precision, **kw):
     from nasa_niswan_b200 import ConvLSTM
     net = ConvLSTM(m["cin"], m["hidden"], m["ks"], m["L"], precision=precision, **kw).cuda()
-    net.load_state_dict({k[6:]: torch.from_numpy(z[k]) for k in z.files if k.startswith("param/")})
+    net.load_state_dict({k[6:]: torch.from_numpy(z[k]) for k in z if k.startswith("param/")})
     return net
 
 

@@ -10,6 +10,7 @@ import pytest
 import torch
 
 from nasa_niswan_b200 import ConvLSTM, ConvLSTMCell, _lib
+from oracle.golden import load_case
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -144,8 +145,8 @@ def test_module_surface_matches_reference_contract(golden_dir):
     # param-count known answer test.ipynb:4698-4699 and state_dict names (utils.py:27,39)
     net = ConvLSTM(5, [64, 32, 16], [5, 3, 3], 3)
     assert [p.numel() for p in net.parameters()] == [441600, 256, 110592, 128, 27648, 64, 16, 1]
-    z = np.load(os.path.join(golden_dir, "lstm_3layer_k533.npz"))
-    ref_sd = {k[6:]: z[k] for k in z.files if k.startswith("param/")}
+    z = load_case(golden_dir, "lstm_3layer_k533")
+    ref_sd = {k[6:]: z[k] for k in z if k.startswith("param/")}
     net = ConvLSTM(5, [32, 16, 16], [5, 3, 3], 3)
     sd = net.state_dict()
     assert list(sd.keys()) == list(ref_sd.keys())
@@ -158,7 +159,7 @@ def test_module_surface_matches_reference_contract(golden_dir):
 
 def test_default_init_matches_reference_rng_stream(golden_dir):
     # same seed -> same parameters as the reference constructor (golden generated with seed 0)
-    z = np.load(os.path.join(golden_dir, "lstm_c21_h32_k3.npz"))
+    z = load_case(golden_dir, "lstm_c21_h32_k3")
     torch.manual_seed(0)
     net = ConvLSTM(21, [32], [3], 1)
     for k, v in net.state_dict().items():

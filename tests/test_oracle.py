@@ -7,20 +7,29 @@ import pytest
 import torch
 
 from oracle import convlstm_oracle as O
+from oracle.golden import load_case
 
 CASES = ["lstm_c21_h32_k3", "lstm_3layer_k533", "lstm_c8_h16_k5"]
 
 
 def load(golden_dir, name):
-    z = np.load(os.path.join(golden_dir, name + ".npz"))
+    z = load_case(golden_dir, name)
     meta = z["meta"].tolist()
     B, T, cin, H, W, L = meta[:6]
     hidden, ks = meta[6:6 + L], meta[6 + L:6 + 2 * L]
-    params = {k[6:]: torch.from_numpy(z[k]) for k in z.files if k.startswith("param/")}
-    grads = {k[5:]: torch.from_numpy(z[k]) for k in z.files if k.startswith("grad/")}
+    params = {k[6:]: torch.from_numpy(z[k]) for k in z if k.startswith("param/")}
+    grads = {k[5:]: torch.from_numpy(z[k]) for k in z if k.startswith("grad/")}
     crop = z["crop"].tolist()
     crop = None if crop[0] < 0 else tuple(crop)
     return z, dict(B=B, T=T, cin=cin, H=H, W=W, L=L, hidden=hidden, ks=ks, crop=crop), params, grads
+
+
+def test_golden_inputs_are_checked_against_the_reference_digest(golden_dir, tmp_path):
+    # a case stores the reference's outputs and the seed of its inputs; inputs drawn from another seed are refused
+    z = np.load(os.path.join(golden_dir, CASES[0] + ".npz"))
+    np.savez(tmp_path / "case.npz", **{k: z[k] for k in z.files if k != "seed"}, seed=z["seed"] + 1)
+    with pytest.raises(RuntimeError, match="draws other inputs"):
+        load_case(str(tmp_path), "case")
 
 
 def test_param_count_known_answer():

@@ -68,17 +68,16 @@ def run_stage(name):
         stage_raw("tf32", 1, 21, 64, 3, 7, 18, True)
         stage_raw("tf32", 3, 8, 16, 5, 11, 13, True)
     elif name in ("fwd_bf16", "fwd_tf32", "bwd_bf16", "bwd_tf32"):
-        import numpy as np
-        from oracle import convlstm_oracle as O
+        from oracle.golden import load_case
         from nasa_niswan_b200 import ConvLSTM
         prec = name.split("_")[1]
         for case in ["lstm_c21_h32_k3", "lstm_c8_h16_k5", "lstm_3layer_k533"]:
-            z = np.load(os.path.join(ROOT, "tests", "golden", case + ".npz"))
+            z = load_case(os.path.join(ROOT, "tests", "golden"), case)
             meta = z["meta"].tolist()
             B, T, cin, H, W, L = meta[:6]
             hidden, ks = meta[6:6 + L], meta[6 + L:6 + 2 * L]
             net = ConvLSTM(cin, hidden, ks, L, precision=prec).cuda()
-            net.load_state_dict({k[6:]: torch.from_numpy(z[k]) for k in z.files if k.startswith("param/")})
+            net.load_state_dict({k[6:]: torch.from_numpy(z[k]) for k in z if k.startswith("param/")})
             x = torch.from_numpy(z["x"]).cuda()
             if name.startswith("fwd"):
                 with torch.no_grad():
