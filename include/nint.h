@@ -48,9 +48,12 @@ typedef struct nint_config {
 /* NINT_FLAG_DETERMINISTIC: gradients are bit-reproducible run to run (utils.py:77-88 asks cuDNN for the same): split-K
  * partial sums go to per-split buffers and are reduced in a fixed order instead of fp32 atomics.
  * NINT_FLAG_INPUT_GRAD: training plans also keep what nint_backward_input / nint_cell_backward need (the reference's
- * autograd yields x.grad and the gradient w.r.t. an explicit initial state, model.py:216-231). */
+ * autograd yields x.grad and the gradient w.r.t. an explicit initial state, model.py:216-231).
+ * NINT_FLAG_STATE_GRAD: training plans also keep what nint_backward_bptt_state / nint_backward_initial_state need (per
+ * layer an fp32 [B,H,W,hc] buffer for dL/dh_T, and the dgrad scratch of dL/dh0). */
 #define NINT_FLAG_DETERMINISTIC 1
 #define NINT_FLAG_INPUT_GRAD 2
+#define NINT_FLAG_STATE_GRAD 4
 #define NINT_X_FP32 0
 #define NINT_X_BF16 1
 
@@ -74,7 +77,9 @@ int nint_plan_set_weights(nint_plan* plan, int layer, const float* weight, const
 int nint_plan_set_head(nint_plan* plan, const float* weight, const float* bias, void* stream);
 
 /* ---- recurrent state.  model.py:258-262 starts every forward from zeros (the default);
- * ConvLSTMCell.forward (model.py:216-217) takes an explicit (h, c). */
+ * ConvLSTMCell.forward (model.py:216-217) takes an explicit (h, c).  A state set here is the initial state of every
+ * later forward until nint_plan_reset_state; nint_plan_get_state reads the final state of the last forward.  On bf16
+ * plans h enters the GEMM rounded to bf16 (like every h_t), on tf32 plans rounded to tf32; c stays fp32. */
 int nint_plan_reset_state(nint_plan* plan, void* stream);
 int nint_plan_set_state(nint_plan* plan, int layer, const float* h, const float* c, void* stream);
 int nint_plan_get_state(nint_plan* plan, int layer, float* h, float* c, void* stream);
@@ -113,6 +118,15 @@ int nint_backward(nint_plan* plan, const float* dpred, const float* dseq, float*
 int nint_backward_bptt(nint_plan* plan, const float* dpred, const float* dseq, float* grad_head_weight,
                        float* grad_head_bias, void* stream);
 int nint_backward_wgrad(nint_plan* plan, int layer, float* grad_weight, float* grad_bias, void* stream);
+/* nint_backward_bptt with upstream gradients of the final state as well: dh_T[l], dc_T[l] [B,Hc_l,H,W] are dL/dh_T and
+ * dL/dc_T of layer l (host arrays of L device pointers; either array and any entry may be NULL = zero).  dpred and dseq
+ * may both be NULL when a state gradient is given.  State gradients need a plan created with NINT_FLAG_STATE_GRAD. */
+int nint_backward_bptt_state(nint_plan* plan, const float* dpred, const float* dseq, const float* const* dh_T,
+                             const float* const* dc_T, float* grad_head_weight, float* grad_head_bias, void* stream);
+/* Gradient w.r.t. the initial state of the last forward (after nint_backward_bptt[_state]; plans created with
+ * NINT_FLAG_STATE_GRAD): dh0[l], dc0[l] [B,Hc_l,H,W] fp32 (host arrays of L device pointers; either array and any entry
+ * may be NULL = not wanted).  dh0 = dgates_0 (*) flip(W_h), dc0 = dc_0 * f_0. */
+int nint_backward_initial_state(nint_plan* plan, float* const* dh0, float* const* dc0, void* stream);
 /* Gradient w.r.t. the input, dx [B,T,C,H,W] fp32 (x.grad of the reference's autograd through model.py:219-220); after
  * nint_backward_bptt, plans created with NINT_FLAG_INPUT_GRAD. */
 int nint_backward_input(nint_plan* plan, float* dx, void* stream);

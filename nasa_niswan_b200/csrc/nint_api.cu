@@ -79,6 +79,7 @@ struct Layer {
   float* Cs = nullptr;     // [nslots_c][B][H][W][hc]
   uint8_t* G = nullptr;    // [T][B][H][W][4hc] E   (training)
   float* dC = nullptr;     // [B][H][W][hc]         (training)
+  float* dh_ext = nullptr; // [B][H][W][hc] upstream dL/dh_T (NINT_FLAG_STATE_GRAD)
   uint8_t *wx = nullptr, *wh = nullptr, *wdx = nullptr, *wdh = nullptr;
   float *bias_q = nullptr, *dw_acc = nullptr, *db_acc = nullptr;
   float* db_resid = nullptr;   // tf32 training plans: [kResidCtas][4][4hc] sums of the dgates rounding residuals (nint_kernels.h)
@@ -133,7 +134,7 @@ struct nint_plan {
   const int* win_start = nullptr;
   CUtensorMap tmb_X, tmbw_X, tmbp_X;
   float *head_w = nullptr, *head_b = nullptr;
-  float* raw = nullptr;      // NINT_FLAG_INPUT_GRAD: [B][H][W][max(cx_pad0, hc0)] fp32 dgrad dump
+  float* raw = nullptr;      // NINT_FLAG_INPUT_GRAD / _STATE_GRAD: [B][H][W][max(cx_pad0, hc0, hc_l)] fp32 dgrad dump
   float* dh_ext = nullptr;   // NINT_FLAG_INPUT_GRAD, cell plans: upstream dL/dh' as [B][H][W][hc] fp32
   float* head_part = nullptr;  // deterministic mode: per-block partial sums of the head gradient
   unsigned* step_done = nullptr;   // [T][B] tile counters of a time-fused conv launch (ConvGemmParams::step_done)
@@ -148,7 +149,7 @@ struct nint_plan {
   bool fwd_done = false;
   bool gates_valid = false; // the saved activated gates of the last forward are intact (BPTT overwrites them in place)
   bool bptt_done = false;   // dgates of the last forward are in place: nint_backward_wgrad may run
-  bool deterministic = false, input_grad = false;
+  bool deterministic = false, input_grad = false, state_grad = false;
   // Programmatic dependent launch of the conv kernels (NINT_PDL=1 switches it on).  OFF by default: it buys 0.4-0.6 % at
   // cfg 2, but with the last build of round 2 the one-launch-per-step schedule of the reference's three-layer recipe
   // died with "unspecified launch failure" at a random step in 4 of 8 (and 5 of 12) 150-step runs with it and in 0 of
@@ -334,12 +335,15 @@ size_t carve(nint_plan* p, uint8_t* base) {
   if (tr && p->deterministic)
     p->head_part = reinterpret_cast<float*>(take(static_cast<size_t>(head_bwd_blocks(p->B)) * (top.hc_real + 1) * 4));
   p->step_done = reinterpret_cast<unsigned*>(take(static_cast<size_t>(p->T) * p->B * 4));
-  if (tr && p->input_grad) {
-    const Layer& y0 = p->layer[0];
-    const size_t cols = y0.cin_rows > y0.hc ? y0.cin_rows : y0.hc;
-    p->raw = reinterpret_cast<float*>(take(npix * cols * 4));
-    p->dh_ext = reinterpret_cast<float*>(take(npix * y0.hc * 4));
-  }
+  // dgrad dump: dx / the cell's dh (layer 0) and dh0 of every layer (nint_backward_initial_state)
+  int raw_cols = 0;
+  if (tr && p->input_grad) raw_cols = p->layer[0].cin_rows > p->layer[0].hc ? p->layer[0].cin_rows : p->layer[0].hc;
+  if (tr && p->state_grad)
+    for (int l = 0; l < p->L; ++l) raw_cols = raw_cols > p->layer[l].hc ? raw_cols : p->layer[l].hc;
+  if (raw_cols > 0) p->raw = reinterpret_cast<float*>(take(npix * raw_cols * 4));
+  if (tr && p->input_grad) p->dh_ext = reinterpret_cast<float*>(take(npix * p->layer[0].hc * 4));
+  if (tr && p->state_grad)
+    for (int l = 0; l < p->L; ++l) p->layer[l].dh_ext = reinterpret_cast<float*>(take(npix * p->layer[l].hc * 4));
   return off;
 }
 
@@ -741,6 +745,7 @@ int nint_plan_create(const nint_config* cfg, nint_plan** out) {
   p->ce = 64 / p->esize;
   p->deterministic = (cfg->flags & NINT_FLAG_DETERMINISTIC) != 0;
   p->input_grad = (cfg->flags & NINT_FLAG_INPUT_GRAD) != 0;
+  p->state_grad = (cfg->flags & NINT_FLAG_STATE_GRAD) != 0;
   {  // debug / A-B knobs (documented in DESIGN.md): CTA pairs on/off, experiment flags
     const char* c = getenv("NINT_CLUSTER");
     p->cluster = c ? atoi(c) : 2;
@@ -1344,9 +1349,16 @@ static int bwd_should_fuse(nint_plan* p, int l, bool* fuse) {
   return 0;
 }
 
+// upstream gradient of the final state, per layer: dh_ext[l] ([B][H][W][hc] fp32) is added to layer l's dh at t = T-1,
+// dc_given[l] says that layer's running dc already holds dL/dc_T
+struct StateGrad {
+  const float* dh_ext[NINT_MAX_LAYERS] = {};
+  bool dc_given[NINT_MAX_LAYERS] = {};
+};
+
 // one fused dgrad + gate-backward launch of layer l at step t for images [b0, b0 + nb) (nb = 0: all); n_steps > 1: steps
 // t, t-1, .. t-n_steps+1 as ONE time-fused launch (t < T-1: all of them have a dgates_{t+1} segment and a running dc)
-static int bwd_step(nint_plan* p, int l, int t, const float* dpred, const float* dseq, const float* dh_ext, bool dc_given,
+static int bwd_step(nint_plan* p, int l, int t, const float* dpred, const float* dseq, const StateGrad& sg,
                     cudaStream_t st, int b0, int nb, int n_steps = 1) {
   const long long HW = static_cast<long long>(p->H) * p->W;
   const int L = p->L, T = p->T;
@@ -1359,7 +1371,7 @@ static int bwd_step(nint_plan* p, int l, int t, const float* dpred, const float*
   if (l < L - 1) g.seg[s++].slot = t;
   g.slot_g = t;
   g.slot_c_prev = (t == 0 && p->zero_init) ? -1 : t;
-  g.has_dc_in = (t == T - 1) ? (dc_given ? 1 : 0) : 1;
+  g.has_dc_in = (t == T - 1) ? (sg.dc_given[l] ? 1 : 0) : 1;
   g.head_dpred = nullptr; g.head_w = nullptr; g.head_dpred_bstride = 0;
   if (l == L - 1) {
     if (dseq) {
@@ -1373,7 +1385,7 @@ static int bwd_step(nint_plan* p, int l, int t, const float* dpred, const float*
       g.head_w = p->head_w;
     }
   }
-  g.dh_ext = (l == L - 1 && t == T - 1) ? dh_ext : nullptr;
+  g.dh_ext = t == T - 1 ? sg.dh_ext[l] : nullptr;
   g.db_resid = resid_on(p) ? y.db_resid : nullptr;
   set_batch_range(p, g, b0, nb);
   g.n_steps = 1;
@@ -1392,7 +1404,7 @@ static int bwd_step(nint_plan* p, int l, int t, const float* dpred, const float*
   return 0;
 }
 
-static int bptt_loop(nint_plan* p, const float* dpred, const float* dseq, const float* dh_ext, bool dc_given, cudaStream_t st) {
+static int bptt_loop(nint_plan* p, const float* dpred, const float* dseq, const StateGrad& sg, cudaStream_t st) {
   // ---- BPTT: reverse time, top layer first.  The dgrad conv of step t+1 (and of the layer
   // above at step t) accumulates dh_t in TMEM; its epilogue is the gate backward of step t and
   // overwrites the saved gates with dgates in place.
@@ -1410,12 +1422,12 @@ static int bptt_loop(nint_plan* p, const float* dpred, const float* dseq, const 
     // A fused layer runs its steps T-2 .. 0 as ONE persistent launch after its step T-1 (which has no dgates_{t+1}
     // segment); the others one launch per step
     for (int l = p->L - 1; l >= 0; --l) {
-      if (bwd_step(p, l, p->T - 1, dpred, dseq, dh_ext, dc_given, st, 0, 0)) return 1;
+      if (bwd_step(p, l, p->T - 1, dpred, dseq, sg, st, 0, 0)) return 1;
       if (fuse_l[l]) {
-        if (bwd_step(p, l, p->T - 2, dpred, dseq, dh_ext, dc_given, st, 0, 0, p->T - 1)) return 1;
+        if (bwd_step(p, l, p->T - 2, dpred, dseq, sg, st, 0, 0, p->T - 1)) return 1;
       } else {
         for (int t = p->T - 2; t >= 0; --t)
-          if (bwd_step(p, l, t, dpred, dseq, dh_ext, dc_given, st, 0, 0)) return 1;
+          if (bwd_step(p, l, t, dpred, dseq, sg, st, 0, 0)) return 1;
       }
     }
   } else
@@ -1423,22 +1435,26 @@ static int bptt_loop(nint_plan* p, const float* dpred, const float* dseq, const 
     const int nb = b0 + SB <= p->B ? SB : p->B - b0;
     for (int t = p->T - 1; t >= 0; --t)
       for (int l = p->L - 1; l >= 0; --l)
-        if (bwd_step(p, l, t, dpred, dseq, dh_ext, dc_given, st, b0, SB < p->B ? nb : 0)) return 1;
+        if (bwd_step(p, l, t, dpred, dseq, sg, st, b0, SB < p->B ? nb : 0)) return 1;
   }
   p->gates_valid = false;
   p->bptt_done = true;
   return 0;
 }
 
-int nint_backward_bptt(nint_plan* p, const float* dpred, const float* dseq, float* grad_head_weight,
-                       float* grad_head_bias, void* stream) {
+int nint_backward_bptt_state(nint_plan* p, const float* dpred, const float* dseq, const float* const* dh_T,
+                             const float* const* dc_T, float* grad_head_weight, float* grad_head_bias, void* stream) {
   if (check_ready(p)) return 1;
   if (!p->cfg.training) return fail("nint_backward needs a training plan");
   if (!p->fwd_done) return fail("nint_backward before nint_forward");
   if (!p->gates_valid)
     return fail("nint_backward: the activations saved by the last forward were already consumed by a backward (BPTT "
                 "turns the saved gates into their gradients in place); run the forward again");
-  if (!dpred && !dseq) return fail("nint_backward: no upstream gradient");
+  bool state_in = false;
+  for (int l = 0; l < p->L; ++l) state_in = state_in || (dh_T && dh_T[l]) || (dc_T && dc_T[l]);
+  if (state_in && !p->state_grad)
+    return fail("nint_backward: gradients of the final state need a training plan created with NINT_FLAG_STATE_GRAD");
+  if (!dpred && !dseq && !state_in) return fail("nint_backward: no upstream gradient");
   if (dseq && !p->cfg.return_sequence) return fail("dseq requires return_sequence in the plan");
   if (dseq && dpred) return fail("pass either dpred or dseq (fold dpred into dseq[:, T-1])");
   p->bptt_done = false;
@@ -1446,6 +1462,20 @@ int nint_backward_bptt(nint_plan* p, const float* dpred, const float* dseq, floa
   const long long HW = static_cast<long long>(p->H) * p->W;
   const int L = p->L, T = p->T;
   const Layer& top = p->layer[L - 1];
+  // ---- final-state gradients: dL/dh_T joins layer l's dh at T-1 (next to the head term), dL/dc_T starts its running dc
+  StateGrad sg;
+  for (int l = 0; l < L && state_in; ++l) {
+    Layer& y = p->layer[l];
+    if (dh_T && dh_T[l]) {
+      LAUNCH(p, K_OTHER, st, launch_nchw_to_nhwc_f32(dh_T[l], y.dh_ext, p->B, y.hc_real, p->H, p->W, y.hc, st));
+      sg.dh_ext[l] = y.dh_ext;   // padding channels stay zero from nint_plan_bind
+    }
+    if (dc_T && dc_T[l]) {
+      CK(cudaMemsetAsync(y.dC, 0, static_cast<size_t>(p->B) * HW * y.hc * 4, st));
+      LAUNCH(p, K_OTHER, st, launch_nchw_to_nhwc_f32(dc_T[l], y.dC, p->B, y.hc_real, p->H, p->W, y.hc, st));
+      sg.dc_given[l] = true;
+    }
+  }
   // ---- head gradients (model.py:274): dw = sum dpred * h_T, db = sum dpred
   if (grad_head_weight && grad_head_bias) {
     CK(cudaMemsetAsync(grad_head_weight, 0, top.hc_real * 4, st));
@@ -1458,7 +1488,32 @@ int nint_backward_bptt(nint_plan* p, const float* dpred, const float* dseq, floa
         LAUNCH(p, K_OTHER, st, launch_head_bwd(p->dtype, slot_ptr(p, top.Hs, t + 1, top.hc_pad), dseq + t * HW, T * HW, grad_head_weight,
                            grad_head_bias, HW, p->B, top.hc_real, top.hc_pad, p->head_part, st));
   }
-  return bptt_loop(p, dpred, dseq, nullptr, false, st);
+  return bptt_loop(p, dpred, dseq, sg, st);
+}
+
+int nint_backward_bptt(nint_plan* p, const float* dpred, const float* dseq, float* grad_head_weight,
+                       float* grad_head_bias, void* stream) {
+  return nint_backward_bptt_state(p, dpred, dseq, nullptr, nullptr, grad_head_weight, grad_head_bias, stream);
+}
+
+// dL/dh_{-1} and dL/dc_{-1} of every layer: h_{-1} only enters layer l's gate convolution at t = 0 (the layer above
+// reads h_t for t >= 0), so dh0 = dgates_0 (*) flip(W_h); the running dc after step 0 is dc_0 * f_0 = dc0
+int nint_backward_initial_state(nint_plan* p, float* const* dh0, float* const* dc0, void* stream) {
+  if (check_ready(p)) return 1;
+  if (!p->cfg.training || !p->state_grad)
+    return fail("nint_backward_initial_state needs a training plan created with NINT_FLAG_STATE_GRAD");
+  if (!p->bptt_done) return fail("nint_backward_initial_state before nint_backward_bptt");
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const long long HW = static_cast<long long>(p->H) * p->W;
+  for (int l = 0; l < p->L; ++l) {
+    Layer& y = p->layer[l];
+    if (dh0 && dh0[l]) {
+      if (dgrad_raw(p, l, 0, 3, y.hc, p->raw, st)) return 1;
+      LAUNCH(p, K_OTHER, st, launch_unpack_raw(p->raw, dh0[l], p->B, y.hc_real, p->H, p->W, y.hc, y.hc_real * HW, st));
+    }
+    if (dc0 && dc0[l]) LAUNCH(p, K_OTHER, st, launch_nhwc_to_nchw_f32(y.dC, dc0[l], p->B, y.hc_real, p->H, p->W, y.hc, st));
+  }
+  return 0;
 }
 
 // ---- weight / bias gradient of one layer, batched over all T steps (needs the dgates nint_backward_bptt left)
@@ -1546,7 +1601,10 @@ int nint_cell_backward(nint_plan* p, const float* dh_out, const float* dc_out, f
     CK(cudaMemsetAsync(y.dC, 0, npix * y.hc * 4, st));
     LAUNCH(p, K_OTHER, st, launch_nchw_to_nhwc_f32(dc_out, y.dC, p->B, y.hc_real, p->H, p->W, y.hc, st));
   }
-  if (bptt_loop(p, nullptr, nullptr, dh_out ? p->dh_ext : nullptr, dc_out != nullptr, st)) return 1;
+  StateGrad sg;
+  sg.dh_ext[0] = dh_out ? p->dh_ext : nullptr;
+  sg.dc_given[0] = dc_out != nullptr;
+  if (bptt_loop(p, nullptr, nullptr, sg, st)) return 1;
   if (dc) LAUNCH(p, K_OTHER, st, launch_nhwc_to_nchw_f32(y.dC, dc, p->B, y.hc_real, p->H, p->W, y.hc, st));
   if (dh) {
     if (dgrad_raw(p, 0, 0, 3, y.hc, p->raw, st)) return 1;

@@ -21,7 +21,8 @@ class Plan:
 
     def __init__(self, batch: int, seq_len: int, height: int, width: int, in_channels: int,
                  hidden: Sequence[int], ksize: Sequence[int], precision: str = "bf16", training: bool = False,
-                 return_sequence: bool = False, device=None, deterministic: bool = False, input_grad: bool = False):
+                 return_sequence: bool = False, device=None, deterministic: bool = False, input_grad: bool = False,
+                 state_grad: bool = False):
         if precision not in PRECISIONS:
             raise ValueError(f"precision must be one of {sorted(PRECISIONS)}")
         if len(hidden) != len(ksize):
@@ -35,14 +36,15 @@ class Plan:
         self.B, self.T, self.H, self.W, self.C = batch, seq_len, height, width, in_channels
         self.hidden, self.ksize, self.L = list(hidden), list(ksize), len(hidden)
         self.training, self.return_sequence, self.precision = bool(training), bool(return_sequence), precision
-        self.deterministic, self.input_grad = bool(deterministic), bool(input_grad)
+        self.deterministic, self.input_grad, self.state_grad = bool(deterministic), bool(input_grad), bool(state_grad)
         cfg = _lib.NintConfig()
         cfg.batch, cfg.seq_len, cfg.height, cfg.width = batch, seq_len, height, width
         cfg.in_channels, cfg.num_layers = in_channels, self.L
         for i, (h, k) in enumerate(zip(hidden, ksize)):
             cfg.hidden[i], cfg.ksize[i] = h, k
         cfg.dtype, cfg.training, cfg.return_sequence = PRECISIONS[precision], int(training), int(return_sequence)
-        cfg.flags = (_lib.FLAG_DETERMINISTIC if deterministic else 0) | (_lib.FLAG_INPUT_GRAD if input_grad else 0)
+        cfg.flags = ((_lib.FLAG_DETERMINISTIC if deterministic else 0) | (_lib.FLAG_INPUT_GRAD if input_grad else 0) |
+                     (_lib.FLAG_STATE_GRAD if state_grad else 0))
         self._h = ctypes.c_void_p()
         _lib.check(self.lib.nint_plan_create(ctypes.byref(cfg), ctypes.byref(self._h)), "nint_plan_create")
         self.workspace_bytes = self.lib.nint_plan_workspace_bytes(self._h)
@@ -53,6 +55,7 @@ class Plan:
         self.generation = 0          # bumped by every forward and every backward: BPTT consumes the saved activations
         self._weight_keys = [None] * (self.L + 1)
         self._keep = None            # tensors the queued kernels still read (frame bank, window indices)
+        self._stateful = False       # the last forward was given an initial state (it stays in the workspace)
 
     def __del__(self):
         h, self._h = getattr(self, "_h", None), None
@@ -114,6 +117,40 @@ class Plan:
     def reset_state(self):
         with _lib.on_device(self.device):
             _lib.check(self.lib.nint_plan_reset_state(self._h, self._stream()), "nint_plan_reset_state")
+        self._stateful = False
+
+    def _state_shape(self, layer: int):
+        return (self.B, self.hidden[layer], self.H, self.W)
+
+    def check_state(self, state) -> bool:
+        """Validates an initial state (see _initial_state); True when it holds at least one tensor."""
+        if state is None:
+            return False
+        state = list(state)
+        if len(state) != self.L or not all(isinstance(pair, (tuple, list)) and len(pair) == 2 for pair in state):
+            raise ValueError(f"the initial state must be a list of {self.L} (h, c) pairs, one per layer")
+        for l, (h, c) in enumerate(state):
+            for t, name in ((h, f"h0[{l}]"), (c, f"c0[{l}]")):
+                if t is not None:
+                    self._check_dev(t, name, self._state_shape(l))
+        return any(t is not None for pair in state for t in pair)
+
+    def _initial_state(self, state):
+        """Makes `state` the initial state of the next forward: None, or per layer (h, c) [B,Hc_l,H,W] fp32 where a
+        missing tensor (None) means zeros.  A plan keeps a state it was given, and plans are cached and shared, so a
+        forward without a state resets the one an earlier forward was given; otherwise it issues no call."""
+        given = self.check_state(state)
+        if self._stateful:
+            self.reset_state()
+        if not given:
+            return
+        for l, (h, c) in enumerate(state):
+            if h is None and c is None:
+                continue
+            shape = self._state_shape(l)
+            zero = lambda: torch.zeros(shape, dtype=torch.float32, device=self.device)
+            self.set_state(l, zero() if h is None else h, zero() if c is None else c)
+        self._stateful = True
 
     def set_state(self, layer: int, h: torch.Tensor, c: torch.Tensor):
         shape = (self.B, self.hidden[layer], self.H, self.W)
@@ -131,6 +168,10 @@ class Plan:
             _lib.check(self.lib.nint_plan_get_state(self._h, layer, _ptr(h), _ptr(c), self._stream()), "nint_plan_get_state")
         return h, c
 
+    def final_state(self):
+        """[(h_T, c_T) per layer] of the last forward, fp32 [B,Hc_l,H,W]"""
+        return [self.get_state(l) for l in range(self.L)]
+
     # ---- compute
     def _outputs(self):
         pred = torch.empty((self.B, 1, self.H, self.W), dtype=torch.float32, device=self.device)
@@ -138,12 +179,14 @@ class Plan:
                if self.return_sequence else None)
         return pred, seq
 
-    def forward(self, x: torch.Tensor):
-        """x [B,T,C,H,W] fp32, or bf16 on a bf16 plan (host-staged windows: half the PCIe bytes, identical results)."""
+    def forward(self, x: torch.Tensor, state=None):
+        """x [B,T,C,H,W] fp32, or bf16 on a bf16 plan (host-staged windows: half the PCIe bytes, identical results).
+        state: optional initial [(h, c) per layer] (see _initial_state); None starts from zeros."""
         self._check_dev(x, "x", (self.B, self.T, self.C, self.H, self.W), dtypes=(torch.float32, torch.bfloat16))
         if x.dtype == torch.bfloat16 and self.precision != "bf16":
             raise TypeError("bf16 inputs need precision='bf16' (a tf32 plan would lose input precision)")
         x = x.detach().contiguous()
+        self._initial_state(state)
         pred, seq = self._outputs()
         with _lib.on_device(self.device):
             _lib.check(self.lib.nint_forward_ex(self._h, _ptr(x), _lib.X_BF16 if x.dtype == torch.bfloat16 else _lib.X_FP32,
@@ -151,9 +194,10 @@ class Plan:
         self.generation += 1
         return pred, seq
 
-    def forward_bank(self, frames: torch.Tensor, win_start: torch.Tensor):
+    def forward_bank(self, frames: torch.Tensor, win_start: torch.Tensor, state=None):
         """frames: frame bank [N,H,W,c_pad] in this plan's operand layout (preprocess.FrameBank); win_start: int32 [B]
-        on the device -- sample b reads frames win_start[b] .. win_start[b]+T-1 through the TMA descriptors."""
+        on the device -- sample b reads frames win_start[b] .. win_start[b]+T-1 through the TMA descriptors.
+        state: as in forward."""
         c_pad, _, dt = self.input_layout()
         if frames.dim() != 4 or tuple(frames.shape[1:]) != (self.H, self.W, c_pad):
             raise ValueError(f"frame bank has shape {tuple(frames.shape)}, expected (N, {self.H}, {self.W}, {c_pad})")
@@ -161,6 +205,7 @@ class Plan:
         self._check_dev(win_start, "win_start", (self.B,), dtypes=(torch.int32,))
         if not frames.is_contiguous() or not win_start.is_contiguous():
             raise ValueError("frame bank and win_start must be contiguous")
+        self._initial_state(state)
         pred, seq = self._outputs()
         with _lib.on_device(self.device):
             _lib.check(self.lib.nint_forward_bank(self._h, _ptr(frames), frames.shape[0], _ptr(win_start), _ptr(pred),
@@ -193,11 +238,14 @@ class Plan:
             ghb = torch.empty((1,), dtype=torch.float32, device=self.device)
         return gw, gb, ghw, ghb
 
-    def backward(self, dpred: Optional[torch.Tensor], dseq: Optional[torch.Tensor] = None, out=None, on_ready=None):
+    def backward(self, dpred: Optional[torch.Tensor], dseq: Optional[torch.Tensor] = None, out=None, on_ready=None,
+                 dh_T=None, dc_T=None):
         """Returns ([grad_weight_l], [grad_bias_l], grad_head_weight, grad_head_bias).  `out`: optional
         (gw list, gb list, ghw, ghb) of preallocated contiguous fp32 tensors the gradients are written into
         (e.g. views of one flat all-reduce buffer).  `on_ready(i)`: called as soon as the kernels producing a
         gradient bucket are queued on the current stream -- i = L for the head, then i = L-1 .. 0 for the layers.
+        dh_T / dc_T: optional per-layer dL/dh_T, dL/dc_T [B,Hc_l,H,W] of the final state (entries may be None; plans
+        made with state_grad=True); backward_initial_state() then gives dL/dh0, dL/dc0.
         BPTT turns the saved gates into their gradients in place: one backward per forward."""
         if dseq is not None:
             dseq = dseq.detach().contiguous().clone() if dpred is not None else dseq.detach().contiguous()
@@ -208,10 +256,12 @@ class Plan:
         if dpred is not None:
             dpred = dpred.detach().contiguous()
             self._check_dev(dpred, "dpred", (self.B, 1, self.H, self.W))
+        dh_T, dc_T = self._state_table(dh_T, "dh_T"), self._state_table(dc_T, "dc_T")
         gw, gb, ghw, ghb = self._grad_buffers(out)
         self.generation += 1        # the saved activations are consumed: a second backward of the same forward must fail
+        state_in = dh_T is not None or dc_T is not None
         with _lib.on_device(self.device):
-            if on_ready is None:
+            if on_ready is None and not state_in:
                 arr_w = (ctypes.c_void_p * self.L)(*[t.data_ptr() for t in gw])
                 arr_b = (ctypes.c_void_p * self.L)(*[t.data_ptr() for t in gb])
                 _lib.check(self.lib.nint_backward(self._h, _ptr(dpred), _ptr(dseq), arr_w, arr_b, _ptr(ghw), _ptr(ghb),
@@ -219,14 +269,48 @@ class Plan:
                 return gw, gb, ghw, ghb
             # staged: the caller hears about every finished gradient bucket (the head's after BPTT, then one layer at a
             # time, top layer first) while the following wgrad kernels are still queued -- nint.h nint_backward_bptt/_wgrad
-            _lib.check(self.lib.nint_backward_bptt(self._h, _ptr(dpred), _ptr(dseq), _ptr(ghw), _ptr(ghb), self._stream()),
-                       "nint_backward_bptt")
-            on_ready(self.L)
+            if state_in:
+                _lib.check(self.lib.nint_backward_bptt_state(self._h, _ptr(dpred), _ptr(dseq), self._ptr_table(dh_T),
+                                                             self._ptr_table(dc_T), _ptr(ghw), _ptr(ghb), self._stream()),
+                           "nint_backward_bptt_state")
+            else:
+                _lib.check(self.lib.nint_backward_bptt(self._h, _ptr(dpred), _ptr(dseq), _ptr(ghw), _ptr(ghb),
+                                                       self._stream()), "nint_backward_bptt")
+            notify = on_ready or (lambda i: None)
+            notify(self.L)
             for l in range(self.L - 1, -1, -1):
                 _lib.check(self.lib.nint_backward_wgrad(self._h, l, _ptr(gw[l]), _ptr(gb[l]), self._stream()),
                            "nint_backward_wgrad")
-                on_ready(l)
+                notify(l)
         return gw, gb, ghw, ghb
+
+    def _state_table(self, ts, name):
+        """per-layer state gradients -> contiguous tensors (None where absent), or None when none is given"""
+        if ts is None or all(t is None for t in ts):
+            return None
+        if len(ts) != self.L:
+            raise ValueError(f"{name} has {len(ts)} layers, expected {self.L}")
+        out = []
+        for l, t in enumerate(ts):
+            if t is not None:
+                self._check_dev(t, f"{name}[{l}]", self._state_shape(l))
+                t = t.detach().contiguous()
+            out.append(t)
+        return out
+
+    def _ptr_table(self, ts):
+        return None if ts is None else (ctypes.c_void_p * self.L)(*[None if t is None else t.data_ptr() for t in ts])
+
+    def backward_initial_state(self):
+        """([dL/dh0_l], [dL/dc0_l]) fp32 [B,Hc_l,H,W] of the last backward (plans made with state_grad=True); call after
+        `backward`."""
+        new = lambda l: torch.empty(self._state_shape(l), dtype=torch.float32, device=self.device)
+        dh0 = [new(l) for l in range(self.L)]
+        dc0 = [new(l) for l in range(self.L)]
+        with _lib.on_device(self.device):
+            _lib.check(self.lib.nint_backward_initial_state(self._h, self._ptr_table(dh0), self._ptr_table(dc0),
+                                                            self._stream()), "nint_backward_initial_state")
+        return dh0, dc0
 
     def backward_input(self) -> torch.Tensor:
         """dx [B,T,C,H,W] of the last backward (plans made with input_grad=True); call after `backward`."""

@@ -132,7 +132,15 @@ class ConvLSTM(nn.Module):
     that test.ipynb:273 was run against: returns `(pred, hs[B,T,H,W])`.
     `precision`: "bf16" (bf16 operands, fp32 accumulate/state) or "tf32".
     x may be fp32 or (bf16 precision) bf16; `forward_windows(bank, starts)` reads the windows from an HBM-resident
-    `preprocess.FrameBank` instead (dataset.py:551-637)."""
+    `preprocess.FrameBank` instead (dataset.py:551-637).
+
+    Both take `hidden_state`, the initial state as a list of L pairs (h_l, c_l) [B, Hc_l, H, W] fp32 (None: zeros, for
+    all layers or, as a pair of Nones, for one), and `return_state`: then the result is (out, [(h_T, c_T) per layer])
+    with `out` what the call returns without it.  Gradients flow to the initial state when it requires grad and from
+    any use of the final state, so windows of one long record can be chained (truncated BPTT: pass the detached final
+    state of window k as the initial state of window k+1).  Precision: h0 enters the gate convolution rounded to the
+    operand format like every h_t (bf16 on bf16 plans, tf32 on tf32 plans); c0 stays fp32.  Two forwards of one shape
+    share a workspace, so a window must be back-propagated before the next forward of the same shape."""
 
     def __init__(self, input_channels, hidden_channels: Sequence[int], kernel_size: Sequence[int], num_layers,
                  precision: str = "bf16", return_sequence: bool = False):
@@ -157,54 +165,83 @@ class ConvLSTM(nn.Module):
             ps += [cell.conv.weight, cell.conv.bias]
         return ps + [self.conv.weight, self.conv.bias]
 
-    def plan_for_shape(self, B, T, H, W, device, training, set_params=True, input_grad=False):
+    def plan_for_shape(self, B, T, H, W, device, training, set_params=True, input_grad=False, state_grad=False):
         device = torch.device(device)
         if device.index is None:
             device = torch.device("cuda", torch.cuda.current_device())
         det = bool(training) and _deterministic_default()
-        key = (B, T, H, W, bool(training), self.return_sequence, self.precision, device, bool(input_grad), det)
+        key = (B, T, H, W, bool(training), self.return_sequence, self.precision, device, bool(input_grad),
+               bool(state_grad), det)
         hidden = [c.hidden_channels for c in self.layers]
         ks = [c.kernel_size for c in self.layers]
         plan = self._plans.get(key, lambda: Plan(B, T, H, W, self.input_channels, hidden, ks, precision=self.precision,
                                                  training=training, return_sequence=self.return_sequence,
-                                                 device=device, deterministic=det, input_grad=input_grad))
+                                                 device=device, deterministic=det, input_grad=input_grad,
+                                                 state_grad=state_grad))
         if set_params:
             for l, cell in enumerate(self.layers):
                 plan.set_weights(l, cell.conv.weight, cell.conv.bias)
             plan.set_head(self.conv.weight, self.conv.bias)
         return plan
 
-    def plan_for(self, x, training, set_params=True, input_grad=False):
+    def plan_for(self, x, training, set_params=True, input_grad=False, state_grad=False):
         B, T, C, H, W = x.size()
         if C != self.input_channels:
             raise ValueError(f"expected {self.input_channels} input channels, got {C}")
-        return self.plan_for_shape(B, T, H, W, x.device, training, set_params, input_grad)
+        return self.plan_for_shape(B, T, H, W, x.device, training, set_params, input_grad, state_grad)
 
     def _wants_grad(self, params):
         return torch.is_grad_enabled() and any(p.requires_grad for p in params)
 
-    def forward(self, x):
+    def _state_requires_grad(self, hidden_state):
+        return (hidden_state is not None and torch.is_grad_enabled() and
+                any(t is not None and t.requires_grad for pair in hidden_state for t in pair))
+
+    def _stateful(self, op, inputs, plan, hidden_state, return_state):
+        """the *_state op from `hidden_state`; the result as forward returns it"""
+        plan.check_state(hidden_state)
+        pairs = hidden_state if hidden_state is not None else [(None, None)] * self.num_layers
+        empty = torch.empty(0, dtype=torch.float32, device=plan.device)     # the ops' stand-in for a zero state
+        h0 = [empty if h is None else h for h, _ in pairs]
+        c0 = [empty if c is None else c for _, c in pairs]
+        pred, seq, hT, cT = op(*inputs, self._params(), h0, c0, ops.register_plan(plan))
+        out = (pred, seq) if self.return_sequence else pred
+        return (out, list(zip(hT, cT))) if return_state else out
+
+    def forward(self, x, hidden_state=None, return_state=False):
         if not x.is_cuda:
             raise RuntimeError("ConvLSTM runs on CUDA (B200) only: there is no CPU fallback; move the module and "
                                "its input to the GPU")
         params = self._params()
         need_dx = torch.is_grad_enabled() and x.requires_grad
-        training = need_dx or self._wants_grad(params)
-        plan = self.plan_for(x, training, set_params=False, input_grad=need_dx)   # the op repacks the weights it is handed
+        state_req = self._state_requires_grad(hidden_state)
+        training = need_dx or state_req or self._wants_grad(params)
+        # the final state is in the graph when returned from a recorded call: it may be used by the loss
+        state_grad = training and (state_req or return_state)
+        plan = self.plan_for(x, training, set_params=False, input_grad=need_dx,     # the op repacks the weights it is
+                             state_grad=state_grad)                                  # handed
+        if hidden_state is not None or return_state:
+            return self._stateful(torch.ops.nint.convlstm_forward_state, (x,), plan, hidden_state, return_state)
         # torch.library op (ops.py): forward = nint_forward (T x L fused cell steps + head), autograd = nint_backward
         pred, seq = torch.ops.nint.convlstm_forward(x, params, ops.register_plan(plan))
         return (pred, seq) if self.return_sequence else pred
 
-    def forward_windows(self, bank, win_start, seq_len):
+    def forward_windows(self, bank, win_start, seq_len, hidden_state=None, return_state=False):
         """bank: preprocess.FrameBank (frames resident in HBM in the operand layout); win_start: int tensor [B] of
-        window start frames -> the same outputs as forward(x) with x[b] = frames[win_start[b] : win_start[b]+T]."""
+        window start frames -> the same outputs as forward(x) with x[b] = frames[win_start[b] : win_start[b]+T].
+        hidden_state / return_state: as in forward."""
         params = self._params()
         starts = win_start.to(device=bank.frames.device, dtype=torch.int32).contiguous()
         bank.check_windows(win_start, seq_len)
         N, H, W, _ = bank.frames.shape
-        plan = self.plan_for_shape(starts.shape[0], int(seq_len), H, W, bank.frames.device, self._wants_grad(params),
-                                   set_params=False)
+        state_req = self._state_requires_grad(hidden_state)
+        training = state_req or self._wants_grad(params)
+        plan = self.plan_for_shape(starts.shape[0], int(seq_len), H, W, bank.frames.device, training,
+                                   set_params=False, state_grad=training and (state_req or return_state))
         bank.check_plan(plan)
+        if hidden_state is not None or return_state:
+            return self._stateful(torch.ops.nint.convlstm_forward_bank_state, (bank.frames, starts), plan, hidden_state,
+                                  return_state)
         pred, seq = torch.ops.nint.convlstm_forward_bank(bank.frames, starts, params, ops.register_plan(plan))
         return (pred, seq) if self.return_sequence else pred
 

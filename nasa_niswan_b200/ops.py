@@ -135,6 +135,141 @@ torch.library.register_autograd("nint::convlstm_forward", _backward, setup_conte
 torch.library.register_autograd("nint::convlstm_forward_bank", _backward_bank, setup_context=_setup_context)
 
 
+# ---- the same forwards from an explicit initial state, returning the final state (nn.LSTM's (h0, c0) -> (h_n, c_n)).
+# h0 / c0 hold one tensor per layer [B,Hc_l,H,W]; an empty tensor stands for the zero state of that layer.
+def _given(ts):
+    return [None if t.numel() == 0 else t for t in ts]
+
+
+def _state_outputs(plan, pred, seq):
+    hT, cT = zip(*plan.final_state())
+    return pred, (seq if seq is not None else pred.new_empty(0)), list(hT), list(cT)
+
+
+def _state_fakes(ref, plan, B, H, W, T):
+    states = [ref.new_empty((B, hc, H, W), dtype=torch.float32) for hc in plan.hidden]
+    return (ref.new_empty((B, 1, H, W), dtype=torch.float32),
+            ref.new_empty((B, T, H, W) if plan.return_sequence else (0,), dtype=torch.float32),
+            states, [torch.empty_like(s) for s in states])
+
+
+@torch.library.custom_op("nint::convlstm_forward_state", mutates_args=(), device_types="cuda")
+def convlstm_forward_state(x: Tensor, params: List[Tensor], h0: List[Tensor], c0: List[Tensor],
+                           plan_id: int) -> Tuple[Tensor, Tensor, List[Tensor], List[Tensor]]:
+    """convlstm_forward started from (h0[l], c0[l]); returns (pred, seq, [h_T per layer], [c_T per layer])."""
+    plan = _plan(plan_id)
+    _set_params(plan, params)
+    pred, seq = plan.forward(x, list(zip(_given(h0), _given(c0))))
+    return _state_outputs(plan, pred, seq)
+
+
+@convlstm_forward_state.register_fake
+def _(x, params, h0, c0, plan_id):
+    B, T, _, H, W = x.shape
+    return _state_fakes(x, _plan(plan_id), B, H, W, T)
+
+
+@torch.library.custom_op("nint::convlstm_forward_bank_state", mutates_args=(), device_types="cuda")
+def convlstm_forward_bank_state(frames: Tensor, win_start: Tensor, params: List[Tensor], h0: List[Tensor],
+                                c0: List[Tensor], plan_id: int) -> Tuple[Tensor, Tensor, List[Tensor], List[Tensor]]:
+    """convlstm_forward_bank started from (h0[l], c0[l]); returns (pred, seq, [h_T per layer], [c_T per layer])."""
+    plan = _plan(plan_id)
+    _set_params(plan, params)
+    pred, seq = plan.forward_bank(frames, win_start, list(zip(_given(h0), _given(c0))))
+    return _state_outputs(plan, pred, seq)
+
+
+@convlstm_forward_bank_state.register_fake
+def _(frames, win_start, params, h0, c0, plan_id):
+    plan = _plan(plan_id)
+    return _state_fakes(frames, plan, win_start.shape[0], frames.shape[1], frames.shape[2], plan.T)
+
+
+@torch.library.custom_op("nint::convlstm_backward_state", mutates_args=(), device_types="cuda")
+def convlstm_backward_state(dpred: Optional[Tensor], dseq: Optional[Tensor], dh_T: List[Tensor], dc_T: List[Tensor],
+                            plan_id: int, generation: int, need_dx: bool, need_state: bool) -> List[Tensor]:
+    """convlstm_backward with upstream gradients of the final state (an empty tensor: none): the gradients in the order
+    of `params`, then dx when asked for, then [dh0 per layer] + [dc0 per layer] when asked for."""
+    plan = _plan(plan_id)
+    if plan.generation != generation:
+        raise RuntimeError("the activations this backward needs are gone: either a later forward() with the same shape "
+                           "overwrote the ConvLSTM workspace, or this forward was already back-propagated once (BPTT "
+                           "turns the saved gates into their gradients in place); run the forward again")
+    gw, gb, ghw, ghb = plan.backward(dpred, dseq, dh_T=_given(dh_T), dc_T=_given(dc_T))
+    grads = []
+    for l in range(plan.L):
+        grads += [gw[l], gb[l]]
+    grads += [ghw, ghb]
+    if need_dx:
+        grads.append(plan.backward_input())
+    if need_state:
+        dh0, dc0 = plan.backward_initial_state()
+        grads += dh0 + dc0
+    return grads
+
+
+@convlstm_backward_state.register_fake
+def _(dpred, dseq, dh_T, dc_T, plan_id, generation, need_dx, need_state):
+    plan = _plan(plan_id)
+    ref = dh_T[0]
+    out, cin = [], plan.C
+    for hc, k in zip(plan.hidden, plan.ksize):
+        out += [ref.new_empty((4 * hc, cin + hc, k, k)), ref.new_empty((4 * hc,))]
+        cin = hc
+    out += [ref.new_empty((1, plan.hidden[-1], 1, 1)), ref.new_empty((1,))]
+    if need_dx:
+        out.append(ref.new_empty((plan.B, plan.T, plan.C, plan.H, plan.W)))
+    if need_state:
+        out += [ref.new_empty((plan.B, hc, plan.H, plan.W)) for hc in plan.hidden] * 2
+    return out
+
+
+def _setup_context_state(ctx, inputs, output):
+    _setup_context(ctx, inputs, output)
+    ctx.set_materialize_grads(False)     # an unused output (pred, or a layer's h_T / c_T) contributes no launch
+
+
+def _backward_state_common(ctx, dpred, dseq, dh_T, dc_T, need_dx, needs_h0, needs_c0):
+    plan = _plan(ctx.plan_id)
+    need_state = any(needs_h0) or any(needs_c0)
+    if need_state and not plan.state_grad:
+        raise RuntimeError("gradient w.r.t. the initial state needs a plan made with state_grad=True (ConvLSTM.forward "
+                           "makes one when the state requires grad)")
+    empty = lambda: torch.empty(0, dtype=torch.float32, device=plan.device)
+    grads = convlstm_backward_state(dpred, dseq if plan.return_sequence else None,
+                                    [empty() if g is None else g for g in dh_T], [empty() if g is None else g for g in dc_T],
+                                    ctx.plan_id, ctx.generation, need_dx, need_state)
+    dh0 = dc0 = [None] * plan.L
+    if need_state:
+        dh0 = [g if n else None for g, n in zip(grads[-2 * plan.L:-plan.L], needs_h0)]
+        dc0 = [g if n else None for g, n in zip(grads[-plan.L:], needs_c0)]
+        del grads[-2 * plan.L:]
+    dx = grads.pop() if need_dx else None
+    return dx, grads, dh0, dc0
+
+
+def _backward_state(ctx, dpred, dseq, dh_T, dc_T):
+    plan = _plan(ctx.plan_id)
+    need_dx = bool(ctx.needs_input_grad[0])
+    if need_dx and not plan.input_grad:
+        raise RuntimeError("gradient w.r.t. the input needs a plan made with input_grad=True (ConvLSTM.forward makes one "
+                           "when x.requires_grad)")
+    dx, grads, dh0, dc0 = _backward_state_common(ctx, dpred, dseq, dh_T, dc_T, need_dx, ctx.needs_input_grad[2],
+                                                 ctx.needs_input_grad[3])
+    return dx, grads, dh0, dc0, None
+
+
+def _backward_bank_state(ctx, dpred, dseq, dh_T, dc_T):
+    _, grads, dh0, dc0 = _backward_state_common(ctx, dpred, dseq, dh_T, dc_T, False, ctx.needs_input_grad[3],
+                                                ctx.needs_input_grad[4])
+    return None, None, grads, dh0, dc0, None
+
+
+torch.library.register_autograd("nint::convlstm_forward_state", _backward_state, setup_context=_setup_context_state)
+torch.library.register_autograd("nint::convlstm_forward_bank_state", _backward_bank_state,
+                                setup_context=_setup_context_state)
+
+
 # ---- ConvLSTMCell (model.py:216-231): one fused step from an explicit state, differentiable w.r.t. x, h, c and the
 # parameters like the reference's autograd module
 @torch.library.custom_op("nint::cell_forward", mutates_args=(), device_types="cuda")
