@@ -130,6 +130,13 @@ int nint_backward_initial_state(nint_plan* plan, float* const* dh0, float* const
 /* Gradient w.r.t. the input, dx [B,T,C,H,W] fp32 (x.grad of the reference's autograd through model.py:219-220); after
  * nint_backward_bptt, plans created with NINT_FLAG_INPUT_GRAD. */
 int nint_backward_input(nint_plan* plan, float* dx, void* stream);
+/* The input gradient of a frame-bank forward, added into the frames it read: after nint_backward_bptt[_state] of a plan
+ * created with NINT_FLAG_INPUT_GRAD whose last forward was nint_forward_bank, dframes[win_start[b] + t] += dL/dx[b][t]
+ * for every (b, t).  dframes: fp32 [n_frames][C][H][W] (NCHW, the layout of nint_fuse_inputs' output), n_frames the
+ * bank's.  ACCUMULATES (several backwards add up, like .grad of a leaf).  Order: steps in increasing t, within a step
+ * samples in increasing b, so an element receives its contributions in (t, b) order -- deterministic, also for
+ * repeated window starts (no atomics).  Frames outside [0, n_frames) are skipped, as the forward reads them as zeros. */
+int nint_backward_input_bank(nint_plan* plan, float* dframes, void* stream);
 
 /* ---- ConvLSTMCell as a differentiable unit (model.py:216-231): one step from an explicit state, and its backward.
  * Plans with seq_len = 1, num_layers = 1, training = 1, NINT_FLAG_INPUT_GRAD.  nint_cell_forward = set_state + one
@@ -158,6 +165,16 @@ int nint_fuse_inputs_bank(const float* levels3d, const float* emis2d, const floa
                           const float* statics, int n_static, long long frames, int levels, int height, int width,
                           int padded_height, int padded_width, int mode, int dtype, int c_pad, int ones_lane,
                           void* bank, void* stream);
+/* Adjoint of nint_fuse_inputs for one set of shapes and one mode: dframes [frames][levels+1+n_static][Hp][Wp] (dL/d of
+ * its output) -> d_levels3d [frames][levels][H][W], d_emis2d [frames][H][W] and d_statics [n_static][H][W] (summed over
+ * every frame).  Outputs are WRITTEN, not accumulated; any may be NULL (not wanted).  Every source element sums its
+ * halo preimages (interior position, cyclic longitude copies, reflected -- or in mode 1 channel-reversed -- latitude
+ * halo rows) in fp32 in increasing padded row, then padded column (statics: over the frames in order, then rows, then
+ * columns), and the z-scored channels divide that sum by std[c] (IEEE), as autograd of (v - mean) / std does.
+ * Deterministic, no atomics.  Same error conditions as nint_fuse_inputs. */
+int nint_fuse_inputs_adjoint(const float* dframes, const float* std, long long frames, int levels, int n_static,
+                             int height, int width, int padded_height, int padded_width, int mode, float* d_levels3d,
+                             float* d_emis2d, float* d_statics, void* stream);
 
 /* ---- the rest of the training step (train.py:101-110), SURVEY.md section 8f rank 1.
  * nint_loss_mse_l1: loss = MSELoss(y, p) + L1Loss(y, p) (train.py:74-75,105) with p = pred[:, 0, y0:y1, x0:x1]

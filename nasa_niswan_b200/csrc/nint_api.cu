@@ -1197,6 +1197,19 @@ int nint_fuse_inputs_bank(const float* levels3d, const float* emis2d, const floa
   return 0;
 }
 
+int nint_fuse_inputs_adjoint(const float* dframes, const float* std, long long frames, int levels, int n_static,
+                             int height, int width, int padded_height, int padded_width, int mode, float* d_levels3d,
+                             float* d_emis2d, float* d_statics, void* stream) {
+  // same conditions as the forward: dframes stands in for its inputs and its output, std for mean and std
+  if (check_fuse_args(levels > 0 ? dframes : nullptr, dframes, dframes, std, d_statics, d_statics ? n_static : 0, frames,
+                      levels, height, width, padded_height, padded_width, mode, dframes)) return 1;
+  if (n_static < 0) return fail("nint_fuse_inputs: %d static fields", n_static);
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  LAUNCH(nullptr, K_OTHER, st, launch_fuse_inputs_adjoint(dframes, std, frames, levels, n_static, height, width, padded_height, padded_width, mode,
+                                                          levels > 0 ? d_levels3d : nullptr, d_emis2d, n_static > 0 ? d_statics : nullptr, st));
+  return 0;
+}
+
 static int check_loss_args(const float* pred, const float* y, const float* loss, const float* stats, int batch, int height,
                            int width, int crop_y0, int crop_y1, int crop_x0, int crop_x1) {
   if (!pred || !y || !loss || !stats) return fail("nint_loss_mse_l1: null argument");
@@ -1564,6 +1577,24 @@ int nint_backward_input(nint_plan* p, float* dx, void* stream) {
   for (int t = 0; t < p->T; ++t) {
     if (dgrad_raw(p, 0, t, 2, y.cin_rows, p->raw, st)) return 1;
     LAUNCH(p, K_OTHER, st, launch_unpack_raw(p->raw, dx + t * C * HW, p->B, C, p->H, p->W, y.cin_rows, static_cast<long long>(p->T) * C * HW, st));
+  }
+  return 0;
+}
+
+// the same dx_t, added into the frames of the bank the last forward read: dframes[win_start[b] + t] += dx[b][t], in
+// increasing t, then increasing b (nint.h)
+int nint_backward_input_bank(nint_plan* p, float* dframes, void* stream) {
+  if (check_ready(p)) return 1;
+  if (!p->cfg.training || !p->input_grad)
+    return fail("nint_backward_input_bank needs a training plan created with NINT_FLAG_INPUT_GRAD");
+  if (!p->bptt_done) return fail("nint_backward_input_bank before nint_backward_bptt");
+  if (!p->x_bank) return fail("nint_backward_input_bank: the last forward did not read a frame bank (nint_forward_bank)");
+  if (!dframes) return fail("nint_backward_input_bank: null dframes");
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const Layer& y = p->layer[0];
+  for (int t = 0; t < p->T; ++t) {
+    if (dgrad_raw(p, 0, t, 2, y.cin_rows, p->raw, st)) return 1;
+    LAUNCH(p, K_OTHER, st, launch_accum_frames(p->raw, dframes, p->win_start, p->B, p->cfg.in_channels, p->H, p->W, y.cin_rows, t, p->bank_frames, st));
   }
   return 0;
 }

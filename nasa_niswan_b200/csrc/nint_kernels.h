@@ -198,6 +198,10 @@ cudaError_t launch_unpack_wgrad(const float* dw_acc, const float* db_acc, float*
 // fp32 accumulator dump [B][H][W][ncols] (EPI_RAW) -> gradient tensor [B][(T)][C][H][W] fp32 (dx / dh of the cell API)
 cudaError_t launch_unpack_raw(const float* raw, float* dst, int B, int C, int H, int W, int ncols, long long dst_bstride,
                               cudaStream_t s);
+// the same dump of step t added into the frames the windows read: dframes[win_start[b] + t][C][H][W] += raw[b], samples
+// in increasing b per element (repeated starts accumulate in that order), frames outside [0, n_frames) skipped
+cudaError_t launch_accum_frames(const float* raw, float* dframes, const int* win_start, int B, int C, int H, int W,
+                                int ncols, int t, long long n_frames, cudaStream_t s);
 
 // preprocessing fusion: stack levels + emission, z-score, cyclic-longitude / reflect-latitude halo
 cudaError_t launch_fuse_inputs(const float* lev, const float* emis, const float* mean, const float* stdv,
@@ -207,6 +211,11 @@ cudaError_t launch_fuse_inputs(const float* lev, const float* emis, const float*
 cudaError_t launch_fuse_inputs_bank(int dtype, const float* lev, const float* emis, const float* mean, const float* stdv,
                                     const float* statics, int S, void* out, long long N, int L, int H, int W, int Hp, int Wp,
                                     int mode, int c_pad, int ones_lane, cudaStream_t s);
+// adjoint of launch_fuse_inputs: dframes [N][L+1+S][Hp][Wp] -> d_lev [N][L][H][W], d_emis [N][H][W], d_statics [S][H][W]
+// (summed over the frames); any output may be null
+cudaError_t launch_fuse_inputs_adjoint(const float* dframes, const float* stdv, long long N, int L, int S, int H, int W,
+                                       int Hp, int Wp, int mode, float* d_lev, float* d_emis, float* d_statics,
+                                       cudaStream_t s);
 // fused training loss MSE + L1 on the cropped prediction (value + gradient); stats = 5 floats of scratch;
 // y_index != null: the target of sample b is image y_index[b] + y_offset of y (frame bank)
 cudaError_t launch_loss_mse_l1(const float* pred, const float* y, float* dpred, float* stats, float* loss, int B, int H,

@@ -208,6 +208,87 @@ cudaError_t launch_unpack_raw(const float* raw, float* dst, int B, int C, int H,
   return cudaGetLastError();
 }
 
+// EPI_RAW dump of step t [B][HW][ncols] added into the frames the windows read, dframes[win_start[b] + t][C][HW].  A
+// block owns 32 pixels x 32 channels of the frame tensor and walks the samples in groups of kAccGroup: the group's dump
+// tiles are staged through shared memory (loads coalesced along the channels-last rows), then every thread adds them
+// into its (channel, pixel) elements (coalesced along the pixels).  A thread owns its elements for every b, so repeated
+// window starts need no atomics: the samples of a group that hit the same frame are summed into one register in
+// increasing b (the frame's first sample of the group holds it), and the frame is read and written once per group.
+constexpr int kAccGroup = 8;
+__global__ void __launch_bounds__(256) accum_frames_kernel(const float* __restrict__ raw, float* __restrict__ dframes,
+                                                           const int* __restrict__ win_start, int B, int C, int ncols,
+                                                           long long HW, int t, long long n_frames) {
+  __shared__ float tile[kAccGroup][32][33];
+  __shared__ long long s_frame[kAccGroup];   // -1: no sample, or a frame outside the bank (skipped)
+  __shared__ int s_root[kAccGroup];          // first sample of the group with the same frame (-1: skipped)
+  const long long p0 = static_cast<long long>(blockIdx.x) * 32;
+  const int c0 = blockIdx.y * 32;
+  const int tid = threadIdx.y * 32 + threadIdx.x;
+  for (int b0 = 0; b0 < B; b0 += kAccGroup) {
+    const int nb = B - b0 < kAccGroup ? B - b0 : kAccGroup;
+    if (tid < kAccGroup) {
+      long long f = -1;
+      if (tid < nb) {
+        f = static_cast<long long>(__ldg(win_start + b0 + tid)) + t;
+        if (f < 0 || f >= n_frames) f = -1;
+      }
+      s_frame[tid] = f;
+    }
+    for (int g = 0; g < nb; ++g) {
+      const float* s = raw + static_cast<long long>(b0 + g) * HW * ncols;
+      for (int r = threadIdx.y; r < 32; r += blockDim.y) {
+        const long long p = p0 + r;
+        const int c = c0 + threadIdx.x;
+        tile[g][r][threadIdx.x] = (p < HW && c < C) ? __ldg(s + p * ncols + c) : 0.f;
+      }
+    }
+    __syncthreads();
+    if (tid < kAccGroup) {
+      const long long f = s_frame[tid];
+      int root = -1;
+      if (f >= 0) {
+        root = tid;
+        for (int h = 0; h < tid; ++h)
+          if (s_frame[h] == f) { root = h; break; }
+      }
+      s_root[tid] = root;
+    }
+    __syncthreads();
+    const long long p = p0 + threadIdx.x;
+#pragma unroll
+    for (int r0 = 0; r0 < 32; r0 += 8) {
+      const int r = r0 + threadIdx.y;
+      const int c = c0 + r;
+      if (c < C && p < HW) {
+        float acc[kAccGroup];
+#pragma unroll
+        for (int g = 0; g < kAccGroup; ++g)
+          acc[g] = s_root[g] == g ? dframes[(s_frame[g] * C + c) * HW + p] : 0.f;
+#pragma unroll
+        for (int g = 0; g < kAccGroup; ++g) {
+          const float v = tile[g][threadIdx.x][r];
+          const int root = s_root[g];
+#pragma unroll
+          for (int h = 0; h <= g; ++h)
+            if (root == h) acc[h] += v;
+        }
+#pragma unroll
+        for (int g = 0; g < kAccGroup; ++g)
+          if (s_root[g] == g) dframes[(s_frame[g] * C + c) * HW + p] = acc[g];
+      }
+    }
+    __syncthreads();
+  }
+}
+
+cudaError_t launch_accum_frames(const float* raw, float* dframes, const int* win_start, int B, int C, int H, int W,
+                                int ncols, int t, long long n_frames, cudaStream_t s) {
+  const long long HW = static_cast<long long>(H) * W;
+  dim3 grid(static_cast<unsigned>((HW + 31) / 32), (C + 31) / 32), block(32, 8);
+  accum_frames_kernel<<<grid, block, 0, s>>>(raw, dframes, win_start, B, C, ncols, HW, t, n_frames);
+  return cudaGetLastError();
+}
+
 __global__ void nchw_to_nhwc_f32_kernel(const float* __restrict__ src, float* __restrict__ dst, int C, int c_pad, long long HW) {
   __shared__ float tile[32][33];
   const int b = blockIdx.z;
@@ -733,6 +814,108 @@ cudaError_t launch_fuse_inputs_bank(int dtype, const float* lev, const float* em
   if (dtype == NINT_BF16)
     return fuse_bank<__nv_bfloat16>(lev, emis, mean, stdv, statics, S, reinterpret_cast<__nv_bfloat16*>(out), N, L, H, W, Hp, Wp, mode, c_pad, ones_lane, s);
   return fuse_bank<float>(lev, emis, mean, stdv, statics, S, reinterpret_cast<float*>(out), N, L, H, W, Hp, Wp, mode, c_pad, ones_lane, s);
+}
+
+// ------------------------------------------------------------------------------------------
+// Adjoint of the fusion (PLANAR layout): every source element gathers the padded positions fuse_kernel copied it to
+// -- at most three rows (the upper halo row, the interior row, the lower halo row; in mode 1 the halo rows hold the
+// element in channel C-1-c) times at most three columns (the interior column and its cyclic copies left and right) --
+// and sums them in fp32 in increasing padded row, then padded column; z-scored channels then take one IEEE division by
+// std (autograd of (v - mean) / std).  No atomics, nothing depends on the launch shape.
+// Threads: one per (static channel, source pixel), running over the frames in order (one fp32 sum in frame, row,
+// column order: d_statics is summed over every frame), then one per (frame, z-scored channel, source pixel).  The
+// static threads come first so that their long loops start first.  A warp's threads are consecutive longitudes of one
+// source row: every gathered load is a coalesced run (the cyclic wrap splits at most one).
+// ------------------------------------------------------------------------------------------
+struct AdjTaps {        // slots in increasing padded order: upper halo / interior / lower halo row; left / interior / right column
+  long long row[3];     // element offset of the preimage row in its frame: (channel * Hp + yp) * Wp
+  int col[3];
+  bool row_ok[3], col_ok[3];
+};
+
+__device__ __forceinline__ AdjTaps adj_taps(int c, int C, int ys, int xs, int H, int W, int Hp, int Wp, int top, int bot,
+                                           int left, int mode) {
+  AdjTaps a;
+  const int cf = mode == 0 ? c : C - 1 - c;   // channel of the element in the halo rows
+  const int j = mode == 0 ? H - 2 - ys : ys - (H - bot - 1);
+  a.row_ok[0] = ys >= 1 && ys <= top;         // upper halo: reflected row top - ys, or (mode 1) row ys - 1
+  a.row[0] = (static_cast<long long>(cf) * Hp + (mode == 0 ? top - ys : ys - 1)) * Wp;
+  a.row_ok[1] = true;
+  a.row[1] = (static_cast<long long>(c) * Hp + top + ys) * Wp;
+  a.row_ok[2] = j >= 0 && j < bot;            // lower halo: row top + H + j
+  a.row[2] = (static_cast<long long>(cf) * Hp + top + H + j) * Wp;
+  a.col_ok[0] = xs + left - W >= 0;
+  a.col[0] = xs + left - W;
+  a.col_ok[1] = true;
+  a.col[1] = xs + left;
+  a.col_ok[2] = xs + left + W < Wp;
+  a.col[2] = xs + left + W;
+  return a;
+}
+
+// adds the element's preimages in frame `f` (pointer to the frame) to acc, in padded row then column order; every load
+// is issued before the first add
+__device__ __forceinline__ float adj_gather(const float* __restrict__ f, const AdjTaps& a, float acc) {
+  float v[9];
+#pragma unroll
+  for (int i = 0; i < 3; ++i)
+#pragma unroll
+    for (int k = 0; k < 3; ++k) v[i * 3 + k] = (a.row_ok[i] && a.col_ok[k]) ? __ldg(f + a.row[i] + a.col[k]) : 0.f;
+#pragma unroll
+  for (int i = 0; i < 3; ++i)
+#pragma unroll
+    for (int k = 0; k < 3; ++k)
+      if (a.row_ok[i] && a.col_ok[k]) acc += v[i * 3 + k];
+  return acc;
+}
+
+__global__ void __launch_bounds__(256, 4) fuse_adjoint_kernel(const float* __restrict__ dframes, const float* __restrict__ stdv,
+                                                           long long N, int L, int S, int H, int W, int Hp, int Wp,
+                                                           int mode, float* __restrict__ d_lev,
+                                                           float* __restrict__ d_emis, float* __restrict__ d_statics) {
+  const int C = L + 1 + S;
+  const long long HW = static_cast<long long>(H) * W;
+  const long long frame = static_cast<long long>(C) * Hp * Wp;
+  const int left = (Wp - W) / 2, top = (Hp - H) / 2, bot = Hp - H - top;
+  const long long n_static = d_statics ? S * HW : 0;
+  const long long idx = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
+  if (idx < n_static) {
+    const int s = static_cast<int>(idx / HW);
+    const int pix = static_cast<int>(idx - s * HW);
+    const int ys = pix / W, xs = pix - ys * W;
+    const AdjTaps a = adj_taps(L + 1 + s, C, ys, xs, H, W, Hp, Wp, top, bot, left, mode);
+    float acc = 0.f;
+#pragma unroll 2
+    for (long long n = 0; n < N; ++n) acc = adj_gather(dframes + n * frame, a, acc);
+    d_statics[idx] = acc;       // the fusion does not z-score the static attributes
+    return;
+  }
+  const long long z = idx - n_static;
+  if (z >= N * (L + 1) * HW) return;
+  const long long pix = z % HW;
+  const long long nc = z / HW;
+  const int c = static_cast<int>(nc % (L + 1));
+  const long long n = nc / (L + 1);
+  float* out = c < L ? d_lev : d_emis;
+  if (!out) return;
+  const int ys = static_cast<int>(pix / W), xs = static_cast<int>(pix - static_cast<long long>(ys) * W);
+  const AdjTaps a = adj_taps(c, C, ys, xs, H, W, Hp, Wp, top, bot, left, mode);
+  const float g = __fdiv_rn(adj_gather(dframes + n * frame, a, 0.f), __ldg(stdv + c));
+  if (c < L) d_lev[(n * L + c) * HW + pix] = g;
+  else d_emis[n * HW + pix] = g;
+}
+
+cudaError_t launch_fuse_inputs_adjoint(const float* dframes, const float* stdv, long long N, int L, int S, int H, int W,
+                                       int Hp, int Wp, int mode, float* d_lev, float* d_emis, float* d_statics,
+                                       cudaStream_t s) {
+  const long long HW = static_cast<long long>(H) * W;
+  const long long items = (d_statics ? S * HW : 0) + ((d_lev || d_emis) ? N * (L + 1) * HW : 0);
+  const long long blocks = (items + 255) / 256;
+  if (blocks <= 0) return cudaSuccess;
+  if (blocks > 0x7fffffffLL) return cudaErrorInvalidValue;
+  fuse_adjoint_kernel<<<static_cast<unsigned>(blocks), 256, 0, s>>>(dframes, stdv, N, L, S, H, W, Hp, Wp, mode, d_lev,
+                                                                   d_emis, d_statics);
+  return cudaGetLastError();
 }
 
 // ------------------------------------------------------------------------------------------

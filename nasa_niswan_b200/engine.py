@@ -187,6 +187,7 @@ class Plan:
             raise TypeError("bf16 inputs need precision='bf16' (a tf32 plan would lose input precision)")
         x = x.detach().contiguous()
         self._initial_state(state)
+        self._keep = None                   # no frame bank behind this forward
         pred, seq = self._outputs()
         with _lib.on_device(self.device):
             _lib.check(self.lib.nint_forward_ex(self._h, _ptr(x), _lib.X_BF16 if x.dtype == torch.bfloat16 else _lib.X_FP32,
@@ -319,6 +320,18 @@ class Plan:
             _lib.check(self.lib.nint_backward_input(self._h, _ptr(dx), self._stream()), "nint_backward_input")
         return dx
 
+    def backward_input_bank(self, dframes: torch.Tensor):
+        """Adds dL/dx of the last backward into `dframes` [N,C,H,W] fp32, the gradient of the N frames of the bank the
+        last forward read (forward_bank): dframes[win_start[b] + t] += dx[b, t], in increasing t, then b (plans made
+        with input_grad=True; call after `backward`)."""
+        if self._keep is None:
+            raise RuntimeError("backward_input_bank: the last forward did not read a frame bank (forward_bank)")
+        self._check_dev(dframes, "dframes", (self._keep[0].shape[0], self.C, self.H, self.W))
+        if not dframes.is_contiguous():
+            raise ValueError("dframes must be contiguous")
+        with _lib.on_device(self.device):
+            _lib.check(self.lib.nint_backward_input_bank(self._h, _ptr(dframes), self._stream()), "nint_backward_input_bank")
+
     # ---- ConvLSTMCell as a differentiable unit (plans with T = 1, L = 1)
     def cell_forward(self, x, h, c):
         shape = (self.B, self.hidden[0], self.H, self.W)
@@ -327,6 +340,7 @@ class Plan:
         self._check_dev(c, "c", shape)
         h_out = torch.empty(shape, dtype=torch.float32, device=self.device)
         c_out = torch.empty(shape, dtype=torch.float32, device=self.device)
+        self._keep = None
         with _lib.on_device(self.device):
             _lib.check(self.lib.nint_cell_forward(self._h, _ptr(x.detach().contiguous()), _ptr(h.detach().contiguous()),
                                                   _ptr(c.detach().contiguous()), _ptr(h_out), _ptr(c_out), self._stream()),

@@ -197,14 +197,15 @@ class ConvLSTM(nn.Module):
         return (hidden_state is not None and torch.is_grad_enabled() and
                 any(t is not None and t.requires_grad for pair in hidden_state for t in pair))
 
-    def _stateful(self, op, inputs, plan, hidden_state, return_state):
-        """the *_state op from `hidden_state`; the result as forward returns it"""
+    def _stateful(self, op, inputs, plan, hidden_state, return_state, extra=()):
+        """the *_state op from `hidden_state` (`extra`: arguments between c0 and plan_id); the result as forward
+        returns it"""
         plan.check_state(hidden_state)
         pairs = hidden_state if hidden_state is not None else [(None, None)] * self.num_layers
         empty = torch.empty(0, dtype=torch.float32, device=plan.device)     # the ops' stand-in for a zero state
         h0 = [empty if h is None else h for h, _ in pairs]
         c0 = [empty if c is None else c for _, c in pairs]
-        pred, seq, hT, cT = op(*inputs, self._params(), h0, c0, ops.register_plan(plan))
+        pred, seq, hT, cT = op(*inputs, self._params(), h0, c0, *extra, ops.register_plan(plan))
         out = (pred, seq) if self.return_sequence else pred
         return (out, list(zip(hT, cT))) if return_state else out
 
@@ -229,16 +230,23 @@ class ConvLSTM(nn.Module):
     def forward_windows(self, bank, win_start, seq_len, hidden_state=None, return_state=False):
         """bank: preprocess.FrameBank (frames resident in HBM in the operand layout); win_start: int tensor [B] of
         window start frames -> the same outputs as forward(x) with x[b] = frames[win_start[b] : win_start[b]+T].
-        hidden_state / return_state: as in forward."""
+        hidden_state / return_state: as in forward.
+        A bank that collects gradients (bank.requires_grad_()) gets dL/dx of these windows added into bank.grad by the
+        backward, under grad mode, also when no parameter requires grad."""
         params = self._params()
         starts = win_start.to(device=bank.frames.device, dtype=torch.int32).contiguous()
         bank.check_windows(win_start, seq_len)
         N, H, W, _ = bank.frames.shape
+        need_dx = torch.is_grad_enabled() and bank.requires_grad
         state_req = self._state_requires_grad(hidden_state)
-        training = state_req or self._wants_grad(params)
+        training = need_dx or state_req or self._wants_grad(params)
         plan = self.plan_for_shape(starts.shape[0], int(seq_len), H, W, bank.frames.device, training,
-                                   set_params=False, state_grad=training and (state_req or return_state))
+                                   set_params=False, input_grad=need_dx,
+                                   state_grad=training and (state_req or return_state))
         bank.check_plan(plan)
+        if need_dx:
+            return self._stateful(torch.ops.nint.convlstm_forward_bank_dx, (bank.frames, starts), plan, hidden_state,
+                                  return_state, extra=(bank._anchor, bank.grad))
         if hidden_state is not None or return_state:
             return self._stateful(torch.ops.nint.convlstm_forward_bank_state, (bank.frames, starts), plan, hidden_state,
                                   return_state)

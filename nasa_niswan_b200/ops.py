@@ -1,7 +1,7 @@
 """torch.library registration of the ConvLSTM hot path (SURVEY.md section 8b: "a thin C-ABI torch custom-op layer").
 
 `torch.ops.nint.convlstm_forward` / `convlstm_forward_bank` / `convlstm_backward` / `cell_forward` / `cell_backward`
-are ordinary dispatcher ops with CUDA-only implementations that call libnint.so through `engine.Plan`; autograd,
+(and the stateful, frame-bank input-gradient and preprocessing variants below) are ordinary dispatcher ops with CUDA-only implementations that call libnint.so through `engine.Plan`; autograd,
 fake-tensor tracing and CUDA-graph capture see them as opaque ops.  A plan (geometry, TMA descriptors, workspace with
 the BPTT state) is host-side state the ops cannot carry in their arguments, so it travels as an integer handle into a
 registry of live plans.  There is no CPU implementation on purpose: calling the ops with CPU tensors raises from the
@@ -268,6 +268,57 @@ def _backward_bank_state(ctx, dpred, dseq, dh_T, dc_T):
 torch.library.register_autograd("nint::convlstm_forward_state", _backward_state, setup_context=_setup_context_state)
 torch.library.register_autograd("nint::convlstm_forward_bank_state", _backward_bank_state,
                                 setup_context=_setup_context_state)
+
+
+# ---- a frame-bank forward whose input gradient is wanted: its backward adds dL/dx of every window into the gradient
+# of the bank's frames (FrameBank.grad).  `anchor` is a zero-size leaf of the bank that requires grad, so autograd
+# records the node even when no parameter or state does (sensitivity maps of a frozen model); `dframes` is the bank's
+# gradient [N,C,Hp,Wp] fp32, which the forward only hands to the backward.
+@torch.library.custom_op("nint::convlstm_forward_bank_dx", mutates_args=(), device_types="cuda")
+def convlstm_forward_bank_dx(frames: Tensor, win_start: Tensor, params: List[Tensor], h0: List[Tensor],
+                             c0: List[Tensor], anchor: Tensor, dframes: Tensor,
+                             plan_id: int) -> Tuple[Tensor, Tensor, List[Tensor], List[Tensor]]:
+    """convlstm_forward_bank_state on a plan made with input_grad=True; returns (pred, seq, [h_T], [c_T])."""
+    plan = _plan(plan_id)
+    _set_params(plan, params)
+    pred, seq = plan.forward_bank(frames, win_start, list(zip(_given(h0), _given(c0))))
+    return _state_outputs(plan, pred, seq)
+
+
+@convlstm_forward_bank_dx.register_fake
+def _(frames, win_start, params, h0, c0, anchor, dframes, plan_id):
+    plan = _plan(plan_id)
+    return _state_fakes(frames, plan, win_start.shape[0], frames.shape[1], frames.shape[2], plan.T)
+
+
+@torch.library.custom_op("nint::bank_input_grad_", mutates_args=("dframes",), device_types="cuda")
+def bank_input_grad_(dframes: Tensor, plan_id: int, generation: int) -> None:
+    """dframes[win_start[b] + t] += dL/dx[b, t] of the plan's last backward, which must be the one that took the plan to
+    `generation` (nint_backward_input_bank)."""
+    plan = _plan(plan_id)
+    if plan.generation != generation:
+        raise RuntimeError("the frame-bank input gradient must follow the backward of its forward at once")
+    plan.backward_input_bank(dframes)
+
+
+@bank_input_grad_.register_fake
+def _(dframes, plan_id, generation):
+    return None
+
+
+def _setup_context_bank_dx(ctx, inputs, output):
+    _setup_context_state(ctx, inputs, output)
+    ctx.dframes = inputs[6]      # not saved for backward: later backwards mutate it, and this one adds to it
+
+
+def _backward_bank_dx(ctx, dpred, dseq, dh_T, dc_T):
+    _, grads, dh0, dc0 = _backward_state_common(ctx, dpred, dseq, dh_T, dc_T, False, ctx.needs_input_grad[3],
+                                                ctx.needs_input_grad[4])
+    bank_input_grad_(ctx.dframes, ctx.plan_id, ctx.generation + 1)     # the backward above bumped the generation once
+    return None, None, grads, dh0, dc0, None, None, None
+
+
+torch.library.register_autograd("nint::convlstm_forward_bank_dx", _backward_bank_dx, setup_context=_setup_context_bank_dx)
 
 
 # ---- ConvLSTMCell (model.py:216-231): one fused step from an explicit state, differentiable w.r.t. x, h, c and the

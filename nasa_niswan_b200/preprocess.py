@@ -2,10 +2,10 @@
 sample (dataset.py:520-537 stack + z-score, dataset.py:67-98 cyclic-longitude / reflect-latitude halo), as one
 memory-bound kernel (`nint_fuse_inputs`).  The README's 20-level module has no shipped code: for more than one
 level this follows the single-level code path and its parity is unpinned upstream (SURVEY.md section 0)."""
-import ctypes
-from typing import Optional, Tuple
+from typing import Dict, Optional, Tuple
 
 import torch
+from torch import Tensor
 
 from . import _lib
 
@@ -27,7 +27,11 @@ class FrameBank:
     E33OMA90D_CRNN keeps the whole file in RAM and cuts windows with sliding_window_view): `frames` [N, Hp, Wp, c_pad]
     of bf16 (bf16 models) or tf32-rounded fp32, and optionally `targets` [N, Hy, Wy] fp32.  A training batch is then B
     window-start indices: sample b = frames[i_b : i_b + T], target = targets[i_b + T - 1] (dataset.py:600-601); the
-    kernels read both through those indices, so a step uploads 4 B bytes instead of B windows."""
+    kernels read both through those indices, so a step uploads 4 B bytes instead of B windows.
+
+    Input gradients: after `requires_grad_()`, every `ConvLSTM.forward_windows` over the bank under grad mode adds, on
+    backward, dL/dx of its windows into `grad` [N, C, Hp, Wp] fp32 (frame win_start[b] + t gets sample b's step t), like
+    `.grad` of a leaf.  `field_grads()` takes that back through the preprocessing of `from_fields` to the raw fields."""
 
     def __init__(self, frames: torch.Tensor, channels: int, precision: str = "bf16", targets: Optional[torch.Tensor] = None):
         if precision not in _DTYPES:
@@ -42,6 +46,39 @@ class FrameBank:
                 raise ValueError("targets must be [N, Hy, Wy] fp32 on the frames' device")
             targets = targets.contiguous()
         self.targets = targets
+        self.grad: Optional[Tensor] = None
+        self._anchor: Optional[Tensor] = None   # zero-size leaf that requires grad: it puts the forward into the graph
+        self._fields: Optional[dict] = None      # from_fields: what the preprocessing adjoint needs (field_grads)
+
+    def requires_grad_(self, flag: bool = True) -> "FrameBank":
+        """Collect dL/d(frames) in `grad`, fp32 [N, C, Hp, Wp] zeros (flag=False drops it).  That is 4*C*Hp*Wp bytes per
+        frame: 497 MB for 384 frames of 21 x 100 x 154, 22.7 GB for a year of half-hourly frames.  The bank's own
+        rounding to bf16 / tf32 counts as identity (straight through), as it does for x.grad of explicit windows."""
+        if flag and self.grad is None:
+            N, Hp, Wp, _ = self.frames.shape
+            self.grad = torch.zeros((N, self.channels, Hp, Wp), dtype=torch.float32, device=self.frames.device)
+            self._anchor = torch.zeros(0, dtype=torch.float32, device=self.frames.device, requires_grad=True)
+        elif not flag:
+            self.grad = self._anchor = None
+        return self
+
+    @property
+    def requires_grad(self) -> bool:
+        return self.grad is not None
+
+    def zero_grad(self):
+        if self.grad is not None:
+            self.grad.zero_()
+
+    def field_grads(self) -> Dict[str, Optional[Tensor]]:
+        """`grad` taken back through the preprocessing of `from_fields` (nint_fuse_inputs_adjoint): {"levels3d"
+        [N, L, H, W], "emis2d" [N, H, W], "statics" [S, H, W] summed over the frames, or None without statics}."""
+        if self._fields is None:
+            raise RuntimeError("field_grads needs a bank built by FrameBank.from_fields; for frames given directly, "
+                               "bank.grad is dL/dx of those frames")
+        if self.grad is None:
+            raise RuntimeError("field_grads: the bank collects no gradient; call requires_grad_() before the forward")
+        return fuse_inputs_adjoint(self.grad, **self._fields)
 
     def __len__(self):
         return self.frames.shape[0]
@@ -103,7 +140,9 @@ class FrameBank:
                                                          _lib.ptr(statics) if S else None, S, lead[0], L, H, W, Hp, Wp,
                                                          MODES[mode], code, c_pad, ones, _lib.ptr(frames),
                                                          _lib.stream_ptr(levels3d.device)), "nint_fuse_inputs_bank")
-        return cls(frames, C, precision, targets)
+        bank = cls(frames, C, precision, targets)
+        bank._fields = _adjoint_record(std, L, S, H, W, mode)
+        return bank
 
 
 def _check_fuse_args(levels3d, emis2d, mean, std, target_hw, mode, statics):
@@ -148,8 +187,18 @@ def fuse_inputs(levels3d: torch.Tensor, emis2d: torch.Tensor, mean: torch.Tensor
     """levels3d [..., L, H, W], emis2d [..., H, W] (same leading dims, e.g. [T] or [B, T]), mean/std [L+1],
     statics [S, H, W] (already z-scored, `normalise_static_attributes`; appended to every frame as channels L+1..,
     dataset.py:532-533) -> [..., L+1+S, Hp, Wp] fp32 on the same CUDA device.  `target_hw=None` keeps the grid size
-    (no halo)."""
+    (no halo).  Differentiable w.r.t. levels3d, emis2d and statics (not mean / std) when one of them requires grad:
+    the backward is nint_fuse_inputs_adjoint."""
     lead, L, H, W, S, Hp, Wp, statics = _check_fuse_args(levels3d, emis2d, mean, std, target_hw, mode, statics)
+    if torch.is_grad_enabled() and any(t is not None and t.requires_grad for t in (levels3d, emis2d, statics)):
+        return torch.ops.nint.fuse_inputs(levels3d, emis2d, mean, std, statics, Hp, Wp, MODES[mode])
+    return _fuse_planar(levels3d, emis2d, mean, std, statics, Hp, Wp, MODES[mode])
+
+
+def _fuse_planar(levels3d, emis2d, mean, std, statics, Hp, Wp, mode):
+    lead = tuple(levels3d.shape[:-3])
+    L, H, W = levels3d.shape[-3:]
+    S = 0 if statics is None else statics.shape[0]
     frames = 1
     for d in lead:
         frames *= d
@@ -158,6 +207,73 @@ def fuse_inputs(levels3d: torch.Tensor, emis2d: torch.Tensor, mean: torch.Tensor
     with _lib.on_device(levels3d.device):
         _lib.check(_lib.load().nint_fuse_inputs(vp(levels3d.contiguous()), vp(emis2d.contiguous()), vp(mean.contiguous()),
                                                 vp(std.contiguous()), vp(statics) if S else None, S, frames, L, H, W, Hp, Wp,
-                                                MODES[mode], vp(out), _lib.stream_ptr(levels3d.device)),
+                                                mode, vp(out), _lib.stream_ptr(levels3d.device)),
                    "nint_fuse_inputs")
+    return out
+
+
+@torch.library.custom_op("nint::fuse_inputs", mutates_args=(), device_types="cuda")
+def _fuse_inputs_op(levels3d: Tensor, emis2d: Tensor, mean: Tensor, std: Tensor, statics: Optional[Tensor],
+                    padded_height: int, padded_width: int, mode: int) -> Tensor:
+    """fuse_inputs as a differentiable op (nint_fuse_inputs; backward nint_fuse_inputs_adjoint)"""
+    return _fuse_planar(levels3d.detach(), emis2d.detach(), mean.detach(), std.detach(),
+                        None if statics is None else statics.detach(), padded_height, padded_width, mode)
+
+
+@_fuse_inputs_op.register_fake
+def _(levels3d, emis2d, mean, std, statics, padded_height, padded_width, mode):
+    C = levels3d.shape[-3] + 1 + (0 if statics is None else statics.shape[0])
+    return levels3d.new_empty(tuple(levels3d.shape[:-3]) + (C, padded_height, padded_width))
+
+
+def _fuse_setup_context(ctx, inputs, output):
+    levels3d, _, _, std, statics, _, _, mode = inputs
+    ctx.std, ctx.mode, ctx.lead = std, mode, tuple(levels3d.shape[:-3])
+    ctx.shape = (levels3d.shape[-3], 0 if statics is None else statics.shape[0]) + tuple(levels3d.shape[-2:])
+
+
+def _fuse_backward(ctx, dout):
+    L, S, H, W = ctx.shape
+    need = ctx.needs_input_grad
+    mode = next(k for k, v in MODES.items() if v == ctx.mode)
+    g = fuse_inputs_adjoint(dout.reshape((-1,) + tuple(dout.shape[-3:])), ctx.std, L, S, H, W, mode,
+                            want=(need[0], need[1], need[4]))
+    dl = None if g["levels3d"] is None else g["levels3d"].reshape(ctx.lead + (L, H, W))
+    de = None if g["emis2d"] is None else g["emis2d"].reshape(ctx.lead + (H, W))
+    return dl, de, None, None, g["statics"], None, None, None
+
+
+torch.library.register_autograd("nint::fuse_inputs", _fuse_backward, setup_context=_fuse_setup_context)
+
+
+def _adjoint_record(std, levels, n_static, height, width, mode):
+    """what fuse_inputs_adjoint needs besides the gradient: kept by banks built from raw fields"""
+    return dict(std=std.detach().contiguous().clone(), levels=int(levels), n_static=int(n_static), height=int(height),
+                width=int(width), mode=mode)
+
+
+def fuse_inputs_adjoint(dframes: Tensor, std: Tensor, levels: int, n_static: int, height: int, width: int,
+                        mode: str = "reflect", want=(True, True, True)) -> Dict[str, Optional[Tensor]]:
+    """Adjoint of `fuse_inputs` (nint_fuse_inputs_adjoint): dframes [N, levels+1+n_static, Hp, Wp] fp32 ->
+    {"levels3d" [N, levels, H, W], "emis2d" [N, H, W], "statics" [n_static, H, W] summed over the N frames} (None
+    where `want` says no, and for statics when there are none).  Every source element sums its halo copies in fp32 in
+    padded row-major order, then the z-scored channels divide by std."""
+    if mode not in MODES:
+        raise ValueError(f"mode must be one of {sorted(MODES)}")
+    C = levels + 1 + n_static
+    if not dframes.is_cuda or dframes.dtype != torch.float32 or dframes.dim() != 4 or dframes.shape[1] != C:
+        raise ValueError(f"dframes must be a CUDA fp32 tensor [N, {C}, Hp, Wp]")
+    if not std.is_cuda or std.device != dframes.device or std.dtype != torch.float32 or std.numel() != levels + 1:
+        raise ValueError(f"std must be {levels + 1} fp32 values on the gradient's device")
+    N, _, Hp, Wp = dframes.shape
+    new = lambda *shape: torch.empty(shape, dtype=torch.float32, device=dframes.device)
+    out = {"levels3d": new(N, levels, height, width) if want[0] else None,
+           "emis2d": new(N, height, width) if want[1] else None,
+           "statics": new(n_static, height, width) if want[2] and n_static > 0 else None}
+    vp = _lib.ptr
+    with _lib.on_device(dframes.device):
+        _lib.check(_lib.load().nint_fuse_inputs_adjoint(vp(dframes.detach().contiguous()), vp(std.contiguous()), N, levels,
+                                                        n_static, height, width, Hp, Wp, MODES[mode], vp(out["levels3d"]),
+                                                        vp(out["emis2d"]), vp(out["statics"]),
+                                                        _lib.stream_ptr(dframes.device)), "nint_fuse_inputs_adjoint")
     return out

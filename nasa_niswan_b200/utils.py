@@ -126,3 +126,25 @@ def sensitivity_sweep(dataloader, model, num_features: int, perturbation: float 
                 chunks[i].append((pred[:, 0] * y_std + y_mean).cpu())
                 X[:, :, i] = saved
     return torch.stack([torch.cat(c, dim=0) for c in chunks], dim=0)
+
+
+def input_sensitivity(model, bank, win_start, seq_len: int,
+                      crop: Optional[Tuple[int, int, int, int]] = (5, 95, 5, 149), y_std: float = 1.0):
+    """The gradient counterpart of `sensitivity_sweep`: d(sum of the de-normalised, cropped predictions of the windows
+    `win_start`) / d(inputs) in one forward and one backward, at every pixel, channel and lag instead of one +5 %
+    perturbation per feature.  Returns `bank.field_grads()` for banks built by `FrameBank.from_fields` (gradients w.r.t.
+    the raw levels, emission and static fields), else dL/d(frames) [N, C, Hp, Wp].  The bank's own gradient state is
+    left as it was, and no parameter gets a .grad."""
+    saved = bank.grad, bank._anchor
+    bank.grad = bank._anchor = None
+    try:
+        bank.requires_grad_()
+        with torch.enable_grad():
+            out = model.forward_windows(bank, win_start, seq_len)
+            pred = out[0] if isinstance(out, tuple) else out
+            if crop is not None:
+                pred = pred[:, :, crop[0]:crop[1], crop[2]:crop[3]]
+            torch.autograd.grad(pred.sum() * y_std, bank._anchor, allow_unused=True)
+        return bank.field_grads() if bank._fields is not None else bank.grad
+    finally:
+        bank.grad, bank._anchor = saved
