@@ -50,10 +50,15 @@ typedef struct nint_config {
  * NINT_FLAG_INPUT_GRAD: training plans also keep what nint_backward_input / nint_cell_backward need (the reference's
  * autograd yields x.grad and the gradient w.r.t. an explicit initial state, model.py:216-231).
  * NINT_FLAG_STATE_GRAD: training plans also keep what nint_backward_bptt_state / nint_backward_initial_state need (per
- * layer an fp32 [B,H,W,hc] buffer for dL/dh_T, and the dgrad scratch of dL/dh0). */
+ * layer an fp32 [B,H,W,hc] buffer for dL/dh_T, and the dgrad scratch of dL/dh0).
+ * NINT_FLAG_TANGENT: training plans also keep what nint_forward_tangent[_bank] needs (the input tangent
+ * [T,B,H,W,cx_pad] in the operand format, per layer a 2-slot dh ring [2,B,H,W,hc_pad] of the operand format and a dc
+ * buffer [B,H,W,hc] fp32, and one fp32 [B,H,W,4*max hc] dump of the tangent gate GEMM).  Plans without it have the
+ * same workspace and issue the same launches. */
 #define NINT_FLAG_DETERMINISTIC 1
 #define NINT_FLAG_INPUT_GRAD 2
 #define NINT_FLAG_STATE_GRAD 4
+#define NINT_FLAG_TANGENT 8
 #define NINT_X_FP32 0
 #define NINT_X_BF16 1
 
@@ -137,6 +142,27 @@ int nint_backward_input(nint_plan* plan, float* dx, void* stream);
  * samples in increasing b, so an element receives its contributions in (t, b) order -- deterministic, also for
  * repeated window starts (no atomics).  Frames outside [0, n_frames) are skipped, as the forward reads them as zeros. */
 int nint_backward_input_bank(nint_plan* plan, float* dframes, void* stream);
+
+/* ---- tangent-linear model: forward-mode derivative (J v) of the last forward w.r.t. its input windows and its initial
+ * state, at fixed parameters.  Per step and layer: da_t = W (*) [dx_t, dh_{t-1}] (no bias), then the cell's
+ * linearisation at the gates the forward saved, dc_t = f dc_{t-1} + c_{t-1} df + g di + i dg and
+ * dh_t = tanh(c_t) do + o (1 - tanh^2(c_t)) dc_t; dpred = head_w . dh_T, dseq[:, t] = head_w . dh_t (no head bias).
+ * The gates are the saved operand-format values BPTT uses too; dh_t enters the next GEMM rounded to the operand format
+ * like h_t.  Training plans created with NINT_FLAG_TANGENT, after nint_forward (explicit windows) and before a backward
+ * (BPTT consumes the saved gates).  G, c and h of the forward stay intact: several tangents and then one backward of
+ * the same forward may follow.
+ * dx: [B,T,C,H,W] fp32 or bf16 (dx_dtype = NINT_X_*; bf16 on bf16 plans only), or NULL = zero input tangent.
+ * dh0[l], dc0[l]: tangent of layer l's initial state [B,Hc_l,H,W] fp32 (host arrays of L device pointers; either array
+ * and any entry may be NULL = zero).  Outputs: dpred [B,1,H,W], dseq [B,T,H,W] (return_sequence plans), dh_T[l], dc_T[l]
+ * [B,Hc_l,H,W] fp32 -- all WRITTEN, any may be NULL (host arrays as for dh0). */
+int nint_forward_tangent(nint_plan* plan, const void* dx, int dx_dtype, const float* const* dh0, const float* const* dc0,
+                         float* dpred, float* dseq, float* const* dh_T, float* const* dc_T, void* stream);
+/* The same after nint_forward_bank: dbank [n_frames][H][W][c_pad] holds the tangent frames in the bank's layout with
+ * the constant-1 lane 0 (nint_pack_frames / nint_fuse_inputs_bank with ones_lane = -1), n_frames the bank's, and the
+ * windows are cut at the forward's win_start. */
+int nint_forward_tangent_bank(nint_plan* plan, const void* dbank, long long n_frames, const float* const* dh0,
+                              const float* const* dc0, float* dpred, float* dseq, float* const* dh_T,
+                              float* const* dc_T, void* stream);
 
 /* ---- ConvLSTMCell as a differentiable unit (model.py:216-231): one step from an explicit state, and its backward.
  * Plans with seq_len = 1, num_layers = 1, training = 1, NINT_FLAG_INPUT_GRAD.  nint_cell_forward = set_state + one

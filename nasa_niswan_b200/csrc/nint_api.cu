@@ -80,6 +80,9 @@ struct Layer {
   uint8_t* G = nullptr;    // [T][B][H][W][4hc] E   (training)
   float* dC = nullptr;     // [B][H][W][hc]         (training)
   float* dh_ext = nullptr; // [B][H][W][hc] upstream dL/dh_T (NINT_FLAG_STATE_GRAD)
+  uint8_t* tH = nullptr;   // NINT_FLAG_TANGENT: [2][B][H][W][hc_pad] E ring of dh (slot t & 1 = dh_{t-1})
+  float* tC = nullptr;     // NINT_FLAG_TANGENT: [B][H][W][hc] running dc
+  CUtensorMap tm_tH, tm_tH_up;   // tH as this layer's recurrent segment / as the x segment of layer l+1
   uint8_t *wx = nullptr, *wh = nullptr, *wdx = nullptr, *wdh = nullptr;
   float *bias_q = nullptr, *dw_acc = nullptr, *db_acc = nullptr;
   float* db_resid = nullptr;   // tf32 training plans: [kResidCtas][4][4hc] sums of the dgates rounding residuals (nint_kernels.h)
@@ -137,6 +140,15 @@ struct nint_plan {
   float* raw = nullptr;      // NINT_FLAG_INPUT_GRAD / _STATE_GRAD: [B][H][W][max(cx_pad0, hc0, hc_l)] fp32 dgrad dump
   float* dh_ext = nullptr;   // NINT_FLAG_INPUT_GRAD, cell plans: upstream dL/dh' as [B][H][W][hc] fp32
   float* head_part = nullptr;  // deterministic mode: per-block partial sums of the head gradient
+  // NINT_FLAG_TANGENT: input tangent [T][B][H][W][cx_pad0] E, the tangent GEMM's fp32 dump [B][H][W][4 * max hc], a zero
+  // head bias; maps over tX and over the caller's tangent bank (re-encoded when its pointer or length changes)
+  bool tangent = false;
+  uint8_t* tX = nullptr;
+  float* traw = nullptr;
+  float* tzero = nullptr;
+  CUtensorMap tm_tX, tmb_tX;
+  const void* tbank_ptr = nullptr;
+  long long tbank_frames = 0;
   unsigned* step_done = nullptr;   // [T][B] tile counters of a time-fused conv launch (ConvGemmParams::step_done)
   // consecutive time steps of a layer as ONE persistent launch whose tiles wait on the previous step's tiles of the same
   // image (ConvGemmParams::n_steps).  -1: automatic -- BPTT launches are fused while they are short (bwd_should_fuse),
@@ -344,6 +356,18 @@ size_t carve(nint_plan* p, uint8_t* base) {
   if (tr && p->input_grad) p->dh_ext = reinterpret_cast<float*>(take(npix * p->layer[0].hc * 4));
   if (tr && p->state_grad)
     for (int l = 0; l < p->L; ++l) p->layer[l].dh_ext = reinterpret_cast<float*>(take(npix * p->layer[l].hc * 4));
+  if (tr && p->tangent) {
+    p->tX = take(act_bytes(p, p->T, p->layer[0].cx_pad));
+    int max_hc = 0;
+    for (int l = 0; l < p->L; ++l) {
+      Layer& y = p->layer[l];
+      y.tH = take(act_bytes(p, 2, y.hc_pad));
+      y.tC = reinterpret_cast<float*>(take(npix * y.hc * 4));
+      max_hc = max_hc > y.hc ? max_hc : y.hc;
+    }
+    p->traw = reinterpret_cast<float*>(take(npix * 4 * max_hc * 4));
+    p->tzero = reinterpret_cast<float*>(take(16));
+  }
   return off;
 }
 
@@ -746,6 +770,7 @@ int nint_plan_create(const nint_config* cfg, nint_plan** out) {
   p->deterministic = (cfg->flags & NINT_FLAG_DETERMINISTIC) != 0;
   p->input_grad = (cfg->flags & NINT_FLAG_INPUT_GRAD) != 0;
   p->state_grad = (cfg->flags & NINT_FLAG_STATE_GRAD) != 0;
+  p->tangent = (cfg->flags & NINT_FLAG_TANGENT) != 0;
   {  // debug / A-B knobs (documented in DESIGN.md): CTA pairs on/off, experiment flags
     const char* c = getenv("NINT_CLUSTER");
     p->cluster = c ? atoi(c) : 2;
@@ -948,6 +973,17 @@ int nint_plan_bind(nint_plan* p, void* workspace, size_t bytes, void* stream) {
       if (any_pair &&
           encode_act_box(&y.tmp_G, p->dtype, y.G, 4 * y.hc, p->W, p->H, p->B, p->T, 64, tw, th, 0, CU_TENSOR_MAP_SWIZZLE_128B)) return 1;
     }
+  }
+  if (p->cfg.training && p->tangent) {   // the tangent GEMM reads its operands through the forward's box geometry
+    if (encode_act_map(&p->tm_tX, p->dtype, p->tX, p->layer[0].cx_pad, p->W, p->H, p->B, p->T, ce, tw, th, false, pad_of(0))) return 1;
+    for (int l = 0; l < p->L; ++l) {
+      Layer& y = p->layer[l];
+      if (encode_act_map(&y.tm_tH, p->dtype, y.tH, y.hc_pad, p->W, p->H, p->B, 2, ce, tw, th, false, pad_of(l))) return 1;
+      if (l + 1 < p->L &&
+          encode_act_map(&y.tm_tH_up, p->dtype, y.tH, y.hc_pad, p->W, p->H, p->B, 2, ce, tw, th, false, pad_of(l + 1))) return 1;
+    }
+    p->tbank_ptr = nullptr;
+    p->tbank_frames = 0;
   }
   p->zero_init = true;
   p->fwd_done = false;
@@ -1597,6 +1633,109 @@ int nint_backward_input_bank(nint_plan* p, float* dframes, void* stream) {
     LAUNCH(p, K_OTHER, st, launch_accum_frames(p->raw, dframes, p->win_start, p->B, p->cfg.in_channels, p->H, p->W, y.cin_rows, t, p->bank_frames, st));
   }
   return 0;
+}
+
+// ---- tangent-linear forward (nint.h nint_forward_tangent): reads the gates, c and h history of the last forward and
+// writes only the NINT_FLAG_TANGENT buffers, so the forward stays available to further tangents and to one backward
+static int tangent_check(nint_plan* p, bool bank, const float* dseq) {
+  if (check_ready(p)) return 1;
+  if (!p->cfg.training || !p->tangent)
+    return fail("nint_forward_tangent needs a training plan created with NINT_FLAG_TANGENT");
+  if (!p->fwd_done) return fail("nint_forward_tangent before nint_forward");
+  if (!p->gates_valid)
+    return fail("nint_forward_tangent: the gates saved by the last forward were already consumed by a backward (BPTT "
+                "turns them into their gradients in place); run the forward again");
+  if (bank && !p->x_bank) return fail("nint_forward_tangent_bank: the last forward did not read a frame bank (nint_forward_bank)");
+  if (!bank && p->x_bank) return fail("nint_forward_tangent: the last forward read a frame bank; use nint_forward_tangent_bank");
+  if (dseq && !p->cfg.return_sequence) return fail("dseq output requires return_sequence in the plan");
+  return 0;
+}
+
+// the T x L tangent steps once the input tangent is in place (tX packed, or the tangent bank's map encoded)
+static int tangent_steps(nint_plan* p, const float* const* dh0, const float* const* dc0, float* dpred, float* dseq,
+                         float* const* dh_T, float* const* dc_T, cudaStream_t st) {
+  const long long HW = static_cast<long long>(p->H) * p->W;
+  const long long npix = p->B * HW;
+  const Layer& top = p->layer[p->L - 1];
+  bool dh_in[NINT_MAX_LAYERS];
+  for (int l = 0; l < p->L; ++l) {
+    Layer& y = p->layer[l];
+    dh_in[l] = dh0 && dh0[l];
+    if (dh_in[l]) LAUNCH(p, K_OTHER, st, launch_pack_state(p->dtype, dh0[l], y.tH, p->B, y.hc_real, p->H, p->W, y.hc_pad, st));
+    CK(cudaMemsetAsync(y.tC, 0, static_cast<size_t>(npix) * y.hc * 4, st));
+    if (dc0 && dc0[l]) LAUNCH(p, K_OTHER, st, launch_nchw_to_nhwc_f32(dc0[l], y.tC, p->B, y.hc_real, p->H, p->W, y.hc, st));
+  }
+  for (int t = 0; t < p->T; ++t) {
+    for (int l = 0; l < p->L; ++l) {
+      Layer& y = p->layer[l];
+      const bool bank = l == 0 && p->x_bank;
+      const bool rec = t > 0 || dh_in[l];   // dh_{-1} = 0 contributes nothing: no recurrent K segment
+      // the forward's gate GEMM (its packed weights, halved i/f/o columns, shared-memory plan) over the tangent
+      // operands; EPI_RAW dumps the accumulators and adds no bias, and the tangent input's constant-1 lane is 0
+      ConvGemmParams g;
+      if (fwd_conv_params(p, l, rec, EPI_RAW, g)) return 1;
+      g.seg[0].tmap_act = l == 0 ? (bank ? p->tmb_tX : p->tm_tX) : p->layer[l - 1].tm_tH_up;
+      g.seg[0].slot = l == 0 ? t : ((t + 1) & 1);
+      g.seg[0].win_start = bank ? p->win_start : nullptr;
+      g.seg[0].bank_frames = bank ? static_cast<int>(p->tbank_frames) : 0;
+      if (rec) {
+        g.seg[1].tmap_act = y.tm_tH;
+        g.seg[1].slot = t & 1;
+      }
+      g.slot_c_in = g.slot_c_out = g.slot_h_out = g.slot_g = g.slot_c_prev = -1;
+      g.raw_out = p->traw;
+      LAUNCH(p, K_FWD, st, launch_conv_halo(EPI_RAW, p->dtype, g, p->num_sms, st));
+      LAUNCH(p, K_OTHER, st, launch_tangent_cell(p->dtype, p->traw, slot_ptr(p, y.G, t, 4 * y.hc), cslot_ptr(p, y, t),
+                                                 cslot_ptr(p, y, t + 1), y.tC, slot_ptr(p, y.tH, (t + 1) & 1, y.hc_pad),
+                                                 npix, y.hc, y.hc_pad, st));
+    }
+    if (dseq)
+      LAUNCH(p, K_OTHER, st, launch_head_fwd(p->dtype, slot_ptr(p, top.tH, (t + 1) & 1, top.hc_pad), p->head_w, p->tzero,
+                                             dseq + t * HW, HW, p->B, top.hc_real, top.hc_pad, p->T * HW, st));
+  }
+  if (dpred)
+    LAUNCH(p, K_OTHER, st, launch_head_fwd(p->dtype, slot_ptr(p, top.tH, p->T & 1, top.hc_pad), p->head_w, p->tzero, dpred,
+                                           HW, p->B, top.hc_real, top.hc_pad, HW, st));
+  for (int l = 0; l < p->L; ++l) {
+    const Layer& y = p->layer[l];
+    if (dh_T && dh_T[l])
+      LAUNCH(p, K_OTHER, st, launch_unpack_state(p->dtype, slot_ptr(p, y.tH, p->T & 1, y.hc_pad), dh_T[l], p->B, y.hc_real,
+                                                 p->H, p->W, y.hc_pad, st));
+    if (dc_T && dc_T[l]) LAUNCH(p, K_OTHER, st, launch_nhwc_to_nchw_f32(y.tC, dc_T[l], p->B, y.hc_real, p->H, p->W, y.hc, st));
+  }
+  return 0;
+}
+
+int nint_forward_tangent(nint_plan* p, const void* dx, int dx_dtype, const float* const* dh0, const float* const* dc0,
+                         float* dpred, float* dseq, float* const* dh_T, float* const* dc_T, void* stream) {
+  if (tangent_check(p, false, dseq)) return 1;
+  if (dx && dx_dtype != NINT_X_FP32 && dx_dtype != NINT_X_BF16) return fail("unknown dx dtype %d", dx_dtype);
+  if (dx && dx_dtype == NINT_X_BF16 && p->dtype != BF16) return fail("bf16 tangents need a bf16 plan");
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const Layer& y = p->layer[0];
+  if (dx)
+    LAUNCH(p, K_OTHER, st, launch_pack_input(p->dtype, dx, dx_dtype == NINT_X_BF16, p->tX, p->B, p->T, p->cfg.in_channels,
+                                             p->H, p->W, y.cx_pad, -1, st));
+  else
+    CK(cudaMemsetAsync(p->tX, 0, act_bytes(p, p->T, y.cx_pad), st));
+  return tangent_steps(p, dh0, dc0, dpred, dseq, dh_T, dc_T, st);
+}
+
+int nint_forward_tangent_bank(nint_plan* p, const void* dbank, long long n_frames, const float* const* dh0,
+                              const float* const* dc0, float* dpred, float* dseq, float* const* dh_T,
+                              float* const* dc_T, void* stream) {
+  if (tangent_check(p, true, dseq)) return 1;
+  if (!dbank) return fail("nint_forward_tangent_bank: null dbank");
+  if (n_frames != p->bank_frames)
+    return fail("nint_forward_tangent_bank: %lld tangent frames for a bank of %lld", n_frames, p->bank_frames);
+  if (reinterpret_cast<uintptr_t>(dbank) % 128) return fail("the tangent frame bank must be 128-byte aligned");
+  if (dbank != p->tbank_ptr || n_frames != p->tbank_frames) {
+    if (encode_act_map(&p->tmb_tX, p->dtype, const_cast<void*>(dbank), p->layer[0].cx_pad, p->W, p->H,
+                       static_cast<int>(n_frames), 1, p->ce, p->tile_w, p->tile_h, false, p->layer[0].k / 2)) return 1;
+    p->tbank_ptr = dbank;
+    p->tbank_frames = n_frames;
+  }
+  return tangent_steps(p, dh0, dc0, dpred, dseq, dh_T, dc_T, static_cast<cudaStream_t>(stream));
 }
 
 int nint_cell_forward(nint_plan* p, const float* x, const float* h, const float* c, float* h_out, float* c_out,

@@ -203,6 +203,13 @@ cudaError_t launch_unpack_raw(const float* raw, float* dst, int B, int C, int H,
 cudaError_t launch_accum_frames(const float* raw, float* dframes, const int* win_start, int B, int C, int H, int W,
                                 int ncols, int t, long long n_frames, cudaStream_t s);
 
+// tangent-linear cell step (nint_forward_tangent): raw = the tangent GEMM's EPI_RAW dump [npix][4*hc] (q-order, i/f/o
+// columns halved like the packed forward weights), gates = the forward's activated gates of this step [npix][4*hc] E,
+// c_prev / c_cur = c_{t-1} / c_t [npix][hc] fp32; dc [npix][hc] fp32 is updated in place, dh_out [npix][hc_pad] E gets
+// dh_t (lanes >= hc are not written)
+cudaError_t launch_tangent_cell(int dtype, const float* raw, const void* gates, const float* c_prev, const float* c_cur,
+                                float* dc, void* dh_out, long long npix, int hc, int hc_pad, cudaStream_t s);
+
 // preprocessing fusion: stack levels + emission, z-score, cyclic-longitude / reflect-latitude halo
 cudaError_t launch_fuse_inputs(const float* lev, const float* emis, const float* mean, const float* stdv,
                                const float* statics, int S, float* out, long long N, int L, int H, int W, int Hp, int Wp,

@@ -320,6 +320,75 @@ cudaError_t launch_nhwc_to_nchw_f32(const float* src, float* dst, int B, int C, 
 }
 
 // ------------------------------------------------------------------------------------------
+// Tangent-linear cell step (nint_forward_tangent), the linearisation of the forward epilogue (model.py:221-229) at the
+// saved gates:  da = the tangent GEMM's raw dump (i, f, o columns hold da/2: the packed forward weights are halved),
+//   di = i(1-i) da_i   df = f(1-f) da_f   dg = (1-g^2) da_g   do = o(1-o) da_o
+//   dc_t = f dc_{t-1} + c_{t-1} df + g di + i dg        dh_t = tanh(c_t) do + o (1 - tanh^2(c_t)) dc_t
+// One thread per (pixel, 8 hidden channels): its raw / gate columns are four 8-wide runs of the q-order row
+// (grp*64 + gate*16 + half*8), c and dc eight consecutive fp32; consecutive threads walk a pixel's channel groups, so a
+// warp reads contiguous spans.  Every load of the thread is issued before the first use.  Padded hidden channels
+// (zero weights) get raw = 0 and c = 0, so their dc and dh stay exactly 0.
+// ------------------------------------------------------------------------------------------
+template <typename E>
+__global__ void __launch_bounds__(256) tangent_cell_kernel(const float* __restrict__ raw, const E* __restrict__ gates,
+                                                           const float* __restrict__ c_prev, const float* __restrict__ c_cur,
+                                                           float* __restrict__ dc, E* __restrict__ dh_out, long long npix,
+                                                           int hc, int hc_pad) {
+  constexpr bool FAST = std::is_same<E, __nv_bfloat16>::value;   // the forward's activation variant (nint_common.cuh)
+  const int groups = hc / 8;
+  const long long total = npix * groups;
+  for (long long i = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; i < total;
+       i += static_cast<long long>(gridDim.x) * blockDim.x) {
+    const long long pix = i / groups;
+    const int c0 = static_cast<int>(i - pix * groups) * 8;
+    const int q0 = (c0 >> 4) * 64 + (c0 & 8);
+    const float* rp = raw + pix * 4 * hc + q0;
+    const E* gp = gates + pix * 4 * hc + q0;
+    const long long ci = pix * hc + c0;
+    float a[4][8], g[4][8], cp[8], cc[8], d[8];
+#pragma unroll
+    for (int k = 0; k < 4; ++k) load_elems<float, 8>(rp + k * 16, a[k]);
+#pragma unroll
+    for (int k = 0; k < 4; ++k) load_elems<E, 8>(gp + k * 16, g[k]);
+    load_elems<float, 8>(c_prev + ci, cp);
+    load_elems<float, 8>(c_cur + ci, cc);
+    load_elems<float, 8>(dc + ci, d);
+    float h[8];
+#pragma unroll
+    for (int j = 0; j < 8; ++j) {
+      const float i_ = g[0][j], f_ = g[1][j], g_ = g[2][j], o_ = g[3][j];
+      const float di = fmaf(-i_, i_, i_) * (2.f * a[0][j]);
+      const float df = fmaf(-f_, f_, f_) * (2.f * a[1][j]);
+      const float dg = fmaf(-g_, g_, 1.f) * a[2][j];
+      const float d_o = fmaf(-o_, o_, o_) * (2.f * a[3][j]);
+      const float dcv = fmaf(f_, d[j], fmaf(cp[j], df, fmaf(g_, di, i_ * dg)));
+      const float tc = act_tanh<FAST>(cc[j]);
+      d[j] = dcv;
+      // dh_t is the next GEMM's operand: tf32 rounds to nearest here (the MMA would truncate), bf16 as it is stored
+      h[j] = round_for(fmaf(tc, d_o, o_ * fmaf(-tc, tc, 1.f) * dcv), static_cast<E*>(nullptr));
+    }
+    store_elems<float, 8>(dc + ci, d);
+    store_elems<E, 8>(dh_out + pix * hc_pad + c0, h);
+  }
+}
+
+cudaError_t launch_tangent_cell(int dtype, const float* raw, const void* gates, const float* c_prev, const float* c_cur,
+                                float* dc, void* dh_out, long long npix, int hc, int hc_pad, cudaStream_t s) {
+  const long long total = npix * (hc / 8);
+  long long blocks = (total + 255) / 256;
+  if (blocks > 148 * 16) blocks = 148 * 16;
+  if (blocks <= 0) return cudaSuccess;
+  if (dtype == NINT_BF16)
+    tangent_cell_kernel<__nv_bfloat16><<<blocks, 256, 0, s>>>(raw, reinterpret_cast<const __nv_bfloat16*>(gates), c_prev,
+                                                               c_cur, dc, reinterpret_cast<__nv_bfloat16*>(dh_out), npix,
+                                                               hc, hc_pad);
+  else
+    tangent_cell_kernel<float><<<blocks, 256, 0, s>>>(raw, reinterpret_cast<const float*>(gates), c_prev, c_cur, dc,
+                                                      reinterpret_cast<float*>(dh_out), npix, hc, hc_pad);
+  return cudaGetLastError();
+}
+
+// ------------------------------------------------------------------------------------------
 // weight packing.  Reference layout: W[n][c][dy][dx], n = gate*hc + channel, c over cat(x, h)
 // (model.py:207-211,219).  Packed panel row index = ((nb*nchunks + chunk)*taps + tap)*n_tile + col,
 // each row holds one chunk (CE elements) of K.

@@ -22,7 +22,7 @@ class Plan:
     def __init__(self, batch: int, seq_len: int, height: int, width: int, in_channels: int,
                  hidden: Sequence[int], ksize: Sequence[int], precision: str = "bf16", training: bool = False,
                  return_sequence: bool = False, device=None, deterministic: bool = False, input_grad: bool = False,
-                 state_grad: bool = False):
+                 state_grad: bool = False, tangent: bool = False):
         if precision not in PRECISIONS:
             raise ValueError(f"precision must be one of {sorted(PRECISIONS)}")
         if len(hidden) != len(ksize):
@@ -37,6 +37,7 @@ class Plan:
         self.hidden, self.ksize, self.L = list(hidden), list(ksize), len(hidden)
         self.training, self.return_sequence, self.precision = bool(training), bool(return_sequence), precision
         self.deterministic, self.input_grad, self.state_grad = bool(deterministic), bool(input_grad), bool(state_grad)
+        self.tangent = bool(tangent)
         cfg = _lib.NintConfig()
         cfg.batch, cfg.seq_len, cfg.height, cfg.width = batch, seq_len, height, width
         cfg.in_channels, cfg.num_layers = in_channels, self.L
@@ -44,7 +45,7 @@ class Plan:
             cfg.hidden[i], cfg.ksize[i] = h, k
         cfg.dtype, cfg.training, cfg.return_sequence = PRECISIONS[precision], int(training), int(return_sequence)
         cfg.flags = ((_lib.FLAG_DETERMINISTIC if deterministic else 0) | (_lib.FLAG_INPUT_GRAD if input_grad else 0) |
-                     (_lib.FLAG_STATE_GRAD if state_grad else 0))
+                     (_lib.FLAG_STATE_GRAD if state_grad else 0) | (_lib.FLAG_TANGENT if tangent else 0))
         self._h = ctypes.c_void_p()
         _lib.check(self.lib.nint_plan_create(ctypes.byref(cfg), ctypes.byref(self._h)), "nint_plan_create")
         self.workspace_bytes = self.lib.nint_plan_workspace_bytes(self._h)
@@ -331,6 +332,53 @@ class Plan:
             raise ValueError("dframes must be contiguous")
         with _lib.on_device(self.device):
             _lib.check(self.lib.nint_backward_input_bank(self._h, _ptr(dframes), self._stream()), "nint_backward_input_bank")
+
+    # ---- tangent-linear model (plans made with training=True, tangent=True)
+    def _tangent_outputs(self, dh0, dc0):
+        dh0, dc0 = self._state_table(dh0, "dh0"), self._state_table(dc0, "dc0")
+        dpred, dseq = self._outputs()
+        new = lambda l: torch.empty(self._state_shape(l), dtype=torch.float32, device=self.device)
+        dh_T = [new(l) for l in range(self.L)]
+        dc_T = [new(l) for l in range(self.L)]
+        return dh0, dc0, dpred, dseq, dh_T, dc_T
+
+    def forward_tangent(self, dx: Optional[torch.Tensor] = None, dh0=None, dc0=None):
+        """J v of the last `forward` for v = (dx [B,T,C,H,W], per-layer dh0 / dc0 [B,Hc_l,H,W]; None = zero) at fixed
+        parameters: returns (dpred [B,1,H,W], dseq [B,T,H,W] or None, [(dh_T, dc_T) per layer]).  The forward's saved
+        activations are only read: more tangents, and then one `backward`, of the same forward may follow."""
+        if dx is not None:
+            self._check_dev(dx, "dx", (self.B, self.T, self.C, self.H, self.W), dtypes=(torch.float32, torch.bfloat16))
+            if dx.dtype == torch.bfloat16 and self.precision != "bf16":
+                raise TypeError("bf16 tangents need precision='bf16'")
+            dx = dx.detach().contiguous()
+        dh0, dc0, dpred, dseq, dh_T, dc_T = self._tangent_outputs(dh0, dc0)
+        with _lib.on_device(self.device):
+            _lib.check(self.lib.nint_forward_tangent(self._h, _ptr(dx),
+                                                     _lib.X_BF16 if dx is not None and dx.dtype == torch.bfloat16 else _lib.X_FP32,
+                                                     self._ptr_table(dh0), self._ptr_table(dc0), _ptr(dpred), _ptr(dseq),
+                                                     self._ptr_table(dh_T), self._ptr_table(dc_T), self._stream()),
+                       "nint_forward_tangent")
+        return dpred, dseq, list(zip(dh_T, dc_T))
+
+    def forward_tangent_bank(self, dframes: torch.Tensor, dh0=None, dc0=None):
+        """forward_tangent after `forward_bank`: dframes [N,H,W,c_pad] are the tangent frames in the bank's layout with
+        the constant-1 lane 0 (FrameBank.tangent / tangent_from_fields), N the bank's; the windows are those of the
+        forward."""
+        if self._keep is None:
+            raise RuntimeError("forward_tangent_bank: the last forward did not read a frame bank (forward_bank)")
+        frames = self._keep[0]
+        if tuple(dframes.shape) != tuple(frames.shape):
+            raise ValueError(f"tangent frames have shape {tuple(dframes.shape)}, expected {tuple(frames.shape)}")
+        self._check_dev(dframes, "tangent frames", dtypes=(frames.dtype,))
+        if not dframes.is_contiguous():
+            raise ValueError("tangent frames must be contiguous")
+        dh0, dc0, dpred, dseq, dh_T, dc_T = self._tangent_outputs(dh0, dc0)
+        with _lib.on_device(self.device):
+            _lib.check(self.lib.nint_forward_tangent_bank(self._h, _ptr(dframes), dframes.shape[0], self._ptr_table(dh0),
+                                                          self._ptr_table(dc0), _ptr(dpred), _ptr(dseq),
+                                                          self._ptr_table(dh_T), self._ptr_table(dc_T), self._stream()),
+                       "nint_forward_tangent_bank")
+        return dpred, dseq, list(zip(dh_T, dc_T))
 
     # ---- ConvLSTMCell as a differentiable unit (plans with T = 1, L = 1)
     def cell_forward(self, x, h, c):

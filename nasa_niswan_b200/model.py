@@ -165,30 +165,31 @@ class ConvLSTM(nn.Module):
             ps += [cell.conv.weight, cell.conv.bias]
         return ps + [self.conv.weight, self.conv.bias]
 
-    def plan_for_shape(self, B, T, H, W, device, training, set_params=True, input_grad=False, state_grad=False):
+    def plan_for_shape(self, B, T, H, W, device, training, set_params=True, input_grad=False, state_grad=False,
+                       tangent=False):
         device = torch.device(device)
         if device.index is None:
             device = torch.device("cuda", torch.cuda.current_device())
         det = bool(training) and _deterministic_default()
         key = (B, T, H, W, bool(training), self.return_sequence, self.precision, device, bool(input_grad),
-               bool(state_grad), det)
+               bool(state_grad), det, bool(tangent))
         hidden = [c.hidden_channels for c in self.layers]
         ks = [c.kernel_size for c in self.layers]
         plan = self._plans.get(key, lambda: Plan(B, T, H, W, self.input_channels, hidden, ks, precision=self.precision,
                                                  training=training, return_sequence=self.return_sequence,
                                                  device=device, deterministic=det, input_grad=input_grad,
-                                                 state_grad=state_grad))
+                                                 state_grad=state_grad, tangent=tangent))
         if set_params:
             for l, cell in enumerate(self.layers):
                 plan.set_weights(l, cell.conv.weight, cell.conv.bias)
             plan.set_head(self.conv.weight, self.conv.bias)
         return plan
 
-    def plan_for(self, x, training, set_params=True, input_grad=False, state_grad=False):
+    def plan_for(self, x, training, set_params=True, input_grad=False, state_grad=False, tangent=False):
         B, T, C, H, W = x.size()
         if C != self.input_channels:
             raise ValueError(f"expected {self.input_channels} input channels, got {C}")
-        return self.plan_for_shape(B, T, H, W, x.device, training, set_params, input_grad, state_grad)
+        return self.plan_for_shape(B, T, H, W, x.device, training, set_params, input_grad, state_grad, tangent)
 
     def _wants_grad(self, params):
         return torch.is_grad_enabled() and any(p.requires_grad for p in params)
@@ -252,6 +253,50 @@ class ConvLSTM(nn.Module):
                                   return_state)
         pred, seq = torch.ops.nint.convlstm_forward_bank(bank.frames, starts, params, ops.register_plan(plan))
         return (pred, seq) if self.return_sequence else pred
+
+    def _jvp_result(self, pred, seq, final, dpred, dseq, dfinal, return_state):
+        out = (pred, seq) if self.return_sequence else pred
+        dout = (dpred, dseq) if self.return_sequence else dpred
+        return ((out, final), (dout, dfinal)) if return_state else (out, dout)
+
+    @staticmethod
+    def _tangent_state(plan, state_tangent):
+        if not plan.check_state(state_tangent):
+            return None, None
+        return [h for h, _ in state_tangent], [c for _, c in state_tangent]
+
+    def jvp(self, x, dx, hidden_state=None, state_tangent=None, return_state=False):
+        """Forward-mode derivative at fixed parameters, the tangent-linear model of `forward`: returns (out, dout) with
+        `out` what forward(x, hidden_state) returns and `dout` its derivative in the direction (dx, state_tangent), like
+        torch.func.jvp's (primals_out, tangents_out).  dx [B,T,C,H,W] (None: zero); state_tangent: per layer (dh0, dc0)
+        [B,Hc_l,H,W] fp32 (None: zero, for all layers or one tensor).  return_state: ((out, [(h_T, c_T)]),
+        (dout, [(dh_T, dc_T)])).  A tangent pass costs about two to three forwards (DESIGN.md section 10, f7).  A
+        direction is exact up to the rounding of the tangent operands (bf16 / tf32 like h), not a difference of two
+        nonlinear runs.  The outputs carry no autograd graph."""
+        if not x.is_cuda:
+            raise RuntimeError("ConvLSTM runs on CUDA (B200) only: there is no CPU fallback")
+        plan = self.plan_for(x, True, tangent=True)
+        dh0, dc0 = self._tangent_state(plan, state_tangent)
+        with torch.no_grad():
+            pred, seq = plan.forward(x, hidden_state)
+            final = plan.final_state() if return_state else None
+            dpred, dseq, dfinal = plan.forward_tangent(dx, dh0, dc0)
+        return self._jvp_result(pred, seq, final, dpred, dseq, dfinal, return_state)
+
+    def jvp_windows(self, bank, win_start, seq_len, dbank, hidden_state=None, state_tangent=None, return_state=False):
+        """`jvp` over frame-bank windows (forward_windows): dbank [N,Hp,Wp,c_pad] holds the tangent of every frame of
+        `bank` in its layout (FrameBank.tangent / FrameBank.tangent_from_fields), cut at the same window starts."""
+        starts = win_start.to(device=bank.frames.device, dtype=torch.int32).contiguous()
+        bank.check_windows(win_start, seq_len)
+        N, H, W, _ = bank.frames.shape
+        plan = self.plan_for_shape(starts.shape[0], int(seq_len), H, W, bank.frames.device, True, tangent=True)
+        bank.check_plan(plan)
+        dh0, dc0 = self._tangent_state(plan, state_tangent)
+        with torch.no_grad():
+            pred, seq = plan.forward_bank(bank.frames, starts, hidden_state)
+            final = plan.final_state() if return_state else None
+            dpred, dseq, dfinal = plan.forward_tangent_bank(dbank, dh0, dc0)
+        return self._jvp_result(pred, seq, final, dpred, dseq, dfinal, return_state)
 
     def release_workspaces(self):
         self._plans.clear()

@@ -31,7 +31,10 @@ class FrameBank:
 
     Input gradients: after `requires_grad_()`, every `ConvLSTM.forward_windows` over the bank under grad mode adds, on
     backward, dL/dx of its windows into `grad` [N, C, Hp, Wp] fp32 (frame win_start[b] + t gets sample b's step t), like
-    `.grad` of a leaf.  `field_grads()` takes that back through the preprocessing of `from_fields` to the raw fields."""
+    `.grad` of a leaf.  `field_grads()` takes that back through the preprocessing of `from_fields` to the raw fields.
+
+    Tangents (forward mode): `tangent(dframes)` and `tangent_from_fields(...)` give a perturbation direction of every
+    frame in the bank's layout, which `ConvLSTM.jvp_windows` reads through the same window starts."""
 
     def __init__(self, frames: torch.Tensor, channels: int, precision: str = "bf16", targets: Optional[torch.Tensor] = None):
         if precision not in _DTYPES:
@@ -79,6 +82,55 @@ class FrameBank:
         if self.grad is None:
             raise RuntimeError("field_grads: the bank collects no gradient; call requires_grad_() before the forward")
         return fuse_inputs_adjoint(self.grad, **self._fields)
+
+    def tangent(self, dframes: torch.Tensor) -> torch.Tensor:
+        """A tangent (perturbation direction) of every frame, dframes [N, C, Hp, Wp] fp32 or bf16, packed into this bank's
+        layout with the constant-1 lane 0 -> [N, Hp, Wp, c_pad] for ConvLSTM.jvp_windows."""
+        N, Hp, Wp, _ = self.frames.shape
+        if not dframes.is_cuda or dframes.device != self.frames.device or dframes.dtype not in (torch.float32, torch.bfloat16):
+            raise ValueError("dframes must be a float32 or bfloat16 tensor on the bank's device")
+        if tuple(dframes.shape) != (N, self.channels, Hp, Wp):
+            raise ValueError(f"dframes has shape {tuple(dframes.shape)}, expected {(N, self.channels, Hp, Wp)}")
+        if dframes.dtype == torch.bfloat16 and self.precision != "bf16":
+            raise TypeError("bf16 tangents need a bf16 bank")
+        out = torch.empty_like(self.frames)
+        with _lib.on_device(dframes.device):
+            _lib.check(_lib.load().nint_pack_frames(_DTYPES[self.precision][0], _lib.ptr(dframes.contiguous()),
+                                                    _lib.X_BF16 if dframes.dtype == torch.bfloat16 else _lib.X_FP32, N,
+                                                    self.channels, Hp, Wp, self.c_pad, -1, _lib.ptr(out),
+                                                    _lib.stream_ptr(dframes.device)), "nint_pack_frames")
+        return out
+
+    def tangent_from_fields(self, d_levels3d: Optional[Tensor] = None, d_emis2d: Optional[Tensor] = None,
+                            d_statics: Optional[Tensor] = None) -> torch.Tensor:
+        """The tangent of the frames of a bank built by `from_fields` for perturbations of its raw fields (d_levels3d
+        [N, L, H, W], d_emis2d [N, H, W], d_statics [S, H, W] fp32; None = zero): the linear part of the fusion -- the
+        z-score without its mean, the same static channels, halo and mode -- written by the same kernel into the bank
+        layout with the constant-1 lane 0, rounded as the bank is.  -> [N, Hp, Wp, c_pad] for ConvLSTM.jvp_windows."""
+        if self._fields is None:
+            raise RuntimeError("tangent_from_fields needs a bank built by FrameBank.from_fields; pack frame tangents with "
+                               "FrameBank.tangent")
+        f = self._fields
+        N, Hp, Wp, _ = self.frames.shape
+        L, S, H, W, dev = f["levels"], f["n_static"], f["height"], f["width"], self.frames.device
+        zeros = lambda *shape: torch.zeros(shape, dtype=torch.float32, device=dev)
+        lev = zeros(N, L, H, W) if d_levels3d is None else d_levels3d
+        emis = zeros(N, H, W) if d_emis2d is None else d_emis2d
+        stat = (zeros(S, H, W) if d_statics is None else d_statics) if S else None
+        if d_statics is not None and not S:
+            raise ValueError("this bank has no static fields")
+        mean0 = zeros(L + 1)
+        _, _, _, _, _, _, _, stat = _check_fuse_args(lev, emis, mean0, f["std"], (Hp, Wp), f["mode"], stat)
+        if tuple(lev.shape) != (N, L, H, W):
+            raise ValueError(f"d_levels3d has shape {tuple(lev.shape)}, expected {(N, L, H, W)}")
+        out = torch.empty_like(self.frames)
+        vp = _lib.ptr
+        with _lib.on_device(dev):
+            _lib.check(_lib.load().nint_fuse_inputs_bank(vp(lev.contiguous()), vp(emis.contiguous()), vp(mean0),
+                                                         vp(f["std"]), vp(stat) if S else None, S, N, L, H, W, Hp, Wp,
+                                                         MODES[f["mode"]], _DTYPES[self.precision][0], self.c_pad, -1,
+                                                         vp(out), _lib.stream_ptr(dev)), "nint_fuse_inputs_bank")
+        return out
 
     def __len__(self):
         return self.frames.shape[0]

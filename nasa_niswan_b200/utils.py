@@ -148,3 +148,43 @@ def input_sensitivity(model, bank, win_start, seq_len: int,
         return bank.field_grads() if bank._fields is not None else bank.grad
     finally:
         bank.grad, bank._anchor = saved
+
+
+def tangent_sweep(dataloader, model, num_features: int, perturbation: float = 0.05,
+                  crop: Optional[Tuple[int, int, int, int]] = (5, 95, 5, 149), y_std: float = 1.0) -> torch.Tensor:
+    """The linearised counterpart of `sensitivity_sweep`: for every feature i, the change of the cropped, de-normalised
+    prediction when channel i of the whole window is scaled by (1 + perturbation), taken from the tangent-linear model
+    (ConvLSTM.jvp) in the direction v = perturbation * x restricted to channel i -> [num_features, N, Hc, Wc] on the
+    host.  `sensitivity_sweep` returns the perturbed predictions; this returns their first-order difference from the
+    unperturbed one, without the rounding of two nonlinear runs.  One forward per batch, then one tangent pass per
+    feature on the same forward."""
+    model.eval()
+    chunks = [[] for _ in range(num_features)]
+    device = next(model.parameters()).device
+    with torch.no_grad():
+        for X, _ in dataloader:
+            X = X.to(device, non_blocking=True)
+            plan = model.plan_for(X, True, tangent=True)
+            plan.forward(X)
+            dx = torch.zeros_like(X, dtype=torch.float32)
+            for i in range(num_features):
+                dx[:, :, i] = X[:, :, i] * perturbation
+                dpred = plan.forward_tangent(dx)[0]
+                dx[:, :, i] = 0
+                if crop is not None:
+                    dpred = dpred[:, :, crop[0]:crop[1], crop[2]:crop[3]]
+                chunks[i].append((dpred[:, 0] * y_std).cpu())
+    return torch.stack([torch.cat(c, dim=0) for c in chunks], dim=0)
+
+
+def emission_response(model, bank, win_start, seq_len: int, d_emis2d: torch.Tensor,
+                      crop: Optional[Tuple[int, int, int, int]] = (5, 95, 5, 149), y_std: float = 1.0) -> torch.Tensor:
+    """The source-oriented question the adjoint cannot answer in one pass: how the de-normalised, cropped prediction of
+    every window `win_start` changes, to first order, when the raw emission field of a bank built by
+    `FrameBank.from_fields` changes by d_emis2d [N, H, W] (e.g. +10 % over a region and a few days) -> [B, Hc, Wc].  One
+    forward and one tangent pass over the windows (FrameBank.tangent_from_fields, then ConvLSTM.jvp_windows)."""
+    _, dout = model.jvp_windows(bank, win_start, seq_len, bank.tangent_from_fields(d_emis2d=d_emis2d))
+    dpred = dout[0] if isinstance(dout, tuple) else dout
+    if crop is not None:
+        dpred = dpred[:, :, crop[0]:crop[1], crop[2]:crop[3]]
+    return dpred[:, 0] * y_std
