@@ -54,11 +54,17 @@ typedef struct nint_config {
  * NINT_FLAG_TANGENT: training plans also keep what nint_forward_tangent[_bank] needs (the input tangent
  * [T,B,H,W,cx_pad] in the operand format, per layer a 2-slot dh ring [2,B,H,W,hc_pad] of the operand format and a dc
  * buffer [B,H,W,hc] fp32, and one fp32 [B,H,W,4*max hc] dump of the tangent gate GEMM).  Plans without it have the
- * same workspace and issue the same launches. */
+ * same workspace and issue the same launches.
+ * NINT_FLAG_SECOND_ORDER: training plans also keep what nint_backward_second_order[_bank] needs, on top of what
+ * NINT_FLAG_TANGENT keeps (the flag implies it): per layer the tangent gate GEMM's fp32 dump of every step
+ * [T,B,H,W,4hc] and the tangent dc of every step [T+1,B,H,W,hc] fp32 (in place of the single dump and dc buffer), the
+ * pass's dgates and their tangents [2,B,H,W,4hc] in the operand format, its running dc and tangent [2,B,H,W,hc] fp32,
+ * and one fp32 dgrad dump [2,B,H,W,max(cin_rows, hc)]. */
 #define NINT_FLAG_DETERMINISTIC 1
 #define NINT_FLAG_INPUT_GRAD 2
 #define NINT_FLAG_STATE_GRAD 4
 #define NINT_FLAG_TANGENT 8
+#define NINT_FLAG_SECOND_ORDER 16
 #define NINT_X_FP32 0
 #define NINT_X_BF16 1
 
@@ -163,6 +169,29 @@ int nint_forward_tangent(nint_plan* plan, const void* dx, int dx_dtype, const fl
 int nint_forward_tangent_bank(nint_plan* plan, const void* dbank, long long n_frames, const float* const* dh0,
                               const float* const* dc0, float* dpred, float* dseq, float* const* dh_T,
                               float* const* dc_T, void* stream);
+
+/* ---- second-order adjoint: the Hessian-vector product H v = d/de grad_z L(z + e v) of a loss L of the last forward's
+ * outputs w.r.t. its input windows and initial state z, at fixed parameters, as forward-over-reverse.  One reverse pass
+ * carries the adjoint (eta = dL/dh_t, kappa = dL/dc_t, da_t = dL/dgates_t) and its tangent in the direction of the
+ * last nint_forward_tangent[_bank] together: per step (descending) and layer (top first), eta and its tangent are one
+ * dgrad of da_{t+1} and its tangent (+ the layer above's x part at t, + the head term u w_head / du w_head), then the
+ * cell's adjoint and its linearisation at the saved gates and tangents (DESIGN.md section 10, f8).
+ * u = dL/dpred: dpred [B,1,H,W] or dseq [B,T,H,W] (return_sequence plans; one of the two); du = its tangent
+ * d2L/dpred2 . dpred_tangent: ddpred / ddseq likewise (NULL = zero).  Outputs, any may be NULL, all WRITTEN: dx (the
+ * gradient) and ddx (H v) w.r.t. x [B,T,C,H,W] fp32; dh0[l], dc0[l], ddh0[l], ddc0[l] [B,Hc_l,H,W] fp32 w.r.t. the initial
+ * state (host arrays of L device pointers; arrays and entries may be NULL).
+ * Training plans created with NINT_FLAG_SECOND_ORDER, after nint_forward and nint_forward_tangent of that forward and
+ * before a backward.  The pass writes only its own buffers: more (tangent, second-order) pairs and then one backward of
+ * the same forward may follow. */
+int nint_backward_second_order(nint_plan* plan, const float* dpred, const float* dseq, const float* ddpred,
+                               const float* ddseq, float* dx, float* ddx, float* const* dh0, float* const* dc0,
+                               float* const* ddh0, float* const* ddc0, void* stream);
+/* The same after nint_forward_bank / nint_forward_tangent_bank: the gradient and H v w.r.t. the frames are ADDED into
+ * dframes / ddframes fp32 [n_frames][C][H][W] (either may be NULL) by the kernel nint_backward_input_bank uses: steps in
+ * DEcreasing t (the pass runs backwards in time), within a step samples in increasing b -- deterministic, no atomics. */
+int nint_backward_second_order_bank(nint_plan* plan, const float* dpred, const float* dseq, const float* ddpred,
+                                    const float* ddseq, float* dframes, float* ddframes, float* const* dh0,
+                                    float* const* dc0, float* const* ddh0, float* const* ddc0, void* stream);
 
 /* ---- ConvLSTMCell as a differentiable unit (model.py:216-231): one step from an explicit state, and its backward.
  * Plans with seq_len = 1, num_layers = 1, training = 1, NINT_FLAG_INPUT_GRAD.  nint_cell_forward = set_state + one

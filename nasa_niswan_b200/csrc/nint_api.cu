@@ -81,8 +81,15 @@ struct Layer {
   float* dC = nullptr;     // [B][H][W][hc]         (training)
   float* dh_ext = nullptr; // [B][H][W][hc] upstream dL/dh_T (NINT_FLAG_STATE_GRAD)
   uint8_t* tH = nullptr;   // NINT_FLAG_TANGENT: [2][B][H][W][hc_pad] E ring of dh (slot t & 1 = dh_{t-1})
-  float* tC = nullptr;     // NINT_FLAG_TANGENT: [B][H][W][hc] running dc
+  float* tC = nullptr;     // NINT_FLAG_TANGENT: [B][H][W][hc] running dc; NINT_FLAG_SECOND_ORDER: [T+1] slots (slot t = dc_{t-1})
   CUtensorMap tm_tH, tm_tH_up;   // tH as this layer's recurrent segment / as the x segment of layer l+1
+  // NINT_FLAG_SECOND_ORDER: the tangent gate GEMM's dump of every step [T][B][H][W][4hc] fp32; the second-order pass's
+  // dgates and their tangents [2][B][H][W][4hc] E (one step: the pass reads da_{t+1} before it writes da_t), seen by
+  // tm_sA as 2B images so one dgrad launch covers both; its running dc (kappa) and tangent [2][B][H][W][hc] fp32
+  float* tR = nullptr;
+  uint8_t* sA = nullptr;
+  float* sK = nullptr;
+  CUtensorMap tm_sA;
   uint8_t *wx = nullptr, *wh = nullptr, *wdx = nullptr, *wdh = nullptr;
   float *bias_q = nullptr, *dw_acc = nullptr, *db_acc = nullptr;
   float* db_resid = nullptr;   // tf32 training plans: [kResidCtas][4][4hc] sums of the dgates rounding residuals (nint_kernels.h)
@@ -149,6 +156,10 @@ struct nint_plan {
   CUtensorMap tm_tX, tmb_tX;
   const void* tbank_ptr = nullptr;
   long long tbank_frames = 0;
+  // NINT_FLAG_SECOND_ORDER: [2][B][H][W][max(cin_rows0, hc_l)] fp32 dgrad dump of the pass (primal, then tangent);
+  // tangent_kept: the per-step tangent dumps belong to the last forward
+  bool second_order = false, tangent_kept = false;
+  float* sraw = nullptr;
   unsigned* step_done = nullptr;   // [T][B] tile counters of a time-fused conv launch (ConvGemmParams::step_done)
   // consecutive time steps of a layer as ONE persistent launch whose tiles wait on the previous step's tiles of the same
   // image (ConvGemmParams::n_steps).  -1: automatic -- BPTT launches are fused while they are short (bwd_should_fuse),
@@ -332,7 +343,7 @@ size_t carve(nint_plan* p, uint8_t* base) {
     y.bias_q = reinterpret_cast<float*>(take(4 * y.hc * 4));
     if (tr) {
       const int nch = 4 * y.hc / p->ce;
-      y.wdx = (l > 0 || p->input_grad) ? take(static_cast<size_t>(y.taps) * nch * y.cin_rows * wrow) : nullptr;
+      y.wdx = (l > 0 || p->input_grad || p->second_order) ? take(static_cast<size_t>(y.taps) * nch * y.cin_rows * wrow) : nullptr;
       y.wdh = take(static_cast<size_t>(y.taps) * nch * y.hc * wrow);
       y.dw_acc_bytes = static_cast<size_t>(y.taps) * 4 * y.hc * y.ncols * 4;
       const size_t slices = p->deterministic ? static_cast<size_t>(y.det_splits) : 1;
@@ -362,11 +373,22 @@ size_t carve(nint_plan* p, uint8_t* base) {
     for (int l = 0; l < p->L; ++l) {
       Layer& y = p->layer[l];
       y.tH = take(act_bytes(p, 2, y.hc_pad));
-      y.tC = reinterpret_cast<float*>(take(npix * y.hc * 4));
+      y.tC = reinterpret_cast<float*>(take(npix * y.hc * 4 * (p->second_order ? p->T + 1 : 1)));
+      if (p->second_order) y.tR = reinterpret_cast<float*>(take(static_cast<size_t>(p->T) * npix * 4 * y.hc * 4));
       max_hc = max_hc > y.hc ? max_hc : y.hc;
     }
-    p->traw = reinterpret_cast<float*>(take(npix * 4 * max_hc * 4));
+    if (!p->second_order) p->traw = reinterpret_cast<float*>(take(npix * 4 * max_hc * 4));
     p->tzero = reinterpret_cast<float*>(take(16));
+  }
+  if (tr && p->second_order) {
+    int cols = p->layer[0].cin_rows;
+    for (int l = 0; l < p->L; ++l) {
+      Layer& y = p->layer[l];
+      y.sA = take(act_bytes(p, 2, 4 * y.hc));
+      y.sK = reinterpret_cast<float*>(take(2 * npix * y.hc * 4));
+      cols = cols > y.hc ? cols : y.hc;
+    }
+    p->sraw = reinterpret_cast<float*>(take(2 * npix * cols * 4));
   }
   return off;
 }
@@ -376,6 +398,10 @@ inline uint8_t* slot_ptr(const nint_plan* p, uint8_t* base, int slot, int c) {
 }
 inline float* cslot_ptr(const nint_plan* p, const Layer& y, int slot) {
   return y.Cs + static_cast<size_t>(slot) * p->B * p->H * p->W * y.hc;
+}
+// the tangent pass's dc before step `slot` (dc_{slot-1}): one running buffer, or the per-step history of second-order plans
+inline float* tc_slot(const nint_plan* p, const Layer& y, int slot) {
+  return p->second_order ? y.tC + static_cast<size_t>(slot) * p->B * p->H * p->W * y.hc : y.tC;
 }
 
 void fill_common(const nint_plan* p, const Layer& y, ConvGemmParams& g) {
@@ -770,7 +796,8 @@ int nint_plan_create(const nint_config* cfg, nint_plan** out) {
   p->deterministic = (cfg->flags & NINT_FLAG_DETERMINISTIC) != 0;
   p->input_grad = (cfg->flags & NINT_FLAG_INPUT_GRAD) != 0;
   p->state_grad = (cfg->flags & NINT_FLAG_STATE_GRAD) != 0;
-  p->tangent = (cfg->flags & NINT_FLAG_TANGENT) != 0;
+  p->second_order = (cfg->flags & NINT_FLAG_SECOND_ORDER) != 0;
+  p->tangent = (cfg->flags & NINT_FLAG_TANGENT) != 0 || p->second_order;
   {  // debug / A-B knobs (documented in DESIGN.md): CTA pairs on/off, experiment flags
     const char* c = getenv("NINT_CLUSTER");
     p->cluster = c ? atoi(c) : 2;
@@ -984,7 +1011,12 @@ int nint_plan_bind(nint_plan* p, void* workspace, size_t bytes, void* stream) {
     }
     p->tbank_ptr = nullptr;
     p->tbank_frames = 0;
+    for (int l = 0; l < p->L && p->second_order; ++l) {
+      Layer& y = p->layer[l];
+      if (encode_act_map(&y.tm_sA, p->dtype, y.sA, 4 * y.hc, p->W, p->H, 2 * p->B, 1, ce, tw, th, false, pad_of(l))) return 1;
+    }
   }
+  p->tangent_kept = false;
   p->zero_init = true;
   p->fwd_done = false;
   p->gates_valid = false;
@@ -1142,6 +1174,7 @@ static int forward_steps(nint_plan* p, float* pred, float* seq, cudaStream_t st)
   p->fwd_done = true;
   p->gates_valid = tr;
   p->bptt_done = false;
+  p->tangent_kept = false;
   return 0;
 }
 
@@ -1683,11 +1716,13 @@ static int tangent_steps(nint_plan* p, const float* const* dh0, const float* con
         g.seg[1].slot = t & 1;
       }
       g.slot_c_in = g.slot_c_out = g.slot_h_out = g.slot_g = g.slot_c_prev = -1;
-      g.raw_out = p->traw;
+      // second-order plans keep every step's dump and dc for nint_backward_second_order
+      float* raw = p->second_order ? y.tR + static_cast<size_t>(t) * npix * 4 * y.hc : p->traw;
+      g.raw_out = raw;
       LAUNCH(p, K_FWD, st, launch_conv_halo(EPI_RAW, p->dtype, g, p->num_sms, st));
-      LAUNCH(p, K_OTHER, st, launch_tangent_cell(p->dtype, p->traw, slot_ptr(p, y.G, t, 4 * y.hc), cslot_ptr(p, y, t),
-                                                 cslot_ptr(p, y, t + 1), y.tC, slot_ptr(p, y.tH, (t + 1) & 1, y.hc_pad),
-                                                 npix, y.hc, y.hc_pad, st));
+      LAUNCH(p, K_OTHER, st, launch_tangent_cell(p->dtype, raw, slot_ptr(p, y.G, t, 4 * y.hc), cslot_ptr(p, y, t),
+                                                 cslot_ptr(p, y, t + 1), tc_slot(p, y, t), tc_slot(p, y, t + 1),
+                                                 slot_ptr(p, y.tH, (t + 1) & 1, y.hc_pad), npix, y.hc, y.hc_pad, st));
     }
     if (dseq)
       LAUNCH(p, K_OTHER, st, launch_head_fwd(p->dtype, slot_ptr(p, top.tH, (t + 1) & 1, top.hc_pad), p->head_w, p->tzero,
@@ -1701,8 +1736,10 @@ static int tangent_steps(nint_plan* p, const float* const* dh0, const float* con
     if (dh_T && dh_T[l])
       LAUNCH(p, K_OTHER, st, launch_unpack_state(p->dtype, slot_ptr(p, y.tH, p->T & 1, y.hc_pad), dh_T[l], p->B, y.hc_real,
                                                  p->H, p->W, y.hc_pad, st));
-    if (dc_T && dc_T[l]) LAUNCH(p, K_OTHER, st, launch_nhwc_to_nchw_f32(y.tC, dc_T[l], p->B, y.hc_real, p->H, p->W, y.hc, st));
+    if (dc_T && dc_T[l])
+      LAUNCH(p, K_OTHER, st, launch_nhwc_to_nchw_f32(tc_slot(p, y, p->T), dc_T[l], p->B, y.hc_real, p->H, p->W, y.hc, st));
   }
+  p->tangent_kept = p->second_order;
   return 0;
 }
 
@@ -1736,6 +1773,135 @@ int nint_forward_tangent_bank(nint_plan* p, const void* dbank, long long n_frame
     p->tbank_frames = n_frames;
   }
   return tangent_steps(p, dh0, dc0, dpred, dseq, dh_T, dc_T, static_cast<cudaStream_t>(stream));
+}
+
+// ---- second-order adjoint (nint.h nint_backward_second_order): reads the forward's gates, c and h history and the
+// tangent pass's per-step dumps and dc, writes only the NINT_FLAG_SECOND_ORDER buffers and the caller's outputs
+static int soa_check(nint_plan* p, bool bank, const float* dpred, const float* dseq, const float* ddpred,
+                     const float* ddseq) {
+  if (check_ready(p)) return 1;
+  if (!p->cfg.training || !p->second_order)
+    return fail("nint_backward_second_order needs a training plan created with NINT_FLAG_SECOND_ORDER");
+  if (!p->fwd_done) return fail("nint_backward_second_order before nint_forward");
+  if (!p->gates_valid)
+    return fail("nint_backward_second_order: the gates saved by the last forward were already consumed by a backward "
+                "(BPTT turns them into their gradients in place); run the forward again");
+  if (!p->tangent_kept) return fail("nint_backward_second_order before nint_forward_tangent of the last forward");
+  if (bank && !p->x_bank)
+    return fail("nint_backward_second_order_bank: the last forward did not read a frame bank (nint_forward_bank)");
+  if (!bank && p->x_bank)
+    return fail("nint_backward_second_order: the last forward read a frame bank; use nint_backward_second_order_bank");
+  if ((dseq || ddseq) && !p->cfg.return_sequence) return fail("dseq / ddseq require return_sequence in the plan");
+  if ((dseq && dpred) || (ddseq && ddpred)) return fail("pass either dpred or dseq (fold dpred into dseq[:, T-1])");
+  return 0;
+}
+
+// EPI_RAW dgrad over the pass's dgates of both kinds (2B images: primal, then tangent) into p->sraw [2][npix][n_rows]:
+// segment i reads layer owner[i]'s dgates through its packed dgrad operand wsel[i] (2: x part, 3: h part)
+static int soa_dgrad(nint_plan* p, int l, int n_rows, int nseg, const int* owner, const int* wsel, cudaStream_t st) {
+  Layer& y = p->layer[l];
+  ConvGemmParams g;
+  fill_common(p, y, g);
+  g.B = 2 * p->B;
+  g.n_tile = n_rows;
+  g.n_blocks = 1;
+  g.cluster = (n_rows % 32 == 0) ? p->cluster : 1;
+  g.idesc = idesc_of(p->dtype, 128 * g.cluster, n_rows, 0, 0);
+  for (int i = 0; i < nseg; ++i) {
+    const Layer& o = p->layer[owner[i]];
+    g.seg[i].tmap_act = o.tm_sA; g.seg[i].wsel = wsel[i]; g.seg[i].slot = 0;
+    g.seg[i].ksize = o.k; g.seg[i].nchunks = 4 * o.hc / p->ce;
+  }
+  g.nseg = nseg;
+  g.tm_c = y.tme_C; g.tm_h = y.tme_H; g.tm_g = y.tme_G; g.tm_dc = y.tme_dC;
+  g.slot_g = g.slot_c_in = g.slot_c_out = g.slot_h_out = g.slot_c_prev = -1;
+  g.raw_out = p->sraw;
+  if (conv_halo_plan(EPI_RAW, p->dtype, g))
+    return fail("layer %d: the second-order dgrad's shared-memory plan does not fit (N %d, k %d)", l, n_rows, y.k);
+  for (int i = 0; i < nseg; ++i)
+    if (get_w_map(p, p->layer[owner[i]], wsel[i], g.n_tile, g.n_tile / g.cluster, g.seg[i].ts, &g.seg[i].tmap_w)) return 1;
+  LAUNCH(p, K_OTHER, st, launch_conv_halo(EPI_RAW, p->dtype, g, p->num_sms, st));
+  return 0;
+}
+
+// the reverse loop once the checks passed: per step t (descending) and layer l (top first) eta = one dgrad, then
+// soa_cell_kernel; layer 0's x part goes to dx / ddx (explicit windows) or is added into dframes / ddframes (bank)
+static int soa_steps(nint_plan* p, const float* dpred, const float* dseq, const float* ddpred, const float* ddseq,
+                     float* dx, float* ddx, float* dframes, float* ddframes, float* const* dh0, float* const* dc0,
+                     float* const* ddh0, float* const* ddc0, cudaStream_t st) {
+  const long long HW = static_cast<long long>(p->H) * p->W;
+  const long long npix = p->B * HW;
+  const int L = p->L, T = p->T, C = p->cfg.in_channels;
+  const Layer& y0 = p->layer[0];
+  const long long xs = static_cast<long long>(npix) * y0.cin_rows;   // tangent half of a dx dump
+  for (int l = 0; l < L; ++l) CK(cudaMemsetAsync(p->layer[l].sK, 0, 2 * static_cast<size_t>(npix) * p->layer[l].hc * 4, st));
+  for (int t = T - 1; t >= 0; --t) {
+    for (int l = L - 1; l >= 0; --l) {
+      Layer& y = p->layer[l];
+      int owner[2], wsel[2], n = 0;
+      if (t < T - 1) { owner[n] = l; wsel[n++] = 3; }       // dh_t += da_{t+1} (*) flip(W_h)
+      if (l < L - 1) { owner[n] = l + 1; wsel[n++] = 2; }   // dh_t += the layer above's x part at t
+      if (n && soa_dgrad(p, l, y.hc, n, owner, wsel, st)) return 1;
+      const float *u = nullptr, *du = nullptr;
+      long long ub = 0, dub = 0;
+      if (l == L - 1) {
+        u = dseq ? dseq + t * HW : (t == T - 1 ? dpred : nullptr);
+        du = ddseq ? ddseq + t * HW : (t == T - 1 ? ddpred : nullptr);
+        ub = dseq ? T * HW : HW;
+        dub = ddseq ? T * HW : HW;
+      }
+      LAUNCH(p, K_OTHER, st, launch_soa_cell(p->dtype, n ? p->sraw : nullptr, u, ub, du, dub, p->head_w,
+                                             slot_ptr(p, y.G, t, 4 * y.hc), y.tR + static_cast<size_t>(t) * npix * 4 * y.hc,
+                                             cslot_ptr(p, y, t), cslot_ptr(p, y, t + 1), tc_slot(p, y, t),
+                                             tc_slot(p, y, t + 1), y.sK, y.sA, npix, HW, y.hc, st));
+    }
+    if (dx || ddx || dframes || ddframes) {
+      const int owner = 0, wsel = 2;
+      if (soa_dgrad(p, 0, y0.cin_rows, 1, &owner, &wsel, st)) return 1;
+      const long long xstride = static_cast<long long>(T) * C * HW;
+      if (dx) LAUNCH(p, K_OTHER, st, launch_unpack_raw(p->sraw, dx + t * C * HW, p->B, C, p->H, p->W, y0.cin_rows, xstride, st));
+      if (ddx) LAUNCH(p, K_OTHER, st, launch_unpack_raw(p->sraw + xs, ddx + t * C * HW, p->B, C, p->H, p->W, y0.cin_rows, xstride, st));
+      if (dframes)
+        LAUNCH(p, K_OTHER, st, launch_accum_frames(p->sraw, dframes, p->win_start, p->B, C, p->H, p->W, y0.cin_rows, t,
+                                                   p->bank_frames, st));
+      if (ddframes)
+        LAUNCH(p, K_OTHER, st, launch_accum_frames(p->sraw + xs, ddframes, p->win_start, p->B, C, p->H, p->W, y0.cin_rows, t,
+                                                   p->bank_frames, st));
+    }
+  }
+  // initial state: h_{-1} enters only layer l's gate GEMM at t = 0, so dh0 = da_0 (*) flip(W_h); dc0 = kappa after t = 0
+  for (int l = 0; l < L; ++l) {
+    Layer& y = p->layer[l];
+    const long long hs = static_cast<long long>(npix) * y.hc;
+    const bool h = dh0 && dh0[l], dh = ddh0 && ddh0[l];
+    if (h || dh) {
+      const int wsel = 3;
+      if (soa_dgrad(p, l, y.hc, 1, &l, &wsel, st)) return 1;
+      const long long bs = static_cast<long long>(y.hc_real) * HW;
+      if (h) LAUNCH(p, K_OTHER, st, launch_unpack_raw(p->sraw, dh0[l], p->B, y.hc_real, p->H, p->W, y.hc, bs, st));
+      if (dh) LAUNCH(p, K_OTHER, st, launch_unpack_raw(p->sraw + hs, ddh0[l], p->B, y.hc_real, p->H, p->W, y.hc, bs, st));
+    }
+    if (dc0 && dc0[l]) LAUNCH(p, K_OTHER, st, launch_nhwc_to_nchw_f32(y.sK, dc0[l], p->B, y.hc_real, p->H, p->W, y.hc, st));
+    if (ddc0 && ddc0[l])
+      LAUNCH(p, K_OTHER, st, launch_nhwc_to_nchw_f32(y.sK + hs, ddc0[l], p->B, y.hc_real, p->H, p->W, y.hc, st));
+  }
+  return 0;
+}
+
+int nint_backward_second_order(nint_plan* p, const float* dpred, const float* dseq, const float* ddpred,
+                               const float* ddseq, float* dx, float* ddx, float* const* dh0, float* const* dc0,
+                               float* const* ddh0, float* const* ddc0, void* stream) {
+  if (soa_check(p, false, dpred, dseq, ddpred, ddseq)) return 1;
+  return soa_steps(p, dpred, dseq, ddpred, ddseq, dx, ddx, nullptr, nullptr, dh0, dc0, ddh0, ddc0,
+                   static_cast<cudaStream_t>(stream));
+}
+
+int nint_backward_second_order_bank(nint_plan* p, const float* dpred, const float* dseq, const float* ddpred,
+                                    const float* ddseq, float* dframes, float* ddframes, float* const* dh0,
+                                    float* const* dc0, float* const* ddh0, float* const* ddc0, void* stream) {
+  if (soa_check(p, true, dpred, dseq, ddpred, ddseq)) return 1;
+  return soa_steps(p, dpred, dseq, ddpred, ddseq, nullptr, nullptr, dframes, ddframes, dh0, dc0, ddh0, ddc0,
+                   static_cast<cudaStream_t>(stream));
 }
 
 int nint_cell_forward(nint_plan* p, const float* x, const float* h, const float* c, float* h_out, float* c_out,

@@ -205,10 +205,22 @@ cudaError_t launch_accum_frames(const float* raw, float* dframes, const int* win
 
 // tangent-linear cell step (nint_forward_tangent): raw = the tangent GEMM's EPI_RAW dump [npix][4*hc] (q-order, i/f/o
 // columns halved like the packed forward weights), gates = the forward's activated gates of this step [npix][4*hc] E,
-// c_prev / c_cur = c_{t-1} / c_t [npix][hc] fp32; dc [npix][hc] fp32 is updated in place, dh_out [npix][hc_pad] E gets
-// dh_t (lanes >= hc are not written)
+// c_prev / c_cur = c_{t-1} / c_t [npix][hc] fp32; dc_in = dc_{t-1}, dc_out = dc_t [npix][hc] fp32 (the same buffer:
+// updated in place), dh_out [npix][hc_pad] E gets dh_t (lanes >= hc are not written)
 cudaError_t launch_tangent_cell(int dtype, const float* raw, const void* gates, const float* c_prev, const float* c_cur,
-                                float* dc, void* dh_out, long long npix, int hc, int hc_pad, cudaStream_t s);
+                                const float* dc_in, float* dc_out, void* dh_out, long long npix, int hc, int hc_pad,
+                                cudaStream_t s);
+
+// second-order adjoint cell step (nint_backward_second_order), per (pixel, hidden channel): eta = [2][npix][hc] fp32
+// dgrad dump (dL/dh_t and its tangent; NULL = 0), u / du = dL/dpred and its tangent at this step (NULL = 0; pixel
+// b*HW + i at u[b*u_bstride + i]) times head_w [hc] (top layer only), gates / traw = the forward's activated gates and
+// the tangent GEMM's dump of this step [npix][4hc] (traw: i/f/o halved), c_prev / c_cur and dc_prev / dc_cur = c and
+// its tangent at t-1 / t [npix][hc] fp32; kappa [2][npix][hc] fp32 (dL/dc and its tangent) is updated in place,
+// da_out [2][npix][4hc] E gets dL/dgates_t and its tangent in the fused backward's q-order and scaling
+cudaError_t launch_soa_cell(int dtype, const float* eta, const float* u, long long u_bstride, const float* du,
+                            long long du_bstride, const float* head_w, const void* gates, const float* traw,
+                            const float* c_prev, const float* c_cur, const float* dc_prev, const float* dc_cur,
+                            float* kappa, void* da_out, long long npix, long long HW, int hc, cudaStream_t s);
 
 // preprocessing fusion: stack levels + emission, z-score, cyclic-longitude / reflect-latitude halo
 cudaError_t launch_fuse_inputs(const float* lev, const float* emis, const float* mean, const float* stdv,

@@ -327,13 +327,14 @@ cudaError_t launch_nhwc_to_nchw_f32(const float* src, float* dst, int B, int C, 
 // One thread per (pixel, 8 hidden channels): its raw / gate columns are four 8-wide runs of the q-order row
 // (grp*64 + gate*16 + half*8), c and dc eight consecutive fp32; consecutive threads walk a pixel's channel groups, so a
 // warp reads contiguous spans.  Every load of the thread is issued before the first use.  Padded hidden channels
-// (zero weights) get raw = 0 and c = 0, so their dc and dh stay exactly 0.
+// (zero weights) get raw = 0 and c = 0, so their dc and dh stay exactly 0.  dc_in / dc_out: the same buffer (updated in
+// place) or, on NINT_FLAG_SECOND_ORDER plans, consecutive slots of the per-step dc history the second-order pass reads.
 // ------------------------------------------------------------------------------------------
 template <typename E>
 __global__ void __launch_bounds__(256) tangent_cell_kernel(const float* __restrict__ raw, const E* __restrict__ gates,
                                                            const float* __restrict__ c_prev, const float* __restrict__ c_cur,
-                                                           float* __restrict__ dc, E* __restrict__ dh_out, long long npix,
-                                                           int hc, int hc_pad) {
+                                                           const float* dc_in, float* dc_out, E* __restrict__ dh_out,
+                                                           long long npix, int hc, int hc_pad) {
   constexpr bool FAST = std::is_same<E, __nv_bfloat16>::value;   // the forward's activation variant (nint_common.cuh)
   const int groups = hc / 8;
   const long long total = npix * groups;
@@ -352,7 +353,7 @@ __global__ void __launch_bounds__(256) tangent_cell_kernel(const float* __restri
     for (int k = 0; k < 4; ++k) load_elems<E, 8>(gp + k * 16, g[k]);
     load_elems<float, 8>(c_prev + ci, cp);
     load_elems<float, 8>(c_cur + ci, cc);
-    load_elems<float, 8>(dc + ci, d);
+    load_elems<float, 8>(dc_in + ci, d);
     float h[8];
 #pragma unroll
     for (int j = 0; j < 8; ++j) {
@@ -367,24 +368,148 @@ __global__ void __launch_bounds__(256) tangent_cell_kernel(const float* __restri
       // dh_t is the next GEMM's operand: tf32 rounds to nearest here (the MMA would truncate), bf16 as it is stored
       h[j] = round_for(fmaf(tc, d_o, o_ * fmaf(-tc, tc, 1.f) * dcv), static_cast<E*>(nullptr));
     }
-    store_elems<float, 8>(dc + ci, d);
+    store_elems<float, 8>(dc_out + ci, d);
     store_elems<E, 8>(dh_out + pix * hc_pad + c0, h);
   }
 }
 
 cudaError_t launch_tangent_cell(int dtype, const float* raw, const void* gates, const float* c_prev, const float* c_cur,
-                                float* dc, void* dh_out, long long npix, int hc, int hc_pad, cudaStream_t s) {
+                                const float* dc_in, float* dc_out, void* dh_out, long long npix, int hc, int hc_pad,
+                                cudaStream_t s) {
   const long long total = npix * (hc / 8);
   long long blocks = (total + 255) / 256;
   if (blocks > 148 * 16) blocks = 148 * 16;
   if (blocks <= 0) return cudaSuccess;
   if (dtype == NINT_BF16)
     tangent_cell_kernel<__nv_bfloat16><<<blocks, 256, 0, s>>>(raw, reinterpret_cast<const __nv_bfloat16*>(gates), c_prev,
-                                                               c_cur, dc, reinterpret_cast<__nv_bfloat16*>(dh_out), npix,
-                                                               hc, hc_pad);
+                                                               c_cur, dc_in, dc_out,
+                                                               reinterpret_cast<__nv_bfloat16*>(dh_out), npix, hc, hc_pad);
   else
-    tangent_cell_kernel<float><<<blocks, 256, 0, s>>>(raw, reinterpret_cast<const float*>(gates), c_prev, c_cur, dc,
-                                                      reinterpret_cast<float*>(dh_out), npix, hc, hc_pad);
+    tangent_cell_kernel<float><<<blocks, 256, 0, s>>>(raw, reinterpret_cast<const float*>(gates), c_prev, c_cur, dc_in,
+                                                      dc_out, reinterpret_cast<float*>(dh_out), npix, hc, hc_pad);
+  return cudaGetLastError();
+}
+
+// ------------------------------------------------------------------------------------------
+// Second-order adjoint cell step (nint_backward_second_order): the cell's adjoint (the fused backward's epilogue,
+// nint_epilogue.cuh) and its linearisation at the saved gates i, f, g, o, c_{t-1} = cp, c_t = c, tau = tanh(c) and the
+// tangent pass's da (raw, i/f/o halved), dc_{t-1} = dcp, dc_t = dc:
+//   eta = dgrad h part + u w_head              deta = its tangent + du w_head
+//   di = i(1-i) da_i  df = f(1-f) da_f  dg = (1-g^2) da_g  do = o(1-o) da_o  dtau = (1-tau^2) dc
+//   kt  = k + eta o (1-tau^2)                  dkt  = dk + deta o (1-tau^2) + eta do (1-tau^2) - 2 eta o tau dtau
+//   ai  = kt g i(1-i)                          dai  = dkt g i(1-i) + kt dg i(1-i) + kt g (1-2i) di
+//   af  = kt cp f(1-f)                         daf  = dkt cp f(1-f) + kt dcp f(1-f) + kt cp (1-2f) df
+//   ag  = kt i (1-g^2)                         dag  = dkt i (1-g^2) + kt di (1-g^2) - 2 kt i g dg
+//   ao  = eta tau o(1-o)                       dao  = deta tau o(1-o) + eta dtau o(1-o) + eta tau (1-2o) do
+//   k <- kt f                                  dk  <- dkt f + kt df
+// ai .. ao and their tangents are stored like the fused backward stores dgates over G (q-order, unscaled, rounded to
+// the operand format: the packed dgrad panels apply unchanged).  Thread layout and load order as tangent_cell_kernel;
+// padded hidden channels have zero raw, c, eta and head weight, so their outputs stay exactly 0.
+// ------------------------------------------------------------------------------------------
+template <typename E>
+__global__ void __launch_bounds__(256) soa_cell_kernel(const float* __restrict__ eta, const float* __restrict__ u,
+                                                       long long u_bstride, const float* __restrict__ du,
+                                                       long long du_bstride, const float* __restrict__ head_w,
+                                                       const E* __restrict__ gates, const float* __restrict__ traw,
+                                                       const float* __restrict__ c_prev, const float* __restrict__ c_cur,
+                                                       const float* __restrict__ dc_prev, const float* __restrict__ dc_cur,
+                                                       float* __restrict__ kappa, E* __restrict__ da_out, long long npix,
+                                                       long long HW, int hc) {
+  constexpr bool FAST = std::is_same<E, __nv_bfloat16>::value;
+  const int groups = hc / 8;
+  const long long total = npix * groups;
+  const long long nk = npix * hc;   // offset of the tangent half of eta / kappa
+  for (long long i = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; i < total;
+       i += static_cast<long long>(gridDim.x) * blockDim.x) {
+    const long long pix = i / groups;
+    const int c0 = static_cast<int>(i - pix * groups) * 8;
+    const int q0 = (c0 >> 4) * 64 + (c0 & 8);
+    const long long gi = pix * 4 * hc + q0;
+    const long long ci = pix * hc + c0;
+    float a[4][8], g[4][8], cp[8], cc[8], dcp[8], dcc[8], e[8], de[8], k[8], dk[8], w[8];
+    float uv = 0.f, duv = 0.f;
+#pragma unroll
+    for (int q = 0; q < 4; ++q) load_elems<float, 8>(traw + gi + q * 16, a[q]);
+#pragma unroll
+    for (int q = 0; q < 4; ++q) load_elems<E, 8>(gates + gi + q * 16, g[q]);
+    load_elems<float, 8>(c_prev + ci, cp);
+    load_elems<float, 8>(c_cur + ci, cc);
+    load_elems<float, 8>(dc_prev + ci, dcp);
+    load_elems<float, 8>(dc_cur + ci, dcc);
+    load_elems<float, 8>(kappa + ci, k);
+    load_elems<float, 8>(kappa + nk + ci, dk);
+    if (eta) {
+      load_elems<float, 8>(eta + ci, e);
+      load_elems<float, 8>(eta + nk + ci, de);
+    } else {
+#pragma unroll
+      for (int j = 0; j < 8; ++j) e[j] = de[j] = 0.f;
+    }
+    if (u || du) {
+      const long long b = pix / HW, r = pix - b * HW;
+      if (u) uv = __ldg(u + b * u_bstride + r);
+      if (du) duv = __ldg(du + b * du_bstride + r);
+      load_elems<float, 8>(head_w + c0, w);
+    } else {
+#pragma unroll
+      for (int j = 0; j < 8; ++j) w[j] = 0.f;
+    }
+    float o0[4][8], o1[4][8];
+#pragma unroll
+    for (int j = 0; j < 8; ++j) {
+      const float i_ = g[0][j], f_ = g[1][j], g_ = g[2][j], o_ = g[3][j];
+      const float si = fmaf(-i_, i_, i_), sf = fmaf(-f_, f_, f_), so = fmaf(-o_, o_, o_), tg = fmaf(-g_, g_, 1.f);
+      const float di = si * (2.f * a[0][j]), df = sf * (2.f * a[1][j]), dg = tg * a[2][j], d_o = so * (2.f * a[3][j]);
+      const float tau = act_tanh<FAST>(cc[j]);
+      const float tt = fmaf(-tau, tau, 1.f);
+      const float dtau = tt * dcc[j];
+      const float et = fmaf(uv, w[j], e[j]), det = fmaf(duv, w[j], de[j]);
+      const float kt = fmaf(et * o_, tt, k[j]);
+      const float dkt = fmaf(det * o_, tt, fmaf(et * d_o, tt, fmaf(-2.f * et * o_, tau * dtau, dk[j])));
+      o0[0][j] = kt * g_ * si;
+      o1[0][j] = fmaf(dkt * g_, si, fmaf(kt * dg, si, kt * g_ * fmaf(-2.f, i_, 1.f) * di));
+      o0[1][j] = kt * cp[j] * sf;
+      o1[1][j] = fmaf(dkt * cp[j], sf, fmaf(kt * dcp[j], sf, kt * cp[j] * fmaf(-2.f, f_, 1.f) * df));
+      o0[2][j] = kt * i_ * tg;
+      o1[2][j] = fmaf(dkt * i_, tg, fmaf(kt * di, tg, -2.f * kt * i_ * g_ * dg));
+      o0[3][j] = et * tau * so;
+      o1[3][j] = fmaf(det * tau, so, fmaf(et * dtau, so, et * tau * fmaf(-2.f, o_, 1.f) * d_o));
+      k[j] = kt * f_;
+      dk[j] = fmaf(dkt, f_, kt * df);
+#pragma unroll
+      for (int q = 0; q < 4; ++q) {
+        // dgates are the next dgrad's operands: tf32 rounds to nearest here (the MMA would truncate), bf16 as stored
+        o0[q][j] = round_for(o0[q][j], static_cast<E*>(nullptr));
+        o1[q][j] = round_for(o1[q][j], static_cast<E*>(nullptr));
+      }
+    }
+    store_elems<float, 8>(kappa + ci, k);
+    store_elems<float, 8>(kappa + nk + ci, dk);
+#pragma unroll
+    for (int q = 0; q < 4; ++q) {
+      store_elems<E, 8>(da_out + gi + q * 16, o0[q]);
+      store_elems<E, 8>(da_out + npix * 4 * hc + gi + q * 16, o1[q]);
+    }
+  }
+}
+
+cudaError_t launch_soa_cell(int dtype, const float* eta, const float* u, long long u_bstride, const float* du,
+                            long long du_bstride, const float* head_w, const void* gates, const float* traw,
+                            const float* c_prev, const float* c_cur, const float* dc_prev, const float* dc_cur,
+                            float* kappa, void* da_out, long long npix, long long HW, int hc, cudaStream_t s) {
+  const long long total = npix * (hc / 8);
+  long long blocks = (total + 255) / 256;
+  if (blocks > 148 * 16) blocks = 148 * 16;
+  if (blocks <= 0) return cudaSuccess;
+  if (dtype == NINT_BF16)
+    soa_cell_kernel<__nv_bfloat16><<<blocks, 256, 0, s>>>(eta, u, u_bstride, du, du_bstride, head_w,
+                                                           reinterpret_cast<const __nv_bfloat16*>(gates), traw, c_prev,
+                                                           c_cur, dc_prev, dc_cur, kappa,
+                                                           reinterpret_cast<__nv_bfloat16*>(da_out), npix, HW, hc);
+  else
+    soa_cell_kernel<float><<<blocks, 256, 0, s>>>(eta, u, u_bstride, du, du_bstride, head_w,
+                                                  reinterpret_cast<const float*>(gates), traw, c_prev, c_cur, dc_prev,
+                                                  dc_cur, kappa, reinterpret_cast<float*>(da_out), npix, HW, hc);
   return cudaGetLastError();
 }
 

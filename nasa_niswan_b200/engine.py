@@ -22,7 +22,7 @@ class Plan:
     def __init__(self, batch: int, seq_len: int, height: int, width: int, in_channels: int,
                  hidden: Sequence[int], ksize: Sequence[int], precision: str = "bf16", training: bool = False,
                  return_sequence: bool = False, device=None, deterministic: bool = False, input_grad: bool = False,
-                 state_grad: bool = False, tangent: bool = False):
+                 state_grad: bool = False, tangent: bool = False, second_order: bool = False):
         if precision not in PRECISIONS:
             raise ValueError(f"precision must be one of {sorted(PRECISIONS)}")
         if len(hidden) != len(ksize):
@@ -37,7 +37,8 @@ class Plan:
         self.hidden, self.ksize, self.L = list(hidden), list(ksize), len(hidden)
         self.training, self.return_sequence, self.precision = bool(training), bool(return_sequence), precision
         self.deterministic, self.input_grad, self.state_grad = bool(deterministic), bool(input_grad), bool(state_grad)
-        self.tangent = bool(tangent)
+        self.second_order = bool(second_order)
+        self.tangent = bool(tangent) or self.second_order     # the second-order pass reads the tangent pass's history
         cfg = _lib.NintConfig()
         cfg.batch, cfg.seq_len, cfg.height, cfg.width = batch, seq_len, height, width
         cfg.in_channels, cfg.num_layers = in_channels, self.L
@@ -45,7 +46,8 @@ class Plan:
             cfg.hidden[i], cfg.ksize[i] = h, k
         cfg.dtype, cfg.training, cfg.return_sequence = PRECISIONS[precision], int(training), int(return_sequence)
         cfg.flags = ((_lib.FLAG_DETERMINISTIC if deterministic else 0) | (_lib.FLAG_INPUT_GRAD if input_grad else 0) |
-                     (_lib.FLAG_STATE_GRAD if state_grad else 0) | (_lib.FLAG_TANGENT if tangent else 0))
+                     (_lib.FLAG_STATE_GRAD if state_grad else 0) | (_lib.FLAG_TANGENT if tangent else 0) |
+                     (_lib.FLAG_SECOND_ORDER if second_order else 0))
         self._h = ctypes.c_void_p()
         _lib.check(self.lib.nint_plan_create(ctypes.byref(cfg), ctypes.byref(self._h)), "nint_plan_create")
         self.workspace_bytes = self.lib.nint_plan_workspace_bytes(self._h)
@@ -379,6 +381,58 @@ class Plan:
                                                           self._ptr_table(dh_T), self._ptr_table(dc_T), self._stream()),
                        "nint_forward_tangent_bank")
         return dpred, dseq, list(zip(dh_T, dc_T))
+
+    # ---- second-order adjoint (plans made with training=True, second_order=True)
+    def _head_seed(self, u, name):
+        """u: dL/dpred [B,1,H,W], or (dpred, dseq) with dseq [B,T,H,W] (return_sequence plans; either may be None) ->
+        (dpred, dseq) for the library, dpred folded into dseq[:, T-1] when both are given (pred is the last step)"""
+        dpred, dseq = tuple(u) if isinstance(u, (tuple, list)) else (u, None)
+        if dseq is not None:
+            self._check_dev(dseq, f"{name} (sequence)", (self.B, self.T, self.H, self.W))
+            dseq = dseq.detach().contiguous().clone() if dpred is not None else dseq.detach().contiguous()
+        if dpred is not None:
+            self._check_dev(dpred, name, (self.B, 1, self.H, self.W))
+            if dseq is not None:
+                dseq[:, -1] += dpred.detach().reshape(self.B, self.H, self.W)
+                dpred = None
+            else:
+                dpred = dpred.detach().contiguous()
+        return dpred, dseq
+
+    def _second_order(self, fn, u, du, targets, state):
+        dpred, dseq = self._head_seed(u, "u")
+        ddpred, ddseq = self._head_seed(du, "du")
+        new = lambda l: torch.empty(self._state_shape(l), dtype=torch.float32, device=self.device)
+        st = [[new(l) for l in range(self.L)] for _ in range(4)] if state else [None] * 4
+        with _lib.on_device(self.device):
+            _lib.check(fn(self._h, _ptr(dpred), _ptr(dseq), _ptr(ddpred), _ptr(ddseq), _ptr(targets[0]), _ptr(targets[1]),
+                          *[self._ptr_table(t) for t in st], self._stream()), fn.__name__)
+        return (list(zip(st[0], st[1])), list(zip(st[2], st[3]))) if state else (None, None)
+
+    def backward_second_order(self, u, du, state: bool = False):
+        """Gradient and Hessian-vector product of a loss L of the last `forward`'s outputs w.r.t. its input and initial
+        state, at fixed parameters, in the direction of the last `forward_tangent` of that forward (forward-over-reverse).
+        u = dL/dout and du = its tangent d2L/dout2 . dout, each dpred [B,1,H,W] or (dpred, dseq [B,T,H,W]) like the
+        plan's outputs (None entries are zero).  Returns (dx, ddx, dstate, ddstate): dx = grad_x L and ddx = (H v)_x
+        [B,T,C,H,W] fp32; with state=True, dstate / ddstate = [(dh0, dc0) per layer] of the gradient / of H v, else None.
+        The saved activations are only read: one forward can serve many (forward_tangent, backward_second_order) pairs,
+        e.g. the Hessian-vector products of a Newton-CG or Lanczos loop, and then one `backward`."""
+        new = lambda: torch.empty((self.B, self.T, self.C, self.H, self.W), dtype=torch.float32, device=self.device)
+        dx, ddx = new(), new()
+        dst, ddst = self._second_order(self.lib.nint_backward_second_order, u, du, (dx, ddx), state)
+        return dx, ddx, dst, ddst
+
+    def backward_second_order_bank(self, u, du, dframes: torch.Tensor, ddframes: torch.Tensor, state: bool = False):
+        """backward_second_order after `forward_bank` / `forward_tangent_bank`: the gradient and H v w.r.t. the frames
+        are ADDED into dframes / ddframes [N,C,H,W] fp32 (frame win_start[b] + t gets sample b's step t, in decreasing t
+        -- the pass runs backwards in time -- then increasing b).  Returns (dstate, ddstate) as backward_second_order."""
+        if self._keep is None:
+            raise RuntimeError("backward_second_order_bank: the last forward did not read a frame bank (forward_bank)")
+        for t, name in ((dframes, "dframes"), (ddframes, "ddframes")):
+            self._check_dev(t, name, (self._keep[0].shape[0], self.C, self.H, self.W))
+            if not t.is_contiguous():
+                raise ValueError(f"{name} must be contiguous")
+        return self._second_order(self.lib.nint_backward_second_order_bank, u, du, (dframes, ddframes), state)
 
     # ---- ConvLSTMCell as a differentiable unit (plans with T = 1, L = 1)
     def cell_forward(self, x, h, c):

@@ -166,30 +166,32 @@ class ConvLSTM(nn.Module):
         return ps + [self.conv.weight, self.conv.bias]
 
     def plan_for_shape(self, B, T, H, W, device, training, set_params=True, input_grad=False, state_grad=False,
-                       tangent=False):
+                       tangent=False, second_order=False):
         device = torch.device(device)
         if device.index is None:
             device = torch.device("cuda", torch.cuda.current_device())
         det = bool(training) and _deterministic_default()
         key = (B, T, H, W, bool(training), self.return_sequence, self.precision, device, bool(input_grad),
-               bool(state_grad), det, bool(tangent))
+               bool(state_grad), det, bool(tangent), bool(second_order))
         hidden = [c.hidden_channels for c in self.layers]
         ks = [c.kernel_size for c in self.layers]
         plan = self._plans.get(key, lambda: Plan(B, T, H, W, self.input_channels, hidden, ks, precision=self.precision,
                                                  training=training, return_sequence=self.return_sequence,
                                                  device=device, deterministic=det, input_grad=input_grad,
-                                                 state_grad=state_grad, tangent=tangent))
+                                                 state_grad=state_grad, tangent=tangent, second_order=second_order))
         if set_params:
             for l, cell in enumerate(self.layers):
                 plan.set_weights(l, cell.conv.weight, cell.conv.bias)
             plan.set_head(self.conv.weight, self.conv.bias)
         return plan
 
-    def plan_for(self, x, training, set_params=True, input_grad=False, state_grad=False, tangent=False):
+    def plan_for(self, x, training, set_params=True, input_grad=False, state_grad=False, tangent=False,
+                 second_order=False):
         B, T, C, H, W = x.size()
         if C != self.input_channels:
             raise ValueError(f"expected {self.input_channels} input channels, got {C}")
-        return self.plan_for_shape(B, T, H, W, x.device, training, set_params, input_grad, state_grad, tangent)
+        return self.plan_for_shape(B, T, H, W, x.device, training, set_params, input_grad, state_grad, tangent,
+                                   second_order)
 
     def _wants_grad(self, params):
         return torch.is_grad_enabled() and any(p.requires_grad for p in params)
@@ -297,6 +299,56 @@ class ConvLSTM(nn.Module):
             final = plan.final_state() if return_state else None
             dpred, dseq, dfinal = plan.forward_tangent_bank(dbank, dh0, dc0)
         return self._jvp_result(pred, seq, final, dpred, dseq, dfinal, return_state)
+
+    def _loss_seeds(self, loss_fn, pred, seq, dpred, dseq):
+        """(loss, u, du): loss_fn at what forward returns, u = its gradient and du = its tangent in the direction the
+        tangent pass gave, by torch.func on the (small) output tensors"""
+        out = (pred, seq) if self.return_sequence else pred
+        dout = (dpred, dseq) if self.return_sequence else dpred
+        (u, loss), (du, _) = torch.func.jvp(torch.func.grad_and_value(loss_fn), (out,), (dout,))
+        return loss.detach(), u, du
+
+    def hvp(self, x, dx, loss_fn, hidden_state=None, state_tangent=None):
+        """Second-order adjoint at fixed parameters: returns (loss, grad, hvp) with loss = loss_fn(forward(x,
+        hidden_state)), grad its gradient and hvp = H v its Hessian-vector product w.r.t. (x, initial state) in the
+        direction v = (dx, state_tangent), the exact Hessian including the curvature of the recurrence (not the
+        Gauss-Newton part of jvp + backward).  grad and hvp are (d/dx [B,T,C,H,W], [(d/dh0, d/dc0)] per layer when
+        hidden_state is given, else None).  loss_fn maps what forward returns to a scalar and must be differentiable
+        twice by torch.func (MSE + L1 is: L1 has zero curvature almost everywhere).  dx / state_tangent as in `jvp`.
+        Cost: a forward, a tangent pass and a second-order pass (DESIGN.md section 10, f8).  For many directions on one
+        forward (Newton-CG, Lanczos) use the plan directly: plan = model.plan_for(x, True, second_order=True),
+        plan.forward(x), then per direction plan.forward_tangent(...) and plan.backward_second_order(u, du), with u, du
+        from the outputs as here; the forward's activations stay intact for one ordinary backward at the end."""
+        if not x.is_cuda:
+            raise RuntimeError("ConvLSTM runs on CUDA (B200) only: there is no CPU fallback")
+        plan = self.plan_for(x, True, second_order=True)
+        dh0, dc0 = self._tangent_state(plan, state_tangent)
+        with torch.no_grad():
+            pred, seq = plan.forward(x, hidden_state)
+            dpred, dseq, _ = plan.forward_tangent(dx, dh0, dc0)
+        loss, u, du = self._loss_seeds(loss_fn, pred, seq, dpred, dseq)
+        state = plan.check_state(hidden_state)
+        gx, hx, gs, hs = plan.backward_second_order(u, du, state=state)
+        return loss, (gx, gs), (hx, hs)
+
+    def hvp_windows(self, bank, win_start, seq_len, dbank, loss_fn, hidden_state=None, state_tangent=None):
+        """`hvp` over frame-bank windows (forward_windows / jvp_windows): the direction of the frames is dbank
+        [N,Hp,Wp,c_pad] (FrameBank.tangent / tangent_from_fields).  grad and hvp are (d/dframes [N,C,Hp,Wp] fp32, state
+        pairs or None): every window's contribution is summed into the frames it read.  bank.grad is not touched."""
+        starts = win_start.to(device=bank.frames.device, dtype=torch.int32).contiguous()
+        bank.check_windows(win_start, seq_len)
+        N, H, W, _ = bank.frames.shape
+        plan = self.plan_for_shape(starts.shape[0], int(seq_len), H, W, bank.frames.device, True, second_order=True)
+        bank.check_plan(plan)
+        dh0, dc0 = self._tangent_state(plan, state_tangent)
+        with torch.no_grad():
+            pred, seq = plan.forward_bank(bank.frames, starts, hidden_state)
+            dpred, dseq, _ = plan.forward_tangent_bank(dbank, dh0, dc0)
+        loss, u, du = self._loss_seeds(loss_fn, pred, seq, dpred, dseq)
+        new = lambda: torch.zeros((N, bank.channels, H, W), dtype=torch.float32, device=bank.frames.device)
+        gf, hf = new(), new()
+        gs, hs = plan.backward_second_order_bank(u, du, gf, hf, state=plan.check_state(hidden_state))
+        return loss, (gf, gs), (hf, hs)
 
     def release_workspaces(self):
         self._plans.clear()

@@ -11,6 +11,7 @@ from typing import Optional, Tuple
 import torch
 
 from . import _lib
+from .preprocess import fuse_inputs_adjoint
 
 
 def save_checkpoint(model, optimizer, filename, learning_rate=None, epoch=None):
@@ -188,3 +189,16 @@ def emission_response(model, bank, win_start, seq_len: int, d_emis2d: torch.Tens
     if crop is not None:
         dpred = dpred[:, :, crop[0]:crop[1], crop[2]:crop[3]]
     return dpred[:, 0] * y_std
+
+
+def emission_hvp(model, bank, win_start, seq_len: int, d_emis2d: torch.Tensor, loss_fn):
+    """The Hessian-vector product of loss_fn(model.forward_windows(bank, win_start, seq_len)) w.r.t. the raw fields of
+    a bank built by `FrameBank.from_fields`, in the direction of an emission perturbation d_emis2d [N, H, W]: the
+    curvature a Newton-CG or truncated-Newton emission inversion needs.  The fusion is affine in the fields, so H v in
+    field space is its adjoint applied to the frame-space H of its tangent: FrameBank.tangent_from_fields, then
+    ConvLSTM.hvp_windows, then the preprocessing adjoint (nint_fuse_inputs_adjoint) of the HVP frames.  Returns the dict
+    of `field_grads()` ({"levels3d", "emis2d", "statics"}) holding H v."""
+    if bank._fields is None:
+        raise RuntimeError("emission_hvp needs a bank built by FrameBank.from_fields")
+    _, _, (hv, _) = model.hvp_windows(bank, win_start, seq_len, bank.tangent_from_fields(d_emis2d=d_emis2d), loss_fn)
+    return fuse_inputs_adjoint(hv, **bank._fields)
