@@ -65,6 +65,14 @@ typedef struct nint_config {
 #define NINT_FLAG_STATE_GRAD 4
 #define NINT_FLAG_TANGENT 8
 #define NINT_FLAG_SECOND_ORDER 16
+/* NINT_FLAG_PARAM_TANGENT: training plans also keep a parameter direction for nint_forward_tangent[_bank] (the flag
+ * implies NINT_FLAG_TANGENT): per layer the direction's weight panels packed like the forward's and its q-order fp32
+ * bias [4*hc], and the head's direction (dw [Hc_last], db).  Together with NINT_FLAG_SECOND_ORDER the plan also keeps
+ * what the parameter terms of nint_backward_second_order[_bank] and nint_backward_second_order_params need: per layer
+ * the direction's dgrad panels, the tangent dh of every step [T+1,B,H,W,hc_pad] E (slot 0 = dh0; in place of the
+ * 2-slot ring) and the pass's dgates and their tangents of every step [T][2B,H,W,4hc] E (in place of one step), and
+ * the head's reductions.  Plans without it have the same workspace and issue the same launches. */
+#define NINT_FLAG_PARAM_TANGENT 32
 #define NINT_X_FP32 0
 #define NINT_X_BF16 1
 
@@ -169,6 +177,33 @@ int nint_forward_tangent(nint_plan* plan, const void* dx, int dx_dtype, const fl
 int nint_forward_tangent_bank(nint_plan* plan, const void* dbank, long long n_frames, const float* const* dh0,
                               const float* const* dc0, float* dpred, float* dseq, float* const* dh_T,
                               float* const* dc_T, void* stream);
+
+/* ---- parameter-space tangent: the direction dtheta = (dW_l, db_l per layer, dw_head, db_head) that later
+ * nint_forward_tangent[_bank] calls include next to (dx, dh0, dc0), giving J (dx, dh0, dc0, dtheta).  Per step and layer
+ * the tangent gate GEMM gains dW (*) [x_t, h_{t-1}] + db over the forward's own operands (one more GEMM launch, added
+ * into the tangent GEMM's fp32 dump), and the head gains dw_head . h_t + db_head.  Shapes as nint_plan_set_weights /
+ * nint_plan_set_head; dbias NULL = zero.  A layer or head without a direction set
+ * has zero direction and costs nothing; nint_plan_clear_param_tangent clears them all (the tangent pass then issues
+ * exactly the launches of a plan without the flag).  Training plans created with NINT_FLAG_PARAM_TANGENT.  Setting or
+ * clearing a direction after a tangent pass makes a following nint_backward_second_order[_bank] fail until the tangent
+ * pass is run again.  On plans that also have NINT_FLAG_SECOND_ORDER the second-order pass takes the direction's terms:
+ * deta_t gains dW_h^T (*) a_{t+1} + dW_x(above)^T (*) a_t (one EPI_RAW_ACC dgrad over the primal dgates), the top
+ * layer's u dw_head, H v w.r.t. x gains dW_x^T (*) a_t and w.r.t. h0 dW_h^T (*) a_0. */
+int nint_plan_set_weight_tangent(nint_plan* plan, int layer, const float* dweight, const float* dbias, void* stream);
+int nint_plan_set_head_tangent(nint_plan* plan, const float* dweight, const float* dbias, void* stream);
+int nint_plan_clear_param_tangent(nint_plan* plan, void* stream);
+/* Parameter outputs of the last nint_backward_second_order[_bank] on a plan created with NINT_FLAG_SECOND_ORDER |
+ * NINT_FLAG_PARAM_TANGENT, for the joint direction (dx, dh0, dc0, dtheta) of the tangent pass it followed:
+ *   grad_W_l = sum_t wgrad(a_t, comb_t), grad_b_l = sum_t a_t; (H v)_W_l = sum_t wgrad(da_t, comb_t) + wgrad(a_t, dcomb_t),
+ *   (H v)_b_l = sum_t da_t; head: grad w = sum u h, grad b = sum u, (H v)_w = sum du h + u dh, (H v)_b = sum du
+ * (a, da = the pass's dgates and their tangents, comb_t = [x_t, h_{t-1}], dcomb_t its tangent; sums over every t with a
+ * head seed).  The second-order pass reduces the head terms while it holds u and du, so this call takes no seeds.
+ * Host arrays of L device pointers with the parameters' shapes (arrays and entries may be NULL = not wanted; a layer's
+ * bias is written with its weight), head outputs [Hc_last] / [1]; all WRITTEN.  Refused before a second-order pass of
+ * the current forward, tangent pass and direction.  Deterministic plans give bit-reproducible outputs. */
+int nint_backward_second_order_params(nint_plan* plan, float* const* grad_weight, float* const* grad_bias,
+                                      float* const* hvp_weight, float* const* hvp_bias, float* grad_head_weight,
+                                      float* grad_head_bias, float* hvp_head_weight, float* hvp_head_bias, void* stream);
 
 /* ---- second-order adjoint: the Hessian-vector product H v = d/de grad_z L(z + e v) of a loss L of the last forward's
  * outputs w.r.t. its input windows and initial state z, at fixed parameters, as forward-over-reverse.  One reverse pass

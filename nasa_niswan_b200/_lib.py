@@ -10,13 +10,15 @@ DTYPE_BF16, DTYPE_TF32 = 0, 1
 DTYPE_BYTES = {DTYPE_BF16: 2, DTYPE_TF32: 4}
 X_FP32, X_BF16 = 0, 1
 FLAG_DETERMINISTIC, FLAG_INPUT_GRAD, FLAG_STATE_GRAD, FLAG_TANGENT, FLAG_SECOND_ORDER = 1, 2, 4, 8, 16
+FLAG_PARAM_TANGENT = 32
 EXPORTS = ["nint_version", "nint_last_error", "nint_plan_create", "nint_plan_destroy", "nint_plan_workspace_bytes",
            "nint_plan_bind", "nint_plan_set_weights", "nint_plan_set_head", "nint_plan_reset_state",
            "nint_plan_set_state", "nint_plan_get_state", "nint_forward", "nint_forward_ex", "nint_forward_bank",
            "nint_plan_input_layout", "nint_pack_frames", "nint_backward", "nint_debug_raw_gates",
            "nint_gate_column", "nint_debug_read_trace", "nint_debug_fail_record", "nint_backward_bptt", "nint_backward_wgrad",
            "nint_backward_bptt_state", "nint_backward_initial_state", "nint_backward_input", "nint_backward_input_bank", "nint_forward_tangent",
-           "nint_forward_tangent_bank", "nint_backward_second_order", "nint_backward_second_order_bank", "nint_cell_forward", "nint_cell_backward", "nint_loss_mse_l1",
+           "nint_forward_tangent_bank", "nint_backward_second_order", "nint_backward_second_order_bank", "nint_plan_set_weight_tangent",
+           "nint_plan_set_head_tangent", "nint_plan_clear_param_tangent", "nint_backward_second_order_params", "nint_cell_forward", "nint_cell_backward", "nint_loss_mse_l1",
            "nint_loss_mse_l1_bank", "nint_adam_step", "nint_adam_step_dev", "nint_dp_allreduce_adam", "nint_fuse_inputs", "nint_fuse_inputs_bank",
            "nint_fuse_inputs_adjoint", "nint_pick_tile", "nint_launch_count", "nint_plan_profile", "nint_plan_profile_read"]
 
@@ -66,6 +68,10 @@ def load():
     L.nint_forward_tangent_bank.argtypes = [vp, fp, ctypes.c_longlong, pp, pp, fp, fp, pp, pp, vp]
     L.nint_backward_second_order.argtypes = [vp, fp, fp, fp, fp, fp, fp, pp, pp, pp, pp, vp]
     L.nint_backward_second_order_bank.argtypes = [vp, fp, fp, fp, fp, fp, fp, pp, pp, pp, pp, vp]
+    L.nint_plan_set_weight_tangent.argtypes = [vp, ci, fp, fp, vp]
+    L.nint_plan_set_head_tangent.argtypes = [vp, fp, fp, vp]
+    L.nint_plan_clear_param_tangent.argtypes = [vp, vp]
+    L.nint_backward_second_order_params.argtypes = [vp, pp, pp, pp, pp, fp, fp, fp, fp, vp]
     L.nint_cell_forward.argtypes = [vp, fp, fp, fp, fp, fp, vp]
     L.nint_cell_backward.argtypes = [vp, fp, fp, fp, fp, fp, fp, fp, vp]
     L.nint_backward.argtypes = [vp, fp, fp, ctypes.POINTER(vp), ctypes.POINTER(vp), fp, fp, vp]

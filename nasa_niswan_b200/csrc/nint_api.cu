@@ -92,6 +92,18 @@ struct Layer {
   CUtensorMap tm_sA;
   uint8_t *wx = nullptr, *wh = nullptr, *wdx = nullptr, *wdh = nullptr;
   float *bias_q = nullptr, *dw_acc = nullptr, *db_acc = nullptr;
+  // NINT_FLAG_PARAM_TANGENT: the parameter direction dW packed like wx / wh (same panels, i/f/o halved) and its bias in
+  // q-order; dw_set: a direction is set for this layer (else dW = 0 and the tangent pass runs no dW GEMM); dbias_add:
+  // the tangent cell adds tbias_q (the bias is not folded into the dW GEMM through the constant-1 lane)
+  uint8_t *twx = nullptr, *twh = nullptr;
+  float* tbias_q = nullptr;
+  bool dw_set = false, dbias_add = false;
+  // NINT_FLAG_PARAM_TANGENT + NINT_FLAG_SECOND_ORDER: dW's dgrad panels (laid out as wdx / wdh) for the second-order
+  // pass's dW^T terms, and the wgrad views of the parameter outputs: the pass's (a, da) history as dgates operand
+  // (primal view / tangent view: images [0, B) / [B, 2B) of every [2B] step slot) and the dh history as the h part /
+  // as the x part of layer l+1 (32-channel boxes, CTA-pair boxes)
+  uint8_t *twdx = nullptr, *twdh = nullptr;
+  CUtensorMap tmw_sA[2], tmp_sA[2], tmw_tH, tmw_tH_up, tmp_tH, tmp_tH_up;
   float* db_resid = nullptr;   // tf32 training plans: [kResidCtas][4][4hc] sums of the dgates rounding residuals (nint_kernels.h)
   size_t dw_acc_bytes = 0;   // one slice [taps][4hc][ncols]; deterministic mode keeps det_splits slices
   int det_splits = 0;
@@ -99,7 +111,7 @@ struct Layer {
   CUtensorMap tm_H, tm_G;
   // weight maps depend on the launch's shared-memory plan (taps per stage): encoded on first use, cached
   struct WMap { int ts = 0, rows = 0, n_tile = 0; CUtensorMap map; };
-  std::vector<WMap> wmaps[4];   // 0: wx, 1: wh, 2: wdx, 3: wdh
+  std::vector<WMap> wmaps[8];   // 0: wx, 1: wh, 2: wdx, 3: wdh, 4: twx, 5: twh, 6: twdx, 7: twdh
   CUtensorMap tm_H_up;       // Hs[l] read as the x segment of layer l+1 (halo of k_{l+1})
   CUtensorMap tmw_H, tmw_G;  // wgrad views (32-channel boxes; differ from tm_* in tf32 mode only)
   CUtensorMap tmw_H_up;      // Hs[l] as the x part of layer l+1's wgrad (halo of k_{l+1})
@@ -160,6 +172,16 @@ struct nint_plan {
   // tangent_kept: the per-step tangent dumps belong to the last forward
   bool second_order = false, tangent_kept = false;
   float* sraw = nullptr;
+  // NINT_FLAG_PARAM_TANGENT: the head's parameter direction (dw [hc], db) and whether one is set; param_in_tangent:
+  // the last tangent pass included a parameter direction (the second-order pass has no parameter terms yet)
+  bool param_tangent = false, dhead_set = false, param_in_tangent = false;
+  float *thead_w = nullptr, *thead_b = nullptr;
+  // both flags: the tangent pass keeps dh of every step (tH [T+1] slots, slot 0 = dh0) and the second-order pass
+  // (a, da) of every step (sA [T][2B]); head_sums = the pass's head reductions {grad w [hc], grad b, hvp w [hc], hvp b};
+  // soa_params: the last second-order pass belongs to the current forward and tangent (the params call may run)
+  bool hist = false, soa_params = false;
+  float* head_sums = nullptr;
+  CUtensorMap tmw_tX, tmp_tX, tmbw_tX, tmbp_tX;
   unsigned* step_done = nullptr;   // [T][B] tile counters of a time-fused conv launch (ConvGemmParams::step_done)
   // consecutive time steps of a layer as ONE persistent launch whose tiles wait on the previous step's tiles of the same
   // image (ConvGemmParams::n_steps).  -1: automatic -- BPTT launches are fused while they are short (bwd_should_fuse),
@@ -230,8 +252,9 @@ int pick_tile(int H, int W, int* tw_out, int* th_out) {
 
 // wgrad = true: 32-channel box; tf32 then needs the 128B swizzle with 32-byte atoms (the MN-major tf32
 // UMMA layout), bf16 is the same 64-byte box either way.
+// slot_images: images between consecutive slots (0: B; a view of B images out of larger slots)
 int encode_act_map(CUtensorMap* m, int dtype, void* base, int C, int W, int H, int B, int slots, int ce, int tw,
-                   int th, bool wgrad = false, int halo = 0) {
+                   int th, bool wgrad = false, int halo = 0, long long slot_images = 0) {
   tw += 2 * halo;
   th += 2 * halo;
   EncodeTiledFn enc = get_encode();
@@ -239,7 +262,7 @@ int encode_act_map(CUtensorMap* m, int dtype, void* base, int C, int W, int H, i
   const cuuint64_t es = dtype == BF16 ? 2 : 4;
   cuuint64_t dims[5] = {(cuuint64_t)C, (cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)B, (cuuint64_t)slots};
   cuuint64_t strides[4] = {C * es, (cuuint64_t)W * C * es, (cuuint64_t)H * W * C * es,
-                           (cuuint64_t)B * H * W * C * es};
+                           (cuuint64_t)(slot_images ? slot_images : B) * H * W * C * es};
   cuuint32_t box[5] = {(cuuint32_t)(wgrad ? 32 : ce), (cuuint32_t)tw, (cuuint32_t)th, 1, 1};
   cuuint32_t estr[5] = {1, 1, 1, 1, 1};
   const CUtensorMapSwizzle sw = (wgrad && dtype == TF32) ? CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B : CU_TENSOR_MAP_SWIZZLE_64B;
@@ -252,13 +275,13 @@ int encode_act_map(CUtensorMap* m, int dtype, void* base, int C, int W, int H, i
 
 // general activation box: `box_c` channels x (tw + 2*halo) x (th + 2*halo) pixels with an explicit swizzle
 int encode_act_box(CUtensorMap* m, int dtype, void* base, int C, int W, int H, int B, int slots, int box_c, int tw,
-                   int th, int halo, CUtensorMapSwizzle sw) {
+                   int th, int halo, CUtensorMapSwizzle sw, long long slot_images = 0) {
   EncodeTiledFn enc = get_encode();
   if (!enc) return fail("cuTensorMapEncodeTiled not available (no CUDA driver?)");
   const cuuint64_t es = dtype == BF16 ? 2 : 4;
   cuuint64_t dims[5] = {(cuuint64_t)C, (cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)B, (cuuint64_t)slots};
   cuuint64_t strides[4] = {C * es, (cuuint64_t)W * C * es, (cuuint64_t)H * W * C * es,
-                           (cuuint64_t)B * H * W * C * es};
+                           (cuuint64_t)(slot_images ? slot_images : B) * H * W * C * es};
   cuuint32_t box[5] = {(cuuint32_t)box_c, (cuuint32_t)(tw + 2 * halo), (cuuint32_t)(th + 2 * halo), 1, 1};
   cuuint32_t estr[5] = {1, 1, 1, 1, 1};
   CUresult r = enc(m, dtype == BF16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 5, base,
@@ -372,7 +395,7 @@ size_t carve(nint_plan* p, uint8_t* base) {
     int max_hc = 0;
     for (int l = 0; l < p->L; ++l) {
       Layer& y = p->layer[l];
-      y.tH = take(act_bytes(p, 2, y.hc_pad));
+      y.tH = take(act_bytes(p, p->hist ? p->T + 1 : 2, y.hc_pad));
       y.tC = reinterpret_cast<float*>(take(npix * y.hc * 4 * (p->second_order ? p->T + 1 : 1)));
       if (p->second_order) y.tR = reinterpret_cast<float*>(take(static_cast<size_t>(p->T) * npix * 4 * y.hc * 4));
       max_hc = max_hc > y.hc ? max_hc : y.hc;
@@ -380,11 +403,32 @@ size_t carve(nint_plan* p, uint8_t* base) {
     if (!p->second_order) p->traw = reinterpret_cast<float*>(take(npix * 4 * max_hc * 4));
     p->tzero = reinterpret_cast<float*>(take(16));
   }
+  if (tr && p->param_tangent) {
+    const size_t wrow = static_cast<size_t>(p->ce) * p->esize;
+    for (int l = 0; l < p->L; ++l) {
+      Layer& y = p->layer[l];
+      y.twx = take(static_cast<size_t>(y.n_blocks) * y.taps * y.chx * y.n_tile * wrow);
+      y.twh = take(static_cast<size_t>(y.n_blocks) * y.taps * y.chh * y.n_tile * wrow);
+      y.tbias_q = reinterpret_cast<float*>(take(4 * y.hc * 4));
+    }
+    p->thead_w = reinterpret_cast<float*>(take(top.hc * 4));
+    p->thead_b = reinterpret_cast<float*>(take(16));
+  }
+  if (tr && p->hist) {
+    const size_t wrow = static_cast<size_t>(p->ce) * p->esize;
+    for (int l = 0; l < p->L; ++l) {
+      Layer& y = p->layer[l];
+      const int nch = 4 * y.hc / p->ce;
+      y.twdx = take(static_cast<size_t>(y.taps) * nch * y.cin_rows * wrow);
+      y.twdh = take(static_cast<size_t>(y.taps) * nch * y.hc * wrow);
+    }
+    p->head_sums = reinterpret_cast<float*>(take(static_cast<size_t>(2 * (top.hc + 1) + 1) * 4));
+  }
   if (tr && p->second_order) {
     int cols = p->layer[0].cin_rows;
     for (int l = 0; l < p->L; ++l) {
       Layer& y = p->layer[l];
-      y.sA = take(act_bytes(p, 2, 4 * y.hc));
+      y.sA = take(act_bytes(p, p->hist ? 2 * p->T : 2, 4 * y.hc));
       y.sK = reinterpret_cast<float*>(take(2 * npix * y.hc * 4));
       cols = cols > y.hc ? cols : y.hc;
     }
@@ -439,15 +483,17 @@ int bwd_cluster(const nint_plan* p, int l) {
 }
 
 // weight map of layer `y` for one K segment: which = 0 wx, 1 wh (forward, N = n_tile per n-block), 2 wdx, 3 wdh
-// (dgrad, N = n_tile input channels); `rows` = N rows per CTA, `ts` = taps per weight stage
+// (dgrad, N = n_tile input channels), 4 twx, 5 twh (the parameter tangent, laid out as wx / wh); `rows` = N rows per
+// CTA, `ts` = taps per weight stage
 int get_w_map(nint_plan* p, Layer& y, int which, int n_tile, int rows, int ts, CUtensorMap* out) {
   for (const Layer::WMap& w : y.wmaps[which])
     if (w.ts == ts && w.rows == rows && w.n_tile == n_tile) { *out = w.map; return 0; }
-  void* base = which == 0 ? y.wx : which == 1 ? y.wh : which == 2 ? y.wdx : y.wdh;
+  void* const bases[8] = {y.wx, y.wh, y.wdx, y.wdh, y.twx, y.twh, y.twdx, y.twdh};
+  void* base = bases[which];
   if (!base) return fail("internal: packed weight tensor %d of this layer was not allocated", which);
   long long chunk_taps;
-  if (which == 0) chunk_taps = (long long)y.n_blocks * y.chx * y.taps;
-  else if (which == 1) chunk_taps = (long long)y.n_blocks * y.chh * y.taps;
+  if (which == 0 || which == 4) chunk_taps = (long long)y.n_blocks * y.chx * y.taps;
+  else if (which == 1 || which == 5) chunk_taps = (long long)y.n_blocks * y.chh * y.taps;
   else chunk_taps = (long long)(4 * y.hc / p->ce) * y.taps;
   Layer::WMap w;
   w.ts = ts; w.rows = rows; w.n_tile = n_tile;
@@ -797,7 +843,9 @@ int nint_plan_create(const nint_config* cfg, nint_plan** out) {
   p->input_grad = (cfg->flags & NINT_FLAG_INPUT_GRAD) != 0;
   p->state_grad = (cfg->flags & NINT_FLAG_STATE_GRAD) != 0;
   p->second_order = (cfg->flags & NINT_FLAG_SECOND_ORDER) != 0;
-  p->tangent = (cfg->flags & NINT_FLAG_TANGENT) != 0 || p->second_order;
+  p->param_tangent = (cfg->flags & NINT_FLAG_PARAM_TANGENT) != 0;
+  p->hist = p->param_tangent && p->second_order && cfg->training;
+  p->tangent = (cfg->flags & NINT_FLAG_TANGENT) != 0 || p->second_order || p->param_tangent;
   {  // debug / A-B knobs (documented in DESIGN.md): CTA pairs on/off, experiment flags
     const char* c = getenv("NINT_CLUSTER");
     p->cluster = c ? atoi(c) : 2;
@@ -936,6 +984,45 @@ static int encode_input_maps(nint_plan* p, void* base, long long images, int slo
   return 0;
 }
 
+static CUtensorMapSwizzle pair_swizzle(int pw) {
+  return pw == 64 ? CU_TENSOR_MAP_SWIZZLE_128B : (pw == 32 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_32B);
+}
+
+// wgrad views of the parameter outputs (plans with both NINT_FLAG_PARAM_TANGENT and NINT_FLAG_SECOND_ORDER), the same box
+// geometries as the ordinary wgrad's maps: the input tangent, the dh history and the pass's (a, da) history
+static int encode_param_wgrad_maps(nint_plan* p) {
+  const int tw = p->tile_w, th = p->tile_h, ce = p->ce, T = p->T, B = p->B;
+  CUtensorMap conv;
+  if (encode_input_maps(p, p->tX, B, T, &conv, &p->tmw_tX, &p->tmp_tX)) return 1;
+  for (int l = 0; l < p->L; ++l) {
+    Layer& y = p->layer[l];
+    const int pad = y.k / 2;
+    for (int v = 0; v < 2; ++v) {   // images [0, B) / [B, 2B) of every [2B] slot
+      uint8_t* base = y.sA + act_bytes(p, v, 4 * y.hc);
+      if (encode_act_map(&y.tmw_sA[v], p->dtype, base, 4 * y.hc, p->W, p->H, B, T, ce, tw, th, true, 0, 2LL * B)) return 1;
+    }
+    if (encode_act_map(&y.tmw_tH, p->dtype, y.tH, y.hc_pad, p->W, p->H, B, T + 1, ce, tw, th, true, pad)) return 1;
+    if (l + 1 < p->L &&
+        encode_act_map(&y.tmw_tH_up, p->dtype, y.tH, y.hc_pad, p->W, p->H, B, T + 1, ce, tw, th, true, p->layer[l + 1].k / 2))
+      return 1;
+    bool any_pair = false;
+    for (const Layer::WgBlock& b : y.wg_blocks) {
+      if (!b.pair || p->dtype != BF16) continue;
+      any_pair = true;
+      if (b.nch_h > 0 &&
+          encode_act_box(&y.tmp_tH, p->dtype, y.tH, y.hc_pad, p->W, p->H, B, T + 1, b.pw, tw, th, pad, pair_swizzle(b.pw))) return 1;
+      if (b.nch_x > 0 && l > 0) {
+        Layer& dn = p->layer[l - 1];
+        if (encode_act_box(&dn.tmp_tH_up, p->dtype, dn.tH, dn.hc_pad, p->W, p->H, B, T + 1, b.pw, tw, th, pad, pair_swizzle(b.pw))) return 1;
+      }
+    }
+    for (int v = 0; v < 2 && any_pair; ++v)
+      if (encode_act_box(&y.tmp_sA[v], p->dtype, y.sA + act_bytes(p, v, 4 * y.hc), 4 * y.hc, p->W, p->H, B, T, 64, tw, th, 0,
+                         CU_TENSOR_MAP_SWIZZLE_128B, 2LL * B)) return 1;
+  }
+  return 0;
+}
+
 int nint_plan_bind(nint_plan* p, void* workspace, size_t bytes, void* stream) {
   if (!p || !workspace) return fail("nint_plan_bind: null argument");
   if (bytes < p->ws_bytes) return fail("workspace too small: %zu < %zu", bytes, p->ws_bytes);
@@ -1003,20 +1090,26 @@ int nint_plan_bind(nint_plan* p, void* workspace, size_t bytes, void* stream) {
   }
   if (p->cfg.training && p->tangent) {   // the tangent GEMM reads its operands through the forward's box geometry
     if (encode_act_map(&p->tm_tX, p->dtype, p->tX, p->layer[0].cx_pad, p->W, p->H, p->B, p->T, ce, tw, th, false, pad_of(0))) return 1;
+    const int th_slots = p->hist ? p->T + 1 : 2;
     for (int l = 0; l < p->L; ++l) {
       Layer& y = p->layer[l];
-      if (encode_act_map(&y.tm_tH, p->dtype, y.tH, y.hc_pad, p->W, p->H, p->B, 2, ce, tw, th, false, pad_of(l))) return 1;
+      if (encode_act_map(&y.tm_tH, p->dtype, y.tH, y.hc_pad, p->W, p->H, p->B, th_slots, ce, tw, th, false, pad_of(l))) return 1;
       if (l + 1 < p->L &&
-          encode_act_map(&y.tm_tH_up, p->dtype, y.tH, y.hc_pad, p->W, p->H, p->B, 2, ce, tw, th, false, pad_of(l + 1))) return 1;
+          encode_act_map(&y.tm_tH_up, p->dtype, y.tH, y.hc_pad, p->W, p->H, p->B, th_slots, ce, tw, th, false, pad_of(l + 1))) return 1;
     }
+    if (p->hist && encode_param_wgrad_maps(p)) return 1;
     p->tbank_ptr = nullptr;
     p->tbank_frames = 0;
     for (int l = 0; l < p->L && p->second_order; ++l) {
       Layer& y = p->layer[l];
-      if (encode_act_map(&y.tm_sA, p->dtype, y.sA, 4 * y.hc, p->W, p->H, 2 * p->B, 1, ce, tw, th, false, pad_of(l))) return 1;
+      if (encode_act_map(&y.tm_sA, p->dtype, y.sA, 4 * y.hc, p->W, p->H, 2 * p->B, p->hist ? p->T : 1, ce, tw, th, false, pad_of(l))) return 1;
     }
   }
   p->tangent_kept = false;
+  p->param_in_tangent = false;
+  p->soa_params = false;
+  p->dhead_set = false;
+  for (int l = 0; l < p->L; ++l) p->layer[l].dw_set = p->layer[l].dbias_add = false;
   p->zero_init = true;
   p->fwd_done = false;
   p->gates_valid = false;
@@ -1046,6 +1139,52 @@ int nint_plan_set_head(nint_plan* p, const float* weight, const float* bias, voi
   CK(cudaMemcpyAsync(p->head_w, weight, p->layer[p->L - 1].hc_real * 4, cudaMemcpyDeviceToDevice, st));
   CK(cudaMemcpyAsync(p->head_b, bias, 4, cudaMemcpyDeviceToDevice, st));
   p->head_set = true;
+  return 0;
+}
+
+static int param_tangent_check(nint_plan* p, const char* what) {
+  if (!p || !p->ws) return fail("plan not bound");
+  if (!p->cfg.training || !p->param_tangent)
+    return fail("%s needs a training plan created with NINT_FLAG_PARAM_TANGENT", what);
+  // the second-order pass must linearise at the direction the tangent pass it follows used
+  p->tangent_kept = false;
+  p->soa_params = false;
+  return 0;
+}
+
+int nint_plan_set_weight_tangent(nint_plan* p, int l, const float* dweight, const float* dbias, void* stream) {
+  if (param_tangent_check(p, "nint_plan_set_weight_tangent")) return 1;
+  if (l < 0 || l >= p->L) return fail("layer %d out of range", l);
+  if (!dweight) return fail("nint_plan_set_weight_tangent: null weight tangent");
+  Layer& y = p->layer[l];
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  // layer 0 with a constant-1 input lane: dbias rides in the dW GEMM over the primal x, like the forward's bias
+  const bool fold = l == 0 && p->ones_lane >= 0 && !(p->debug_flags & 512);
+  LAUNCH(p, K_OTHER, st, launch_pack_weights_fwd(p->dtype, dweight, dbias, y.twx, y.twh, y.tbias_q, y.cin, y.hc_real, y.hc, y.hcb,
+                                                 y.k, y.cx_pad, y.hc_pad, fold ? p->ones_lane : -1, st));
+  if (p->hist)
+    LAUNCH(p, K_OTHER, st, launch_pack_weights_bwd(p->dtype, dweight, y.twdx, y.twdh, y.cin, y.cin_rows, y.hc_real, y.hc, y.k, st));
+  y.dw_set = true;
+  y.dbias_add = dbias != nullptr && !fold;
+  return 0;
+}
+
+int nint_plan_set_head_tangent(nint_plan* p, const float* dweight, const float* dbias, void* stream) {
+  if (param_tangent_check(p, "nint_plan_set_head_tangent")) return 1;
+  if (!dweight) return fail("nint_plan_set_head_tangent: null weight tangent");
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  CK(cudaMemcpyAsync(p->thead_w, dweight, p->layer[p->L - 1].hc_real * 4, cudaMemcpyDeviceToDevice, st));
+  if (dbias) CK(cudaMemcpyAsync(p->thead_b, dbias, 4, cudaMemcpyDeviceToDevice, st));
+  else CK(cudaMemsetAsync(p->thead_b, 0, 4, st));
+  p->dhead_set = true;
+  return 0;
+}
+
+int nint_plan_clear_param_tangent(nint_plan* p, void* stream) {
+  (void)stream;
+  if (param_tangent_check(p, "nint_plan_clear_param_tangent")) return 1;
+  for (int l = 0; l < p->L; ++l) p->layer[l].dw_set = p->layer[l].dbias_add = false;
+  p->dhead_set = false;
   return 0;
 }
 
@@ -1175,6 +1314,7 @@ static int forward_steps(nint_plan* p, float* pred, float* seq, cudaStream_t st)
   p->gates_valid = tr;
   p->bptt_done = false;
   p->tangent_kept = false;
+  p->soa_params = false;
   return 0;
 }
 
@@ -1684,17 +1824,47 @@ static int tangent_check(nint_plan* p, bool bank, const float* dseq) {
   return 0;
 }
 
+// the parameter direction's term of layer l's tangent gate GEMM at step t: dW (*) [x_t, h_{t-1}] over the forward's own
+// operands (its slots, bank windows and zero-state rule, as cell_step reads them) through the packed dW panels, added
+// into the dump `raw` that the tangent GEMM W (*) [dx_t, dh_{t-1}] wrote (EPI_RAW_ACC); on layer 0 with the constant-1
+// lane the GEMM also adds dbias
+static int param_tangent_gemm(nint_plan* p, int l, int t, float* raw, cudaStream_t st) {
+  Layer& y = p->layer[l];
+  const bool bank = l == 0 && p->x_bank;
+  const bool have_state = !(t == 0 && p->zero_init);
+  ConvGemmParams g;
+  if (fwd_conv_params(p, l, have_state, EPI_RAW_ACC, g)) return 1;
+  g.seg[0].slot = l == 0 ? t : t + 1;
+  g.seg[0].win_start = bank ? p->win_start : nullptr;
+  g.seg[0].bank_frames = bank ? static_cast<int>(p->bank_frames) : 0;
+  if (have_state) g.seg[1].slot = t;
+  for (int i = 0; i < g.nseg; ++i) {
+    g.seg[i].wsel += 4;
+    if (get_w_map(p, y, g.seg[i].wsel, g.n_tile, g.n_tile / g.cluster, g.seg[i].ts, &g.seg[i].tmap_w)) return 1;
+  }
+  g.slot_c_in = g.slot_c_out = g.slot_h_out = g.slot_g = g.slot_c_prev = -1;
+  g.raw_out = raw;
+  LAUNCH(p, K_FWD, st, launch_conv_halo(EPI_RAW_ACC, p->dtype, g, p->num_sms, st));
+  return 0;
+}
+
+// slot of dh_{s-1} in tH: a 2-slot ring, or the history of plans with both parameter-tangent and second-order flags
+inline int th_slot(const nint_plan* p, int s) { return p->hist ? s : (s & 1); }
+
 // the T x L tangent steps once the input tangent is in place (tX packed, or the tangent bank's map encoded)
 static int tangent_steps(nint_plan* p, const float* const* dh0, const float* const* dc0, float* dpred, float* dseq,
                          float* const* dh_T, float* const* dc_T, cudaStream_t st) {
   const long long HW = static_cast<long long>(p->H) * p->W;
   const long long npix = p->B * HW;
   const Layer& top = p->layer[p->L - 1];
+  bool any_param = p->dhead_set;
+  for (int l = 0; l < p->L; ++l) any_param = any_param || p->layer[l].dw_set;
   bool dh_in[NINT_MAX_LAYERS];
   for (int l = 0; l < p->L; ++l) {
     Layer& y = p->layer[l];
     dh_in[l] = dh0 && dh0[l];
     if (dh_in[l]) LAUNCH(p, K_OTHER, st, launch_pack_state(p->dtype, dh0[l], y.tH, p->B, y.hc_real, p->H, p->W, y.hc_pad, st));
+    else if (p->hist) CK(cudaMemsetAsync(y.tH, 0, act_bytes(p, 1, y.hc_pad), st));   // dh0 = 0 is read by the params call
     CK(cudaMemsetAsync(y.tC, 0, static_cast<size_t>(npix) * y.hc * 4, st));
     if (dc0 && dc0[l]) LAUNCH(p, K_OTHER, st, launch_nchw_to_nhwc_f32(dc0[l], y.tC, p->B, y.hc_real, p->H, p->W, y.hc, st));
   }
@@ -1708,38 +1878,55 @@ static int tangent_steps(nint_plan* p, const float* const* dh0, const float* con
       ConvGemmParams g;
       if (fwd_conv_params(p, l, rec, EPI_RAW, g)) return 1;
       g.seg[0].tmap_act = l == 0 ? (bank ? p->tmb_tX : p->tm_tX) : p->layer[l - 1].tm_tH_up;
-      g.seg[0].slot = l == 0 ? t : ((t + 1) & 1);
+      g.seg[0].slot = l == 0 ? t : th_slot(p, t + 1);
       g.seg[0].win_start = bank ? p->win_start : nullptr;
       g.seg[0].bank_frames = bank ? static_cast<int>(p->tbank_frames) : 0;
       if (rec) {
         g.seg[1].tmap_act = y.tm_tH;
-        g.seg[1].slot = t & 1;
+        g.seg[1].slot = th_slot(p, t);
       }
       g.slot_c_in = g.slot_c_out = g.slot_h_out = g.slot_g = g.slot_c_prev = -1;
       // second-order plans keep every step's dump and dc for nint_backward_second_order
       float* raw = p->second_order ? y.tR + static_cast<size_t>(t) * npix * 4 * y.hc : p->traw;
       g.raw_out = raw;
       LAUNCH(p, K_FWD, st, launch_conv_halo(EPI_RAW, p->dtype, g, p->num_sms, st));
+      if (y.dw_set && param_tangent_gemm(p, l, t, raw, st)) return 1;
       LAUNCH(p, K_OTHER, st, launch_tangent_cell(p->dtype, raw, slot_ptr(p, y.G, t, 4 * y.hc), cslot_ptr(p, y, t),
                                                  cslot_ptr(p, y, t + 1), tc_slot(p, y, t), tc_slot(p, y, t + 1),
-                                                 slot_ptr(p, y.tH, (t + 1) & 1, y.hc_pad), npix, y.hc, y.hc_pad, st));
+                                                 slot_ptr(p, y.tH, th_slot(p, t + 1), y.hc_pad), npix, y.hc, y.hc_pad, st,
+                                                 y.dbias_add ? y.tbias_q : nullptr));
     }
-    if (dseq)
-      LAUNCH(p, K_OTHER, st, launch_head_fwd(p->dtype, slot_ptr(p, top.tH, (t + 1) & 1, top.hc_pad), p->head_w, p->tzero,
-                                             dseq + t * HW, HW, p->B, top.hc_real, top.hc_pad, p->T * HW, st));
+    if (dseq) {
+      const void* dh = slot_ptr(p, top.tH, th_slot(p, t + 1), top.hc_pad);
+      if (p->dhead_set)
+        LAUNCH(p, K_OTHER, st, launch_head_tangent(p->dtype, slot_ptr(p, top.Hs, t + 1, top.hc_pad), dh, p->head_w,
+                                                   p->thead_w, p->thead_b, dseq + t * HW, HW, p->B, top.hc_real,
+                                                   top.hc_pad, p->T * HW, st));
+      else
+        LAUNCH(p, K_OTHER, st, launch_head_fwd(p->dtype, dh, p->head_w, p->tzero, dseq + t * HW, HW, p->B, top.hc_real,
+                                               top.hc_pad, p->T * HW, st));
+    }
   }
-  if (dpred)
-    LAUNCH(p, K_OTHER, st, launch_head_fwd(p->dtype, slot_ptr(p, top.tH, p->T & 1, top.hc_pad), p->head_w, p->tzero, dpred,
-                                           HW, p->B, top.hc_real, top.hc_pad, HW, st));
+  if (dpred) {
+    const void* dh = slot_ptr(p, top.tH, th_slot(p, p->T), top.hc_pad);
+    if (p->dhead_set)
+      LAUNCH(p, K_OTHER, st, launch_head_tangent(p->dtype, slot_ptr(p, top.Hs, p->T, top.hc_pad), dh, p->head_w, p->thead_w,
+                                                 p->thead_b, dpred, HW, p->B, top.hc_real, top.hc_pad, HW, st));
+    else
+      LAUNCH(p, K_OTHER, st, launch_head_fwd(p->dtype, dh, p->head_w, p->tzero, dpred, HW, p->B, top.hc_real, top.hc_pad,
+                                             HW, st));
+  }
   for (int l = 0; l < p->L; ++l) {
     const Layer& y = p->layer[l];
     if (dh_T && dh_T[l])
-      LAUNCH(p, K_OTHER, st, launch_unpack_state(p->dtype, slot_ptr(p, y.tH, p->T & 1, y.hc_pad), dh_T[l], p->B, y.hc_real,
+      LAUNCH(p, K_OTHER, st, launch_unpack_state(p->dtype, slot_ptr(p, y.tH, th_slot(p, p->T), y.hc_pad), dh_T[l], p->B, y.hc_real,
                                                  p->H, p->W, y.hc_pad, st));
     if (dc_T && dc_T[l])
       LAUNCH(p, K_OTHER, st, launch_nhwc_to_nchw_f32(tc_slot(p, y, p->T), dc_T[l], p->B, y.hc_real, p->H, p->W, y.hc, st));
   }
   p->tangent_kept = p->second_order;
+  p->param_in_tangent = any_param;
+  p->soa_params = false;
   return 0;
 }
 
@@ -1767,8 +1954,10 @@ int nint_forward_tangent_bank(nint_plan* p, const void* dbank, long long n_frame
     return fail("nint_forward_tangent_bank: %lld tangent frames for a bank of %lld", n_frames, p->bank_frames);
   if (reinterpret_cast<uintptr_t>(dbank) % 128) return fail("the tangent frame bank must be 128-byte aligned");
   if (dbank != p->tbank_ptr || n_frames != p->tbank_frames) {
-    if (encode_act_map(&p->tmb_tX, p->dtype, const_cast<void*>(dbank), p->layer[0].cx_pad, p->W, p->H,
-                       static_cast<int>(n_frames), 1, p->ce, p->tile_w, p->tile_h, false, p->layer[0].k / 2)) return 1;
+    if (p->hist) {   // the params call's wgrad reads the tangent frames too
+      if (encode_input_maps(p, const_cast<void*>(dbank), n_frames, 1, &p->tmb_tX, &p->tmbw_tX, &p->tmbp_tX)) return 1;
+    } else if (encode_act_map(&p->tmb_tX, p->dtype, const_cast<void*>(dbank), p->layer[0].cx_pad, p->W, p->H,
+                              static_cast<int>(n_frames), 1, p->ce, p->tile_w, p->tile_h, false, p->layer[0].k / 2)) return 1;
     p->tbank_ptr = dbank;
     p->tbank_frames = n_frames;
   }
@@ -1786,7 +1975,9 @@ static int soa_check(nint_plan* p, bool bank, const float* dpred, const float* d
   if (!p->gates_valid)
     return fail("nint_backward_second_order: the gates saved by the last forward were already consumed by a backward "
                 "(BPTT turns them into their gradients in place); run the forward again");
-  if (!p->tangent_kept) return fail("nint_backward_second_order before nint_forward_tangent of the last forward");
+  if (!p->tangent_kept)
+    return fail("nint_backward_second_order before nint_forward_tangent of the last forward (or the parameter direction "
+                "changed since)");
   if (bank && !p->x_bank)
     return fail("nint_backward_second_order_bank: the last forward did not read a frame bank (nint_forward_bank)");
   if (!bank && p->x_bank)
@@ -1797,35 +1988,56 @@ static int soa_check(nint_plan* p, bool bank, const float* dpred, const float* d
 }
 
 // EPI_RAW dgrad over the pass's dgates of both kinds (2B images: primal, then tangent) into p->sraw [2][npix][n_rows]:
-// segment i reads layer owner[i]'s dgates through its packed dgrad operand wsel[i] (2: x part, 3: h part)
-static int soa_dgrad(nint_plan* p, int l, int n_rows, int nseg, const int* owner, const int* wsel, cudaStream_t st) {
+// segment i reads layer owner[i]'s dgates through its packed dgrad operand wsel[i] (2: x part, 3: h part) at step slot
+// slot[i] of the history (slot 0 of the single step on plans without it).  dW = true: the parameter direction's
+// dW^T terms instead -- operands 6 / 7 (dW's dgrad panels) over the PRIMAL dgates only (B images), added into the
+// tangent half of the dump (EPI_RAW_ACC); layers without a direction are left out
+static int soa_dgrad(nint_plan* p, int l, int n_rows, int nseg, const int* owner, const int* wsel, const int* slot,
+                     bool dW, cudaStream_t st) {
   Layer& y = p->layer[l];
   ConvGemmParams g;
   fill_common(p, y, g);
-  g.B = 2 * p->B;
+  g.B = dW ? p->B : 2 * p->B;
   g.n_tile = n_rows;
   g.n_blocks = 1;
   g.cluster = (n_rows % 32 == 0) ? p->cluster : 1;
   g.idesc = idesc_of(p->dtype, 128 * g.cluster, n_rows, 0, 0);
+  int n = 0;
   for (int i = 0; i < nseg; ++i) {
     const Layer& o = p->layer[owner[i]];
-    g.seg[i].tmap_act = o.tm_sA; g.seg[i].wsel = wsel[i]; g.seg[i].slot = 0;
-    g.seg[i].ksize = o.k; g.seg[i].nchunks = 4 * o.hc / p->ce;
+    if (dW && !o.dw_set) continue;
+    g.seg[n].tmap_act = o.tm_sA; g.seg[n].wsel = wsel[i] + (dW ? 4 : 0); g.seg[n].slot = p->hist ? slot[i] : 0;
+    g.seg[n].ksize = o.k; g.seg[n].nchunks = 4 * o.hc / p->ce;
+    ++n;
   }
-  g.nseg = nseg;
+  if (n == 0) return 0;
+  g.nseg = n;
   g.tm_c = y.tme_C; g.tm_h = y.tme_H; g.tm_g = y.tme_G; g.tm_dc = y.tme_dC;
   g.slot_g = g.slot_c_in = g.slot_c_out = g.slot_h_out = g.slot_c_prev = -1;
-  g.raw_out = p->sraw;
-  if (conv_halo_plan(EPI_RAW, p->dtype, g))
+  g.raw_out = dW ? p->sraw + static_cast<size_t>(p->B) * p->H * p->W * n_rows : p->sraw;
+  const int epi = dW ? EPI_RAW_ACC : EPI_RAW;
+  if (conv_halo_plan(epi, p->dtype, g))
     return fail("layer %d: the second-order dgrad's shared-memory plan does not fit (N %d, k %d)", l, n_rows, y.k);
-  for (int i = 0; i < nseg; ++i)
-    if (get_w_map(p, p->layer[owner[i]], wsel[i], g.n_tile, g.n_tile / g.cluster, g.seg[i].ts, &g.seg[i].tmap_w)) return 1;
-  LAUNCH(p, K_OTHER, st, launch_conv_halo(EPI_RAW, p->dtype, g, p->num_sms, st));
+  int k = 0;
+  for (int i = 0; i < nseg; ++i) {
+    if (dW && !p->layer[owner[i]].dw_set) continue;
+    if (get_w_map(p, p->layer[owner[i]], g.seg[k].wsel, g.n_tile, g.n_tile / g.cluster, g.seg[k].ts, &g.seg[k].tmap_w)) return 1;
+    ++k;
+  }
+  LAUNCH(p, K_OTHER, st, launch_conv_halo(epi, p->dtype, g, p->num_sms, st));
   return 0;
 }
 
+// the primal and tangent dgrad of (a, da), then, when the tangent pass had a parameter direction, its dW^T terms
+static int soa_dgrad_all(nint_plan* p, int l, int n_rows, int nseg, const int* owner, const int* wsel, const int* slot,
+                         cudaStream_t st) {
+  if (soa_dgrad(p, l, n_rows, nseg, owner, wsel, slot, false, st)) return 1;
+  return p->param_in_tangent ? soa_dgrad(p, l, n_rows, nseg, owner, wsel, slot, true, st) : 0;
+}
+
 // the reverse loop once the checks passed: per step t (descending) and layer l (top first) eta = one dgrad, then
-// soa_cell_kernel; layer 0's x part goes to dx / ddx (explicit windows) or is added into dframes / ddframes (bank)
+// soa_cell_kernel; layer 0's x part goes to dx / ddx (explicit windows) or is added into dframes / ddframes (bank).
+// Plans with both parameter flags also reduce the head's parameter gradient and H v terms into p->head_sums.
 static int soa_steps(nint_plan* p, const float* dpred, const float* dseq, const float* ddpred, const float* ddseq,
                      float* dx, float* ddx, float* dframes, float* ddframes, float* const* dh0, float* const* dc0,
                      float* const* ddh0, float* const* ddc0, cudaStream_t st) {
@@ -1833,15 +2045,19 @@ static int soa_steps(nint_plan* p, const float* dpred, const float* dseq, const 
   const long long npix = p->B * HW;
   const int L = p->L, T = p->T, C = p->cfg.in_channels;
   const Layer& y0 = p->layer[0];
+  const Layer& top = p->layer[L - 1];
   const long long xs = static_cast<long long>(npix) * y0.cin_rows;   // tangent half of a dx dump
   for (int l = 0; l < L; ++l) CK(cudaMemsetAsync(p->layer[l].sK, 0, 2 * static_cast<size_t>(npix) * p->layer[l].hc * 4, st));
+  float* hs = p->head_sums;   // {grad w [hc], grad b, hvp w [hc], hvp b, scratch}
+  float* hpart = p->deterministic ? p->head_part : nullptr;
+  if (p->hist) CK(cudaMemsetAsync(hs, 0, static_cast<size_t>(2 * (top.hc + 1) + 1) * 4, st));
   for (int t = T - 1; t >= 0; --t) {
     for (int l = L - 1; l >= 0; --l) {
       Layer& y = p->layer[l];
-      int owner[2], wsel[2], n = 0;
-      if (t < T - 1) { owner[n] = l; wsel[n++] = 3; }       // dh_t += da_{t+1} (*) flip(W_h)
-      if (l < L - 1) { owner[n] = l + 1; wsel[n++] = 2; }   // dh_t += the layer above's x part at t
-      if (n && soa_dgrad(p, l, y.hc, n, owner, wsel, st)) return 1;
+      int owner[2], wsel[2], slot[2], n = 0;
+      if (t < T - 1) { owner[n] = l; wsel[n] = 3; slot[n++] = t + 1; }       // dh_t += da_{t+1} (*) flip(W_h)
+      if (l < L - 1) { owner[n] = l + 1; wsel[n] = 2; slot[n++] = t; }       // dh_t += the layer above's x part at t
+      if (n && soa_dgrad_all(p, l, y.hc, n, owner, wsel, slot, st)) return 1;
       const float *u = nullptr, *du = nullptr;
       long long ub = 0, dub = 0;
       if (l == L - 1) {
@@ -1850,14 +2066,28 @@ static int soa_steps(nint_plan* p, const float* dpred, const float* dseq, const 
         ub = dseq ? T * HW : HW;
         dub = ddseq ? T * HW : HW;
       }
+      uint8_t* da = p->hist ? slot_ptr(p, y.sA, 2 * t, 4 * y.hc) : y.sA;
       LAUNCH(p, K_OTHER, st, launch_soa_cell(p->dtype, n ? p->sraw : nullptr, u, ub, du, dub, p->head_w,
                                              slot_ptr(p, y.G, t, 4 * y.hc), y.tR + static_cast<size_t>(t) * npix * 4 * y.hc,
                                              cslot_ptr(p, y, t), cslot_ptr(p, y, t + 1), tc_slot(p, y, t),
-                                             tc_slot(p, y, t + 1), y.sK, y.sA, npix, HW, y.hc, st));
+                                             tc_slot(p, y, t + 1), y.sK, da, npix, HW, y.hc, st,
+                                             p->dhead_set ? p->thead_w : nullptr));
+      // head parameters: grad w += u h_t, grad b += u; H v: w += du h_t + u dh_t, b += du
+      if (p->hist && l == L - 1) {
+        const uint8_t* h = slot_ptr(p, top.Hs, t + 1, top.hc_pad);
+        const uint8_t* dh = slot_ptr(p, top.tH, t + 1, top.hc_pad);
+        float *gw = hs, *gb = hs + top.hc, *hw = hs + top.hc + 1, *hb = hs + 2 * top.hc + 1;
+        if (u) {
+          LAUNCH(p, K_OTHER, st, launch_head_bwd(p->dtype, h, u, ub, gw, gb, HW, p->B, top.hc_real, top.hc_pad, hpart, st));
+          // u dh_t reaches only the weight: its bias sum goes to a scratch slot
+          LAUNCH(p, K_OTHER, st, launch_head_bwd(p->dtype, dh, u, ub, hw, hb + 1, HW, p->B, top.hc_real, top.hc_pad, hpart, st));
+        }
+        if (du) LAUNCH(p, K_OTHER, st, launch_head_bwd(p->dtype, h, du, dub, hw, hb, HW, p->B, top.hc_real, top.hc_pad, hpart, st));
+      }
     }
     if (dx || ddx || dframes || ddframes) {
       const int owner = 0, wsel = 2;
-      if (soa_dgrad(p, 0, y0.cin_rows, 1, &owner, &wsel, st)) return 1;
+      if (soa_dgrad_all(p, 0, y0.cin_rows, 1, &owner, &wsel, &t, st)) return 1;
       const long long xstride = static_cast<long long>(T) * C * HW;
       if (dx) LAUNCH(p, K_OTHER, st, launch_unpack_raw(p->sraw, dx + t * C * HW, p->B, C, p->H, p->W, y0.cin_rows, xstride, st));
       if (ddx) LAUNCH(p, K_OTHER, st, launch_unpack_raw(p->sraw + xs, ddx + t * C * HW, p->B, C, p->H, p->W, y0.cin_rows, xstride, st));
@@ -1872,19 +2102,20 @@ static int soa_steps(nint_plan* p, const float* dpred, const float* dseq, const 
   // initial state: h_{-1} enters only layer l's gate GEMM at t = 0, so dh0 = da_0 (*) flip(W_h); dc0 = kappa after t = 0
   for (int l = 0; l < L; ++l) {
     Layer& y = p->layer[l];
-    const long long hs = static_cast<long long>(npix) * y.hc;
+    const long long hs_ = static_cast<long long>(npix) * y.hc;
     const bool h = dh0 && dh0[l], dh = ddh0 && ddh0[l];
     if (h || dh) {
-      const int wsel = 3;
-      if (soa_dgrad(p, l, y.hc, 1, &l, &wsel, st)) return 1;
+      const int wsel = 3, slot = 0;
+      if (soa_dgrad_all(p, l, y.hc, 1, &l, &wsel, &slot, st)) return 1;
       const long long bs = static_cast<long long>(y.hc_real) * HW;
       if (h) LAUNCH(p, K_OTHER, st, launch_unpack_raw(p->sraw, dh0[l], p->B, y.hc_real, p->H, p->W, y.hc, bs, st));
-      if (dh) LAUNCH(p, K_OTHER, st, launch_unpack_raw(p->sraw + hs, ddh0[l], p->B, y.hc_real, p->H, p->W, y.hc, bs, st));
+      if (dh) LAUNCH(p, K_OTHER, st, launch_unpack_raw(p->sraw + hs_, ddh0[l], p->B, y.hc_real, p->H, p->W, y.hc, bs, st));
     }
     if (dc0 && dc0[l]) LAUNCH(p, K_OTHER, st, launch_nhwc_to_nchw_f32(y.sK, dc0[l], p->B, y.hc_real, p->H, p->W, y.hc, st));
     if (ddc0 && ddc0[l])
-      LAUNCH(p, K_OTHER, st, launch_nhwc_to_nchw_f32(y.sK + hs, ddc0[l], p->B, y.hc_real, p->H, p->W, y.hc, st));
+      LAUNCH(p, K_OTHER, st, launch_nhwc_to_nchw_f32(y.sK + hs_, ddc0[l], p->B, y.hc_real, p->H, p->W, y.hc, st));
   }
+  p->soa_params = p->hist;
   return 0;
 }
 
@@ -1902,6 +2133,71 @@ int nint_backward_second_order_bank(nint_plan* p, const float* dpred, const floa
   if (soa_check(p, true, dpred, dseq, ddpred, ddseq)) return 1;
   return soa_steps(p, dpred, dseq, ddpred, ddseq, nullptr, nullptr, dframes, ddframes, dh0, dc0, ddh0, ddc0,
                    static_cast<cudaStream_t>(stream));
+}
+
+// one wgrad reduction of the parameter outputs over all T steps of layer l into gw / gb (accumulate: add):
+// kind 0 = wgrad(a, comb) (the gradient), 1 = wgrad(da, comb), 2 = wgrad(a, dcomb) -- the ordinary wgrad's launches
+// with the pass's (a, da) history as the dgates operand and, for kind 2, the input tangent and dh history as the
+// activations.  Kind 2 has no bias term: the caller passes gb = NULL (its bias column / sum is not read)
+static int param_wgrad(nint_plan* p, int l, int kind, float* gw, float* gb, int accumulate, cudaStream_t st) {
+  Layer& y = p->layer[l];
+  const size_t slices = p->deterministic ? static_cast<size_t>(y.det_splits) : 1;
+  CK(cudaMemsetAsync(y.dw_acc, 0, y.dw_acc_bytes * slices, st));
+  CK(cudaMemsetAsync(y.db_acc, 0, 4 * y.hc * 4 * slices, st));
+  const bool bank = l == 0 && p->x_bank;
+  for (size_t bi = 0; bi < y.wg_blocks.size(); ++bi) {
+    WgradParams w;
+    if (wgrad_params(p, l, bi, p->num_sms, w)) return 1;
+    const Layer::WgBlock& blk = y.wg_blocks[bi];
+    const bool pv = w.pair && p->dtype == BF16;   // CTA-pair boxes, else the 32-channel wgrad boxes
+    w.tmap_dg = pv ? y.tmp_sA[kind == 1 ? 1 : 0] : y.tmw_sA[kind == 1 ? 1 : 0];
+    if (kind == 2) {
+      if (l == 0) w.tmap_b[0] = bank ? (pv ? p->tmbp_tX : p->tmbw_tX) : (pv ? p->tmp_tX : p->tmw_tX);
+      else w.tmap_b[0] = pv ? p->layer[l - 1].tmp_tH_up : p->layer[l - 1].tmw_tH_up;
+      w.tmap_b[1] = pv ? y.tmp_tH : y.tmw_tH;
+      if (blk.nch_x == 0) w.tmap_b[0] = w.tmap_b[1];
+      if (blk.nch_h == 0) w.tmap_b[1] = w.tmap_b[0];
+    }
+    if (p->deterministic && wgrad_max_splits(w) > y.det_splits)
+      return fail("deterministic wgrad: this device splits the reduction %d ways, the plan reserved %d slices", wgrad_max_splits(w), y.det_splits);
+    LAUNCH(p, K_WGRAD, st, launch_wgrad(p->dtype, w, st));
+  }
+  LAUNCH(p, K_OTHER, st, launch_unpack_wgrad(y.dw_acc, y.db_acc, gw, gb, y.cin, y.hc_real, y.hc, y.k, y.ncols, y.cx_pad,
+                                             l == 0 ? p->ones_lane : -1, accumulate, p->deterministic ? y.det_splits : 0,
+                                             nullptr, 0, st));
+  return 0;
+}
+
+int nint_backward_second_order_params(nint_plan* p, float* const* grad_weight, float* const* grad_bias,
+                                      float* const* hvp_weight, float* const* hvp_bias, float* grad_head_weight,
+                                      float* grad_head_bias, float* hvp_head_weight, float* hvp_head_bias, void* stream) {
+  if (check_ready(p)) return 1;
+  if (!p->cfg.training || !p->hist)
+    return fail("nint_backward_second_order_params needs a training plan created with NINT_FLAG_SECOND_ORDER | "
+                "NINT_FLAG_PARAM_TANGENT");
+  if (!p->gates_valid)
+    return fail("nint_backward_second_order_params: the gates saved by the last forward were already consumed by a "
+                "backward; run the forward again");
+  if (!p->soa_params)
+    return fail("nint_backward_second_order_params before nint_backward_second_order[_bank] of the current forward, "
+                "tangent pass and parameter direction");
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  for (int l = 0; l < p->L; ++l) {
+    if (grad_weight && grad_weight[l] && param_wgrad(p, l, 0, grad_weight[l], grad_bias ? grad_bias[l] : nullptr, 0, st))
+      return 1;
+    if (hvp_weight && hvp_weight[l]) {   // term 1, then term 2 added: a fixed order (deterministic plans stay bit-exact)
+      if (param_wgrad(p, l, 1, hvp_weight[l], hvp_bias ? hvp_bias[l] : nullptr, 0, st)) return 1;
+      if (param_wgrad(p, l, 2, hvp_weight[l], nullptr, 1, st)) return 1;
+    }
+  }
+  const Layer& top = p->layer[p->L - 1];
+  const float* hs = p->head_sums;
+  const size_t hb = static_cast<size_t>(top.hc_real) * 4;
+  if (grad_head_weight) CK(cudaMemcpyAsync(grad_head_weight, hs, hb, cudaMemcpyDeviceToDevice, st));
+  if (grad_head_bias) CK(cudaMemcpyAsync(grad_head_bias, hs + top.hc, 4, cudaMemcpyDeviceToDevice, st));
+  if (hvp_head_weight) CK(cudaMemcpyAsync(hvp_head_weight, hs + top.hc + 1, hb, cudaMemcpyDeviceToDevice, st));
+  if (hvp_head_bias) CK(cudaMemcpyAsync(hvp_head_bias, hs + 2 * top.hc + 1, 4, cudaMemcpyDeviceToDevice, st));
+  return 0;
 }
 
 int nint_cell_forward(nint_plan* p, const float* x, const float* h, const float* c, float* h_out, float* c_out,

@@ -117,7 +117,7 @@ __global__ void __launch_bounds__(kConvThreads, 1) conv_halo_kernel(const __grid
       prefetch_tensormap(&p.seg[s].tmap_w);
     }
   }
-  if (warp == 3 && lane == 0 && EPI != EPI_RAW) {
+  if (warp == 3 && lane == 0 && !epi_is_raw(EPI)) {
     prefetch_tensormap(&p.tm_c);
     prefetch_tensormap(&p.tm_g);
     prefetch_tensormap(EPI == EPI_FWD ? &p.tm_h : &p.tm_dc);
@@ -333,7 +333,7 @@ __global__ void __launch_bounds__(kConvThreads, 1) conv_halo_kernel(const __grid
   };
 
   // two activation producers when a tile needs many chunk loads (dgrad: K = 4*hc channels, G tiles per chunk)
-  const bool a_split = (EPI != EPI_RAW);   // one producer warp cannot issue a box per 1152-cycle chunk (timeline: 670 cycles per box + waits)
+  const bool a_split = !epi_is_raw(EPI);   // one producer warp cannot issue a box per 1152-cycle chunk (timeline: 670 cycles per box + waits)
 
   if (warp == 0) {
     if (p.nseg > 0) produce(true, 0, a_split ? 2 : 1, false);
@@ -607,8 +607,8 @@ __global__ void __launch_bounds__(kConvThreads, 1) conv_halo_kernel(const __grid
     // the epilogue of either CTA releases the accumulator buffer on the LEADER's "tmem empty" barrier
     uint32_t tempty_remote = 0;
     if constexpr (pair) tempty_remote = mapa_rank(smem_u32(&tempty_bar[0]), 0);
-    if constexpr (EPI == EPI_RAW)
-      epi_raw(p, warp, lane, tmem_base, tfull_bar, tempty_bar, walk, tempty_remote);
+    if constexpr (epi_is_raw(EPI))
+      epi_raw<EPI == EPI_RAW_ACC>(p, warp, lane, tmem_base, tfull_bar, tempty_bar, walk, tempty_remote);
     else if constexpr (EPI == EPI_FWD)
       fwd_math<E, FUSED>(p, warp, lane, tmem_base, sE, FwdEpiBars{e_full, e_empty, st_ready, hg_ready, hg_empty}, tfull_bar,
                   tempty_bar, s_bias, walk, tempty_remote);
@@ -651,7 +651,7 @@ int conv_halo_plan(int epi, int dtype, ConvGemmParams& p) {
   if (p.a_halo_bytes == 0) p.a_halo_bytes = 1024;
   const int total = 227 * 1024 - 1024 - kHaloCtrlBytes - (4 * p.hc + p.hc) * 4 - 1024 - p.c_ring * kEpiBoxBytes16;
   const int w_bytes = (p.n_tile / p.cluster) * kChunkBytes;
-  const int ns_max = epi == EPI_RAW ? 0 : (epi == EPI_FWD ? 2 : 3), ns_min = epi == EPI_RAW ? 0 : 2;
+  const int ns_max = epi_is_raw(epi) ? 0 : (epi == EPI_FWD ? 2 : 3), ns_min = epi_is_raw(epi) ? 0 : 2;
   int max_k = 1;
   for (int s = 0; s < p.nseg; ++s) if (p.seg[s].ksize > max_k) max_k = p.seg[s].ksize;
   // ---- plan A: weights resident.  One stage per (segment, chunk) holding all taps; needs >= 3 halo buffers.
@@ -817,6 +817,7 @@ static cudaError_t launch_e(int epi, const ConvGemmParams& p, int num_sms, cudaS
   if (epi == EPI_FWD) return fused ? launch_h<E, EPI_FWD, PAIR, true>(p, num_sms, stream) : launch_h<E, EPI_FWD, PAIR, false>(p, num_sms, stream);
   if (epi == EPI_BWD) return fused ? launch_h<E, EPI_BWD, PAIR, true>(p, num_sms, stream) : launch_h<E, EPI_BWD, PAIR, false>(p, num_sms, stream);
   if (fused) return cudaErrorInvalidValue;
+  if (epi == EPI_RAW_ACC) return launch_h<E, EPI_RAW_ACC, PAIR, false>(p, num_sms, stream);
   return launch_h<E, EPI_RAW, PAIR, false>(p, num_sms, stream);
 }
 
@@ -825,7 +826,7 @@ cudaError_t launch_conv_halo(int epi, int dtype, const ConvGemmParams& p, int nu
   if (p.cluster != 1 && p.cluster != 2) return cudaErrorInvalidValue;
   if (p.cluster == 2 && (p.n_tile % 32)) return cudaErrorInvalidValue;
   if (p.n_acc < 1 || p.n_acc > kMaxAcc || p.n_acc * p.acc_cols > kTmemCols) return cudaErrorInvalidValue;
-  if (epi != EPI_RAW && (p.e_stages < 2 || p.e_stages > kEpiMaxStages)) return cudaErrorInvalidValue;
+  if (!epi_is_raw(epi) && (p.e_stages < 2 || p.e_stages > kEpiMaxStages)) return cudaErrorInvalidValue;
   if (dtype == NINT_BF16)
     return p.cluster == 2 ? launch_e<__nv_bfloat16, true>(epi, p, num_sms, stream)
                           : launch_e<__nv_bfloat16, false>(epi, p, num_sms, stream);

@@ -858,7 +858,9 @@ __device__ __forceinline__ void epi_math(const ConvGemmParams& p, int warp, int 
   }
 }
 
-// debug epilogue: dump the fp32 accumulators [B,H,W,n_blocks*n_tile] (nint_debug_raw_gates)
+// dump the fp32 accumulators [B,H,W,n_blocks*n_tile] (nint_debug_raw_gates, dgrad, the tangent GEMM); ACC: add them to
+// what the dump holds (every element belongs to one thread of the launch: a plain read-add-write)
+template <bool ACC>
 __device__ __forceinline__ void epi_raw(const ConvGemmParams& p, int warp, int lane, uint32_t tmem_base,
                                         uint64_t* tfull_bar, uint64_t* tempty_bar, const TileWalk& w,
                                         uint32_t tempty_remote) {
@@ -885,6 +887,14 @@ __device__ __forceinline__ void epi_raw(const ConvGemmParams& p, int warp, int l
         float v[16];
         tmem_ld16(taddr + c0, v);
         tmem_ld_wait();
+        if constexpr (ACC) {
+          if (valid) {
+            float o[16];
+            load_elems<float, 16>(ro + c0, o);
+#pragma unroll
+            for (int j = 0; j < 16; ++j) v[j] += o[j];
+          }
+        }
         if (valid) store_elems<float, 16>(ro + c0, v);
       }
     }

@@ -26,7 +26,10 @@
 
 namespace nint {
 
-enum : int { EPI_FWD = 0, EPI_BWD = 1, EPI_RAW = 2 };
+// EPI_RAW_ACC: EPI_RAW that adds the accumulators into the dump instead of overwriting it (a second GEMM summed into the
+// first one's dump: the parameter tangent's dW (*) comb_t on top of W (*) dcomb_t)
+enum : int { EPI_FWD = 0, EPI_BWD = 1, EPI_RAW = 2, EPI_RAW_ACC = 3 };
+__host__ __device__ constexpr bool epi_is_raw(int epi) { return epi == EPI_RAW || epi == EPI_RAW_ACC; }
 
 // One K-segment of an implicit-GEMM convolution: an activation tensor read through a 5-D TMA
 // map (box = one chunk x tile_w x tile_h pixels; out-of-image pixels are zero-filled by TMA =
@@ -86,7 +89,7 @@ struct alignas(64) ConvGemmParams {
   // every (CTA, pixel quadrant) adds into its own slots (deterministic), reduced by unpack_wgrad_kernel
   float* db_resid;
   const float* dh_ext;      // optional [B,H,W,hc] fp32 channels-last: dh += dh_ext (standalone cell backward, model.py:216-231)
-  // ---- EPI_RAW: dump fp32 accumulators [B,H,W,n_blocks*n_tile] (debug / generic conv)
+  // ---- EPI_RAW: dump fp32 accumulators [B,H,W,n_blocks*n_tile] (debug / generic conv); EPI_RAW_ACC adds into it
   float* raw_out;
   // ---- time-fused launch: n_steps > 1 consecutive time steps of one layer run as ONE persistent launch.  The tile walk
   // covers n_steps x tiles (step-major); in step s every slot field advances by its `d_*` (forward +1, BPTT -1; fields in
@@ -185,6 +188,11 @@ cudaError_t launch_pack_weights_bwd(int dtype, const float* w, void* wpack_dx, v
 // 1x1 head (model.py:251,274)
 cudaError_t launch_head_fwd(int dtype, const void* h, const float* w, const float* b, float* out, long long npix_per_img,
                             int B, int hc, int hc_pad, long long out_bstride, cudaStream_t s);
+// tangent of the head with a parameter direction: out = db + sum_c dh[pix][c] w[c] + h[pix][c] dw[c] (one pass over
+// the primal and the tangent h; model.py:274 differentiated in (h, w, b))
+cudaError_t launch_head_tangent(int dtype, const void* h, const void* dh, const float* w, const float* dw, const float* db,
+                                float* out, long long npix_per_img, int B, int hc, int hc_pad, long long out_bstride,
+                                cudaStream_t s);
 // part: null (fp32 atomics) or head_bwd_blocks(B) * (hc + 1) floats of scratch (deterministic fixed-order sum)
 int head_bwd_blocks(int B);
 cudaError_t launch_head_bwd(int dtype, const void* h, const float* dpred, long long dpred_bstride, float* dw, float* db,
@@ -207,9 +215,12 @@ cudaError_t launch_accum_frames(const float* raw, float* dframes, const int* win
 // columns halved like the packed forward weights), gates = the forward's activated gates of this step [npix][4*hc] E,
 // c_prev / c_cur = c_{t-1} / c_t [npix][hc] fp32; dc_in = dc_{t-1}, dc_out = dc_t [npix][hc] fp32 (the same buffer:
 // updated in place), dh_out [npix][hc_pad] E gets dh_t (lanes >= hc are not written)
-cudaError_t launch_tangent_cell(int dtype, const float* raw, const void* gates, const float* c_prev, const float* c_cur,
+// dbias_q: null, or the parameter tangent's q-order bias [4*hc] (i/f/o halved like bias_q) added to raw and stored back
+// into it (the dump then holds the whole tangent pre-activation) -- a separate kernel (tangent_cell_bias_kernel), so the
+// launch without it is unchanged
+cudaError_t launch_tangent_cell(int dtype, float* raw, const void* gates, const float* c_prev, const float* c_cur,
                                 const float* dc_in, float* dc_out, void* dh_out, long long npix, int hc, int hc_pad,
-                                cudaStream_t s);
+                                cudaStream_t s, const float* dbias_q = nullptr);
 
 // second-order adjoint cell step (nint_backward_second_order), per (pixel, hidden channel): eta = [2][npix][hc] fp32
 // dgrad dump (dL/dh_t and its tangent; NULL = 0), u / du = dL/dpred and its tangent at this step (NULL = 0; pixel
@@ -220,7 +231,8 @@ cudaError_t launch_tangent_cell(int dtype, const float* raw, const void* gates, 
 cudaError_t launch_soa_cell(int dtype, const float* eta, const float* u, long long u_bstride, const float* du,
                             long long du_bstride, const float* head_w, const void* gates, const float* traw,
                             const float* c_prev, const float* c_cur, const float* dc_prev, const float* dc_cur,
-                            float* kappa, void* da_out, long long npix, long long HW, int hc, cudaStream_t s);
+                            float* kappa, void* da_out, long long npix, long long HW, int hc, cudaStream_t s,
+                            const float* dhead_w = nullptr);   // dhead_w: the head weight's tangent (soa_cell_dhead_kernel)
 
 // preprocessing fusion: stack levels + emission, z-score, cyclic-longitude / reflect-latitude halo
 cudaError_t launch_fuse_inputs(const float* lev, const float* emis, const float* mean, const float* stdv,

@@ -330,11 +330,13 @@ cudaError_t launch_nhwc_to_nchw_f32(const float* src, float* dst, int B, int C, 
 // (zero weights) get raw = 0 and c = 0, so their dc and dh stay exactly 0.  dc_in / dc_out: the same buffer (updated in
 // place) or, on NINT_FLAG_SECOND_ORDER plans, consecutive slots of the per-step dc history the second-order pass reads.
 // ------------------------------------------------------------------------------------------
-template <typename E>
-__global__ void __launch_bounds__(256) tangent_cell_kernel(const float* __restrict__ raw, const E* __restrict__ gates,
-                                                           const float* __restrict__ c_prev, const float* __restrict__ c_cur,
-                                                           const float* dc_in, float* dc_out, E* __restrict__ dh_out,
-                                                           long long npix, int hc, int hc_pad) {
+// BIAS: add the parameter tangent's q-order bias dbias_q [4*hc] (i/f/o halved like raw) to raw first, and store the
+// sum back into raw, so the dump holds the whole tangent pre-activation (the second-order pass linearises at it)
+template <typename E, bool BIAS>
+__device__ __forceinline__ void tangent_cell_body(float* __restrict__ raw, const E* __restrict__ gates,
+                                                  const float* __restrict__ c_prev, const float* __restrict__ c_cur,
+                                                  const float* dc_in, float* dc_out, E* __restrict__ dh_out, long long npix,
+                                                  int hc, int hc_pad, const float* __restrict__ dbias_q) {
   constexpr bool FAST = std::is_same<E, __nv_bfloat16>::value;   // the forward's activation variant (nint_common.cuh)
   const int groups = hc / 8;
   const long long total = npix * groups;
@@ -354,6 +356,16 @@ __global__ void __launch_bounds__(256) tangent_cell_kernel(const float* __restri
     load_elems<float, 8>(c_prev + ci, cp);
     load_elems<float, 8>(c_cur + ci, cc);
     load_elems<float, 8>(dc_in + ci, d);
+    if constexpr (BIAS) {
+#pragma unroll
+      for (int k = 0; k < 4; ++k) {
+        float b[8];
+        load_elems<float, 8>(dbias_q + q0 + k * 16, b);
+#pragma unroll
+        for (int j = 0; j < 8; ++j) a[k][j] += b[j];
+        store_elems<float, 8>(raw + pix * 4 * hc + q0 + k * 16, a[k]);
+      }
+    }
     float h[8];
 #pragma unroll
     for (int j = 0; j < 8; ++j) {
@@ -373,20 +385,47 @@ __global__ void __launch_bounds__(256) tangent_cell_kernel(const float* __restri
   }
 }
 
-cudaError_t launch_tangent_cell(int dtype, const float* raw, const void* gates, const float* c_prev, const float* c_cur,
+template <typename E>
+__global__ void __launch_bounds__(256) tangent_cell_kernel(const float* __restrict__ raw, const E* __restrict__ gates,
+                                                           const float* __restrict__ c_prev, const float* __restrict__ c_cur,
+                                                           const float* dc_in, float* dc_out, E* __restrict__ dh_out,
+                                                           long long npix, int hc, int hc_pad) {
+  tangent_cell_body<E, false>(const_cast<float*>(raw), gates, c_prev, c_cur, dc_in, dc_out, dh_out, npix, hc, hc_pad, nullptr);
+}
+
+// the same with a parameter tangent's bias (layers whose bias is not folded into the GEMM through the constant-1 lane)
+template <typename E>
+__global__ void __launch_bounds__(256) tangent_cell_bias_kernel(float* __restrict__ raw, const E* __restrict__ gates,
+                                                                const float* __restrict__ c_prev,
+                                                                const float* __restrict__ c_cur, const float* dc_in,
+                                                                float* dc_out, E* __restrict__ dh_out, long long npix,
+                                                                int hc, int hc_pad, const float* __restrict__ dbias_q) {
+  tangent_cell_body<E, true>(raw, gates, c_prev, c_cur, dc_in, dc_out, dh_out, npix, hc, hc_pad, dbias_q);
+}
+
+template <typename E>
+static void launch_tangent_cell_e(long long blocks, float* raw, const void* gates, const float* c_prev,
+                                  const float* c_cur, const float* dc_in, float* dc_out, void* dh_out, long long npix,
+                                  int hc, int hc_pad, cudaStream_t s, const float* dbias_q) {
+  const E* g = reinterpret_cast<const E*>(gates);
+  E* dh = reinterpret_cast<E*>(dh_out);
+  if (dbias_q)
+    tangent_cell_bias_kernel<E><<<blocks, 256, 0, s>>>(raw, g, c_prev, c_cur, dc_in, dc_out, dh, npix, hc, hc_pad, dbias_q);
+  else
+    tangent_cell_kernel<E><<<blocks, 256, 0, s>>>(raw, g, c_prev, c_cur, dc_in, dc_out, dh, npix, hc, hc_pad);
+}
+
+cudaError_t launch_tangent_cell(int dtype, float* raw, const void* gates, const float* c_prev, const float* c_cur,
                                 const float* dc_in, float* dc_out, void* dh_out, long long npix, int hc, int hc_pad,
-                                cudaStream_t s) {
+                                cudaStream_t s, const float* dbias_q) {
   const long long total = npix * (hc / 8);
   long long blocks = (total + 255) / 256;
   if (blocks > 148 * 16) blocks = 148 * 16;
   if (blocks <= 0) return cudaSuccess;
   if (dtype == NINT_BF16)
-    tangent_cell_kernel<__nv_bfloat16><<<blocks, 256, 0, s>>>(raw, reinterpret_cast<const __nv_bfloat16*>(gates), c_prev,
-                                                               c_cur, dc_in, dc_out,
-                                                               reinterpret_cast<__nv_bfloat16*>(dh_out), npix, hc, hc_pad);
+    launch_tangent_cell_e<__nv_bfloat16>(blocks, raw, gates, c_prev, c_cur, dc_in, dc_out, dh_out, npix, hc, hc_pad, s, dbias_q);
   else
-    tangent_cell_kernel<float><<<blocks, 256, 0, s>>>(raw, reinterpret_cast<const float*>(gates), c_prev, c_cur, dc_in,
-                                                      dc_out, reinterpret_cast<float*>(dh_out), npix, hc, hc_pad);
+    launch_tangent_cell_e<float>(blocks, raw, gates, c_prev, c_cur, dc_in, dc_out, dh_out, npix, hc, hc_pad, s, dbias_q);
   return cudaGetLastError();
 }
 
@@ -406,15 +445,16 @@ cudaError_t launch_tangent_cell(int dtype, const float* raw, const void* gates, 
 // the operand format: the packed dgrad panels apply unchanged).  Thread layout and load order as tangent_cell_kernel;
 // padded hidden channels have zero raw, c, eta and head weight, so their outputs stay exactly 0.
 // ------------------------------------------------------------------------------------------
-template <typename E>
-__global__ void __launch_bounds__(256) soa_cell_kernel(const float* __restrict__ eta, const float* __restrict__ u,
-                                                       long long u_bstride, const float* __restrict__ du,
-                                                       long long du_bstride, const float* __restrict__ head_w,
-                                                       const E* __restrict__ gates, const float* __restrict__ traw,
-                                                       const float* __restrict__ c_prev, const float* __restrict__ c_cur,
-                                                       const float* __restrict__ dc_prev, const float* __restrict__ dc_cur,
-                                                       float* __restrict__ kappa, E* __restrict__ da_out, long long npix,
-                                                       long long HW, int hc) {
+// DHW: the head weight has a tangent too (parameter direction): deta also gains u dhead_w
+template <typename E, bool DHW>
+__device__ __forceinline__ void soa_cell_body(const float* __restrict__ eta, const float* __restrict__ u,
+                                              long long u_bstride, const float* __restrict__ du, long long du_bstride,
+                                              const float* __restrict__ head_w, const E* __restrict__ gates,
+                                              const float* __restrict__ traw, const float* __restrict__ c_prev,
+                                              const float* __restrict__ c_cur, const float* __restrict__ dc_prev,
+                                              const float* __restrict__ dc_cur, float* __restrict__ kappa,
+                                              E* __restrict__ da_out, long long npix, long long HW, int hc,
+                                              const float* __restrict__ dhead_w) {
   constexpr bool FAST = std::is_same<E, __nv_bfloat16>::value;
   const int groups = hc / 8;
   const long long total = npix * groups;
@@ -426,7 +466,7 @@ __global__ void __launch_bounds__(256) soa_cell_kernel(const float* __restrict__
     const int q0 = (c0 >> 4) * 64 + (c0 & 8);
     const long long gi = pix * 4 * hc + q0;
     const long long ci = pix * hc + c0;
-    float a[4][8], g[4][8], cp[8], cc[8], dcp[8], dcc[8], e[8], de[8], k[8], dk[8], w[8];
+    float a[4][8], g[4][8], cp[8], cc[8], dcp[8], dcc[8], e[8], de[8], k[8], dk[8], w[8], dw[8];
     float uv = 0.f, duv = 0.f;
 #pragma unroll
     for (int q = 0; q < 4; ++q) load_elems<float, 8>(traw + gi + q * 16, a[q]);
@@ -450,9 +490,10 @@ __global__ void __launch_bounds__(256) soa_cell_kernel(const float* __restrict__
       if (u) uv = __ldg(u + b * u_bstride + r);
       if (du) duv = __ldg(du + b * du_bstride + r);
       load_elems<float, 8>(head_w + c0, w);
+      if constexpr (DHW) load_elems<float, 8>(dhead_w + c0, dw);
     } else {
 #pragma unroll
-      for (int j = 0; j < 8; ++j) w[j] = 0.f;
+      for (int j = 0; j < 8; ++j) w[j] = dw[j] = 0.f;
     }
     float o0[4][8], o1[4][8];
 #pragma unroll
@@ -463,7 +504,9 @@ __global__ void __launch_bounds__(256) soa_cell_kernel(const float* __restrict__
       const float tau = act_tanh<FAST>(cc[j]);
       const float tt = fmaf(-tau, tau, 1.f);
       const float dtau = tt * dcc[j];
-      const float et = fmaf(uv, w[j], e[j]), det = fmaf(duv, w[j], de[j]);
+      const float et = fmaf(uv, w[j], e[j]);
+      float det = fmaf(duv, w[j], de[j]);
+      if constexpr (DHW) det = fmaf(uv, dw[j], det);
       const float kt = fmaf(et * o_, tt, k[j]);
       const float dkt = fmaf(det * o_, tt, fmaf(et * d_o, tt, fmaf(-2.f * et * o_, tau * dtau, dk[j])));
       o0[0][j] = kt * g_ * si;
@@ -493,23 +536,66 @@ __global__ void __launch_bounds__(256) soa_cell_kernel(const float* __restrict__
   }
 }
 
+template <typename E>
+__global__ void __launch_bounds__(256) soa_cell_kernel(const float* __restrict__ eta, const float* __restrict__ u,
+                                                       long long u_bstride, const float* __restrict__ du,
+                                                       long long du_bstride, const float* __restrict__ head_w,
+                                                       const E* __restrict__ gates, const float* __restrict__ traw,
+                                                       const float* __restrict__ c_prev, const float* __restrict__ c_cur,
+                                                       const float* __restrict__ dc_prev, const float* __restrict__ dc_cur,
+                                                       float* __restrict__ kappa, E* __restrict__ da_out, long long npix,
+                                                       long long HW, int hc) {
+  soa_cell_body<E, false>(eta, u, u_bstride, du, du_bstride, head_w, gates, traw, c_prev, c_cur, dc_prev, dc_cur, kappa,
+                          da_out, npix, HW, hc, nullptr);
+}
+
+// the same with the head weight's tangent of a parameter direction
+template <typename E>
+__global__ void __launch_bounds__(256) soa_cell_dhead_kernel(const float* __restrict__ eta, const float* __restrict__ u,
+                                                             long long u_bstride, const float* __restrict__ du,
+                                                             long long du_bstride, const float* __restrict__ head_w,
+                                                             const E* __restrict__ gates, const float* __restrict__ traw,
+                                                             const float* __restrict__ c_prev,
+                                                             const float* __restrict__ c_cur,
+                                                             const float* __restrict__ dc_prev,
+                                                             const float* __restrict__ dc_cur, float* __restrict__ kappa,
+                                                             E* __restrict__ da_out, long long npix, long long HW, int hc,
+                                                             const float* __restrict__ dhead_w) {
+  soa_cell_body<E, true>(eta, u, u_bstride, du, du_bstride, head_w, gates, traw, c_prev, c_cur, dc_prev, dc_cur, kappa,
+                         da_out, npix, HW, hc, dhead_w);
+}
+
+template <typename E>
+static void launch_soa_cell_e(long long blocks, const float* eta, const float* u, long long u_bstride, const float* du,
+                              long long du_bstride, const float* head_w, const void* gates, const float* traw,
+                              const float* c_prev, const float* c_cur, const float* dc_prev, const float* dc_cur,
+                              float* kappa, void* da_out, long long npix, long long HW, int hc, cudaStream_t s,
+                              const float* dhead_w) {
+  const E* g = reinterpret_cast<const E*>(gates);
+  E* da = reinterpret_cast<E*>(da_out);
+  if (dhead_w)
+    soa_cell_dhead_kernel<E><<<blocks, 256, 0, s>>>(eta, u, u_bstride, du, du_bstride, head_w, g, traw, c_prev, c_cur,
+                                                    dc_prev, dc_cur, kappa, da, npix, HW, hc, dhead_w);
+  else
+    soa_cell_kernel<E><<<blocks, 256, 0, s>>>(eta, u, u_bstride, du, du_bstride, head_w, g, traw, c_prev, c_cur, dc_prev,
+                                              dc_cur, kappa, da, npix, HW, hc);
+}
+
 cudaError_t launch_soa_cell(int dtype, const float* eta, const float* u, long long u_bstride, const float* du,
                             long long du_bstride, const float* head_w, const void* gates, const float* traw,
                             const float* c_prev, const float* c_cur, const float* dc_prev, const float* dc_cur,
-                            float* kappa, void* da_out, long long npix, long long HW, int hc, cudaStream_t s) {
+                            float* kappa, void* da_out, long long npix, long long HW, int hc, cudaStream_t s,
+                            const float* dhead_w) {
   const long long total = npix * (hc / 8);
   long long blocks = (total + 255) / 256;
   if (blocks > 148 * 16) blocks = 148 * 16;
   if (blocks <= 0) return cudaSuccess;
   if (dtype == NINT_BF16)
-    soa_cell_kernel<__nv_bfloat16><<<blocks, 256, 0, s>>>(eta, u, u_bstride, du, du_bstride, head_w,
-                                                           reinterpret_cast<const __nv_bfloat16*>(gates), traw, c_prev,
-                                                           c_cur, dc_prev, dc_cur, kappa,
-                                                           reinterpret_cast<__nv_bfloat16*>(da_out), npix, HW, hc);
+    launch_soa_cell_e<__nv_bfloat16>(blocks, eta, u, u_bstride, du, du_bstride, head_w, gates, traw, c_prev, c_cur, dc_prev,
+                                     dc_cur, kappa, da_out, npix, HW, hc, s, dhead_w);
   else
-    soa_cell_kernel<float><<<blocks, 256, 0, s>>>(eta, u, u_bstride, du, du_bstride, head_w,
-                                                  reinterpret_cast<const float*>(gates), traw, c_prev, c_cur, dc_prev,
-                                                  dc_cur, kappa, reinterpret_cast<float*>(da_out), npix, HW, hc);
+    launch_soa_cell_e<float>(blocks, eta, u, u_bstride, du, du_bstride, head_w, gates, traw, c_prev, c_cur, dc_prev,
+                             dc_cur, kappa, da_out, npix, HW, hc, s, dhead_w);
   return cudaGetLastError();
 }
 
@@ -660,6 +746,56 @@ cudaError_t launch_head_fwd(int dtype, const void* h, const float* w, const floa
   else
     head_fwd_kernel<float><<<blocks, 256, hc_pad * 4, s>>>(reinterpret_cast<const float*>(h), w, b, out, npix, B, hc,
                                                           hc_pad, out_bstride);
+  return cudaGetLastError();
+}
+
+// Head tangent with a parameter direction: out = db + sum_c dh[pix][c] w[c] + h[pix][c] dw[c].  Same thread layout as
+// head_fwd_kernel, reading the primal and the tangent h of a pixel in the same pass.
+template <typename E>
+__global__ void head_tangent_kernel(const E* __restrict__ h, const E* __restrict__ dh, const float* __restrict__ w,
+                                    const float* __restrict__ dw, const float* __restrict__ db, float* __restrict__ out,
+                                    long long npix, int B, int hc, int hc_pad, long long out_bstride) {
+  extern __shared__ float s_w[];   // [hc_pad] w, then [hc_pad] dw
+  for (int i = threadIdx.x; i < hc_pad; i += blockDim.x) {
+    s_w[i] = i < hc ? w[i] : 0.f;
+    s_w[hc_pad + i] = i < hc ? dw[i] : 0.f;
+  }
+  __syncthreads();
+  constexpr int V = 16 / sizeof(E);
+  const long long total = static_cast<long long>(B) * npix;
+  const float b0 = db[0];
+  for (long long gp = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; gp < total;
+       gp += static_cast<long long>(gridDim.x) * blockDim.x) {
+    const E* hp = h + gp * hc_pad;
+    const E* dp = dh + gp * hc_pad;
+    float acc = b0;
+    for (int c0 = 0; c0 < hc_pad; c0 += V) {
+      float f[V], d[V];
+      load_elems<E, V>(dp + c0, d);
+      load_elems<E, V>(hp + c0, f);
+#pragma unroll
+      for (int j = 0; j < V; ++j) acc = fmaf(f[j], s_w[hc_pad + c0 + j], fmaf(d[j], s_w[c0 + j], acc));
+    }
+    const long long b = gp / npix;
+    out[b * out_bstride + (gp - b * npix)] = acc;
+  }
+}
+
+cudaError_t launch_head_tangent(int dtype, const void* h, const void* dh, const float* w, const float* dw, const float* db,
+                                float* out, long long npix, int B, int hc, int hc_pad, long long out_bstride,
+                                cudaStream_t s) {
+  const long long total = static_cast<long long>(B) * npix;
+  long long blocks = (total + 255) / 256;
+  if (blocks > 148 * 8) blocks = 148 * 8;
+  if (blocks <= 0) return cudaSuccess;
+  if (dtype == NINT_BF16)
+    head_tangent_kernel<__nv_bfloat16><<<blocks, 256, 2 * hc_pad * 4, s>>>(
+        reinterpret_cast<const __nv_bfloat16*>(h), reinterpret_cast<const __nv_bfloat16*>(dh), w, dw, db, out, npix, B, hc,
+        hc_pad, out_bstride);
+  else
+    head_tangent_kernel<float><<<blocks, 256, 2 * hc_pad * 4, s>>>(reinterpret_cast<const float*>(h),
+                                                                  reinterpret_cast<const float*>(dh), w, dw, db, out,
+                                                                  npix, B, hc, hc_pad, out_bstride);
   return cudaGetLastError();
 }
 

@@ -22,7 +22,8 @@ class Plan:
     def __init__(self, batch: int, seq_len: int, height: int, width: int, in_channels: int,
                  hidden: Sequence[int], ksize: Sequence[int], precision: str = "bf16", training: bool = False,
                  return_sequence: bool = False, device=None, deterministic: bool = False, input_grad: bool = False,
-                 state_grad: bool = False, tangent: bool = False, second_order: bool = False):
+                 state_grad: bool = False, tangent: bool = False, second_order: bool = False,
+                 param_tangent: bool = False):
         if precision not in PRECISIONS:
             raise ValueError(f"precision must be one of {sorted(PRECISIONS)}")
         if len(hidden) != len(ksize):
@@ -37,8 +38,9 @@ class Plan:
         self.hidden, self.ksize, self.L = list(hidden), list(ksize), len(hidden)
         self.training, self.return_sequence, self.precision = bool(training), bool(return_sequence), precision
         self.deterministic, self.input_grad, self.state_grad = bool(deterministic), bool(input_grad), bool(state_grad)
-        self.second_order = bool(second_order)
-        self.tangent = bool(tangent) or self.second_order     # the second-order pass reads the tangent pass's history
+        self.second_order, self.param_tangent = bool(second_order), bool(param_tangent)
+        # the second-order pass reads the tangent pass's history; a parameter direction rides in the tangent pass
+        self.tangent = bool(tangent) or self.second_order or self.param_tangent
         cfg = _lib.NintConfig()
         cfg.batch, cfg.seq_len, cfg.height, cfg.width = batch, seq_len, height, width
         cfg.in_channels, cfg.num_layers = in_channels, self.L
@@ -47,7 +49,7 @@ class Plan:
         cfg.dtype, cfg.training, cfg.return_sequence = PRECISIONS[precision], int(training), int(return_sequence)
         cfg.flags = ((_lib.FLAG_DETERMINISTIC if deterministic else 0) | (_lib.FLAG_INPUT_GRAD if input_grad else 0) |
                      (_lib.FLAG_STATE_GRAD if state_grad else 0) | (_lib.FLAG_TANGENT if tangent else 0) |
-                     (_lib.FLAG_SECOND_ORDER if second_order else 0))
+                     (_lib.FLAG_SECOND_ORDER if second_order else 0) | (_lib.FLAG_PARAM_TANGENT if param_tangent else 0))
         self._h = ctypes.c_void_p()
         _lib.check(self.lib.nint_plan_create(ctypes.byref(cfg), ctypes.byref(self._h)), "nint_plan_create")
         self.workspace_bytes = self.lib.nint_plan_workspace_bytes(self._h)
@@ -344,9 +346,55 @@ class Plan:
         dc_T = [new(l) for l in range(self.L)]
         return dh0, dc0, dpred, dseq, dh_T, dc_T
 
+    def set_param_tangent(self, layers=None, head=None):
+        """Makes dtheta the parameter direction of the following forward_tangent[_bank] calls (plans made with
+        param_tangent=True): layers = per layer (dW [4Hc, Cin+Hc, k, k], db [4Hc] or None) or None, head = (dw
+        [1,Hc_last,1,1], db [1] or None) or None, shapes as set_weights / set_head; a missing entry is zero.  Replaces the
+        whole previous direction.  One forward serves many directions:
+
+            plan.forward(x)
+            for layers, head in directions:
+                plan.set_param_tangent(layers, head)
+                dpred, dseq, dstate = plan.forward_tangent(dx, dh0, dc0)    # J (dx, dh0, dc0, dtheta)
+            plan.clear_param_tangent()
+            plan.backward(dpred_seed)                                       # one ordinary backward at the end
+        """
+        self.clear_param_tangent()
+        if layers is not None and len(layers) != self.L:
+            raise ValueError(f"layers has {len(layers)} entries, expected {self.L}")
+        checked = []
+        cin = self.C
+        for l, entry in enumerate(layers or [None] * self.L):
+            hc, k = self.hidden[l], self.ksize[l]
+            if entry is not None:
+                dw, db = entry
+                self._check_dev(dw, f"weight tangent [{l}]", (4 * hc, cin + hc, k, k))
+                if db is not None:
+                    self._check_dev(db, f"bias tangent [{l}]", (4 * hc,))
+                checked.append((l, dw.detach().contiguous(), None if db is None else db.detach().contiguous()))
+            cin = hc
+        if head is not None:
+            hw, hb = head
+            self._check_dev(hw, "head weight tangent", (1, self.hidden[-1], 1, 1))
+            if hb is not None:
+                self._check_dev(hb, "head bias tangent", (1,))
+            head = (hw.detach().contiguous(), None if hb is None else hb.detach().contiguous())
+        with _lib.on_device(self.device):
+            for l, dw, db in checked:
+                _lib.check(self.lib.nint_plan_set_weight_tangent(self._h, l, _ptr(dw), _ptr(db), self._stream()),
+                           "nint_plan_set_weight_tangent")
+            if head is not None:
+                _lib.check(self.lib.nint_plan_set_head_tangent(self._h, _ptr(head[0]), _ptr(head[1]), self._stream()),
+                           "nint_plan_set_head_tangent")
+
+    def clear_param_tangent(self):
+        """Zero parameter direction: forward_tangent is J (dx, dh0, dc0) at fixed parameters again."""
+        with _lib.on_device(self.device):
+            _lib.check(self.lib.nint_plan_clear_param_tangent(self._h, self._stream()), "nint_plan_clear_param_tangent")
+
     def forward_tangent(self, dx: Optional[torch.Tensor] = None, dh0=None, dc0=None):
-        """J v of the last `forward` for v = (dx [B,T,C,H,W], per-layer dh0 / dc0 [B,Hc_l,H,W]; None = zero) at fixed
-        parameters: returns (dpred [B,1,H,W], dseq [B,T,H,W] or None, [(dh_T, dc_T) per layer]).  The forward's saved
+        """J v of the last `forward` for v = (dx [B,T,C,H,W], per-layer dh0 / dc0 [B,Hc_l,H,W]; None = zero), plus the
+        parameter direction set by set_param_tangent (param_tangent plans; else at fixed parameters): returns (dpred [B,1,H,W], dseq [B,T,H,W] or None, [(dh_T, dc_T) per layer]).  The forward's saved
         activations are only read: more tangents, and then one `backward`, of the same forward may follow."""
         if dx is not None:
             self._check_dev(dx, "dx", (self.B, self.T, self.C, self.H, self.W), dtypes=(torch.float32, torch.bfloat16))
@@ -433,6 +481,38 @@ class Plan:
             if not t.is_contiguous():
                 raise ValueError(f"{name} must be contiguous")
         return self._second_order(self.lib.nint_backward_second_order_bank, u, du, (dframes, ddframes), state)
+
+    def backward_second_order_params(self, grad: bool = True):
+        """Parameter outputs of the last backward_second_order[_bank] (plans made with second_order=True and
+        param_tangent=True): (grads, hvps), each a list in ConvLSTM._params() order -- per layer weight, bias, then the
+        head's weight and bias -- with grads = dL/dtheta (None when grad=False: its wgrad launches are skipped) and hvps =
+        the theta block of H v for the joint direction (dx, dh0, dc0, dtheta) of the tangent pass the second-order pass
+        followed.  One forward serves many directions:
+
+            plan.forward(x)
+            for direction in directions:
+                plan.set_param_tangent(*model.param_direction(direction))
+                dpred, dseq, _ = plan.forward_tangent()
+                u, du = ...                                   # loss gradient and its tangent on (dpred, dseq)
+                plan.backward_second_order(u, du)
+                _, hv = plan.backward_second_order_params(grad=False)
+            plan.backward(dpred_seed)                         # one ordinary backward at the end
+        """
+        new = lambda s: torch.empty(s, dtype=torch.float32, device=self.device)
+        shapes, cin = [], self.C
+        for hc, k in zip(self.hidden, self.ksize):
+            shapes += [(4 * hc, cin + hc, k, k), (4 * hc,)]
+            cin = hc
+        shapes += [(1, self.hidden[-1], 1, 1), (1,)]
+        g = [new(s) for s in shapes] if grad else None
+        h = [new(s) for s in shapes]
+        table = lambda ts, j: None if ts is None else (ctypes.c_void_p * self.L)(*[ts[2 * l + j].data_ptr()
+                                                                                 for l in range(self.L)])
+        with _lib.on_device(self.device):
+            _lib.check(self.lib.nint_backward_second_order_params(
+                self._h, table(g, 0), table(g, 1), table(h, 0), table(h, 1), _ptr(g[-2] if g else None),
+                _ptr(g[-1] if g else None), _ptr(h[-2]), _ptr(h[-1]), self._stream()), "nint_backward_second_order_params")
+        return g, h
 
     # ---- ConvLSTMCell as a differentiable unit (plans with T = 1, L = 1)
     def cell_forward(self, x, h, c):

@@ -166,19 +166,20 @@ class ConvLSTM(nn.Module):
         return ps + [self.conv.weight, self.conv.bias]
 
     def plan_for_shape(self, B, T, H, W, device, training, set_params=True, input_grad=False, state_grad=False,
-                       tangent=False, second_order=False):
+                       tangent=False, second_order=False, param_tangent=False):
         device = torch.device(device)
         if device.index is None:
             device = torch.device("cuda", torch.cuda.current_device())
         det = bool(training) and _deterministic_default()
         key = (B, T, H, W, bool(training), self.return_sequence, self.precision, device, bool(input_grad),
-               bool(state_grad), det, bool(tangent), bool(second_order))
+               bool(state_grad), det, bool(tangent), bool(second_order), bool(param_tangent))
         hidden = [c.hidden_channels for c in self.layers]
         ks = [c.kernel_size for c in self.layers]
         plan = self._plans.get(key, lambda: Plan(B, T, H, W, self.input_channels, hidden, ks, precision=self.precision,
                                                  training=training, return_sequence=self.return_sequence,
                                                  device=device, deterministic=det, input_grad=input_grad,
-                                                 state_grad=state_grad, tangent=tangent, second_order=second_order))
+                                                 state_grad=state_grad, tangent=tangent, second_order=second_order,
+                                                 param_tangent=param_tangent))
         if set_params:
             for l, cell in enumerate(self.layers):
                 plan.set_weights(l, cell.conv.weight, cell.conv.bias)
@@ -186,12 +187,12 @@ class ConvLSTM(nn.Module):
         return plan
 
     def plan_for(self, x, training, set_params=True, input_grad=False, state_grad=False, tangent=False,
-                 second_order=False):
+                 second_order=False, param_tangent=False):
         B, T, C, H, W = x.size()
         if C != self.input_channels:
             raise ValueError(f"expected {self.input_channels} input channels, got {C}")
         return self.plan_for_shape(B, T, H, W, x.device, training, set_params, input_grad, state_grad, tangent,
-                                   second_order)
+                                   second_order, param_tangent)
 
     def _wants_grad(self, params):
         return torch.is_grad_enabled() and any(p.requires_grad for p in params)
@@ -267,36 +268,77 @@ class ConvLSTM(nn.Module):
             return None, None
         return [h for h, _ in state_tangent], [c for _, c in state_tangent]
 
-    def jvp(self, x, dx, hidden_state=None, state_tangent=None, return_state=False):
+    def param_direction(self, direction):
+        """A parameter direction as a dict keyed by named_parameters() names (`layers.{l}.conv.weight|bias`,
+        `conv.weight|bias`; the format of torch.func.functional_call) -> (layers, head) for Plan.set_param_tangent.
+        Missing keys are zero; unknown keys and shapes other than the parameter's raise."""
+        params = dict(self.named_parameters())
+        unknown = sorted(set(direction) - set(params))
+        if unknown:
+            raise KeyError(f"parameter direction has unknown keys {unknown}; expected names from named_parameters()")
+        for name, t in direction.items():
+            if tuple(t.shape) != tuple(params[name].shape):
+                raise ValueError(f"direction[{name!r}] has shape {tuple(t.shape)}, expected {tuple(params[name].shape)}")
+
+        def pair(w_name, b_name):
+            dw, db = direction.get(w_name), direction.get(b_name)
+            if dw is None and db is None:
+                return None
+            return (torch.zeros_like(params[w_name]) if dw is None else dw, db)
+
+        layers = [pair(f"layers.{l}.conv.weight", f"layers.{l}.conv.bias") for l in range(self.num_layers)]
+        return (None if all(e is None for e in layers) else layers), pair("conv.weight", "conv.bias")
+
+    def _tangent_plan(self, plan, param_tangent):
+        if param_tangent is not None:
+            plan.set_param_tangent(*self.param_direction(param_tangent))
+
+    def jvp(self, x, dx, hidden_state=None, state_tangent=None, return_state=False, param_tangent=None):
         """Forward-mode derivative at fixed parameters, the tangent-linear model of `forward`: returns (out, dout) with
         `out` what forward(x, hidden_state) returns and `dout` its derivative in the direction (dx, state_tangent), like
         torch.func.jvp's (primals_out, tangents_out).  dx [B,T,C,H,W] (None: zero); state_tangent: per layer (dh0, dc0)
         [B,Hc_l,H,W] fp32 (None: zero, for all layers or one tensor).  return_state: ((out, [(h_T, c_T)]),
         (dout, [(dh_T, dc_T)])).  A tangent pass costs about two to three forwards (DESIGN.md section 10, f7).  A
         direction is exact up to the rounding of the tangent operands (bf16 / tf32 like h), not a difference of two
-        nonlinear runs.  The outputs carry no autograd graph."""
+        nonlinear runs.  The outputs carry no autograd graph.
+        param_tangent: a direction in parameter space as well, a dict keyed by named_parameters() names (missing keys:
+        zero; see param_direction), so dout = J_x dx + J_state dstate + J_theta dtheta and the result compares directly
+        with torch.func.jvp(lambda p: functional_call(model, p, x), (params,), (param_tangent,)).  It costs one more
+        gate GEMM per step and layer that has a direction.  For many directions on one forward (a Laplace or Lanczos
+        loop) use the plan: Plan.set_param_tangent.  A call with param_tangent uses its own cached plan (the flag's
+        buffers); alternating calls with and without it at one shape keep both plans' workspaces."""
         if not x.is_cuda:
             raise RuntimeError("ConvLSTM runs on CUDA (B200) only: there is no CPU fallback")
-        plan = self.plan_for(x, True, tangent=True)
+        if param_tangent is None:
+            plan = self.plan_for(x, True, tangent=True)
+        else:
+            plan = self.plan_for(x, True, param_tangent=True)
         dh0, dc0 = self._tangent_state(plan, state_tangent)
         with torch.no_grad():
             pred, seq = plan.forward(x, hidden_state)
             final = plan.final_state() if return_state else None
+            self._tangent_plan(plan, param_tangent)
             dpred, dseq, dfinal = plan.forward_tangent(dx, dh0, dc0)
         return self._jvp_result(pred, seq, final, dpred, dseq, dfinal, return_state)
 
-    def jvp_windows(self, bank, win_start, seq_len, dbank, hidden_state=None, state_tangent=None, return_state=False):
+    def jvp_windows(self, bank, win_start, seq_len, dbank, hidden_state=None, state_tangent=None, return_state=False,
+                    param_tangent=None):
         """`jvp` over frame-bank windows (forward_windows): dbank [N,Hp,Wp,c_pad] holds the tangent of every frame of
-        `bank` in its layout (FrameBank.tangent / FrameBank.tangent_from_fields), cut at the same window starts."""
+        `bank` in its layout (FrameBank.tangent / FrameBank.tangent_from_fields), cut at the same window starts.
+        param_tangent: as in `jvp`."""
         starts = win_start.to(device=bank.frames.device, dtype=torch.int32).contiguous()
         bank.check_windows(win_start, seq_len)
         N, H, W, _ = bank.frames.shape
-        plan = self.plan_for_shape(starts.shape[0], int(seq_len), H, W, bank.frames.device, True, tangent=True)
+        if param_tangent is None:
+            plan = self.plan_for_shape(starts.shape[0], int(seq_len), H, W, bank.frames.device, True, tangent=True)
+        else:
+            plan = self.plan_for_shape(starts.shape[0], int(seq_len), H, W, bank.frames.device, True, param_tangent=True)
         bank.check_plan(plan)
         dh0, dc0 = self._tangent_state(plan, state_tangent)
         with torch.no_grad():
             pred, seq = plan.forward_bank(bank.frames, starts, hidden_state)
             final = plan.final_state() if return_state else None
+            self._tangent_plan(plan, param_tangent)
             dpred, dseq, dfinal = plan.forward_tangent_bank(dbank, dh0, dc0)
         return self._jvp_result(pred, seq, final, dpred, dseq, dfinal, return_state)
 
@@ -308,7 +350,15 @@ class ConvLSTM(nn.Module):
         (u, loss), (du, _) = torch.func.jvp(torch.func.grad_and_value(loss_fn), (out,), (dout,))
         return loss.detach(), u, du
 
-    def hvp(self, x, dx, loss_fn, hidden_state=None, state_tangent=None):
+    def _param_results(self, plan, param_direction, wrt_params):
+        """({name: grad}, {name: hvp}) of the last second-order pass when wrt_params"""
+        if not wrt_params:
+            return None
+        g, h = plan.backward_second_order_params()
+        names = [n for n, _ in self.named_parameters()]
+        return dict(zip(names, g)), dict(zip(names, h))
+
+    def hvp(self, x, dx, loss_fn, hidden_state=None, state_tangent=None, param_direction=None, wrt_params=False):
         """Second-order adjoint at fixed parameters: returns (loss, grad, hvp) with loss = loss_fn(forward(x,
         hidden_state)), grad its gradient and hvp = H v its Hessian-vector product w.r.t. (x, initial state) in the
         direction v = (dx, state_tangent), the exact Hessian including the curvature of the recurrence (not the
@@ -318,36 +368,57 @@ class ConvLSTM(nn.Module):
         Cost: a forward, a tangent pass and a second-order pass (DESIGN.md section 10, f8).  For many directions on one
         forward (Newton-CG, Lanczos) use the plan directly: plan = model.plan_for(x, True, second_order=True),
         plan.forward(x), then per direction plan.forward_tangent(...) and plan.backward_second_order(u, du), with u, du
-        from the outputs as here; the forward's activations stay intact for one ordinary backward at the end."""
+        from the outputs as here; the forward's activations stay intact for one ordinary backward at the end.
+        param_direction: a direction in parameter space as well (a dict keyed by named_parameters() names, missing keys
+        zero; see param_direction), so v = (dx, state_tangent, param_direction) is a joint direction and every mixed
+        block of the Hessian enters.  wrt_params=True: grad and hvp are (x part, state part, {name: tensor}) with the
+        parameter block as the third entry -- the exact H_theta.v of Lanczos, sharpness, Newton-CG and influence
+        functions (Plan.backward_second_order_params for many directions on one forward).  Both use a plan with
+        param_tangent=True, which keeps the tangent dh and the pass's dgates of every step (DESIGN.md section 10, f9)."""
         if not x.is_cuda:
             raise RuntimeError("ConvLSTM runs on CUDA (B200) only: there is no CPU fallback")
-        plan = self.plan_for(x, True, second_order=True)
+        with_params = param_direction is not None or wrt_params
+        plan = self.plan_for(x, True, second_order=True, param_tangent=with_params)
         dh0, dc0 = self._tangent_state(plan, state_tangent)
         with torch.no_grad():
             pred, seq = plan.forward(x, hidden_state)
+            if with_params:
+                plan.set_param_tangent(*self.param_direction(param_direction or {}))
             dpred, dseq, _ = plan.forward_tangent(dx, dh0, dc0)
         loss, u, du = self._loss_seeds(loss_fn, pred, seq, dpred, dseq)
         state = plan.check_state(hidden_state)
         gx, hx, gs, hs = plan.backward_second_order(u, du, state=state)
+        pr = self._param_results(plan, param_direction, wrt_params)
+        if pr is not None:
+            return loss, (gx, gs, pr[0]), (hx, hs, pr[1])
         return loss, (gx, gs), (hx, hs)
 
-    def hvp_windows(self, bank, win_start, seq_len, dbank, loss_fn, hidden_state=None, state_tangent=None):
+    def hvp_windows(self, bank, win_start, seq_len, dbank, loss_fn, hidden_state=None, state_tangent=None,
+                    param_direction=None, wrt_params=False):
         """`hvp` over frame-bank windows (forward_windows / jvp_windows): the direction of the frames is dbank
         [N,Hp,Wp,c_pad] (FrameBank.tangent / tangent_from_fields).  grad and hvp are (d/dframes [N,C,Hp,Wp] fp32, state
-        pairs or None): every window's contribution is summed into the frames it read.  bank.grad is not touched."""
+        pairs or None): every window's contribution is summed into the frames it read.  bank.grad is not touched.
+        param_direction / wrt_params: as in `hvp`."""
         starts = win_start.to(device=bank.frames.device, dtype=torch.int32).contiguous()
         bank.check_windows(win_start, seq_len)
         N, H, W, _ = bank.frames.shape
-        plan = self.plan_for_shape(starts.shape[0], int(seq_len), H, W, bank.frames.device, True, second_order=True)
+        with_params = param_direction is not None or wrt_params
+        plan = self.plan_for_shape(starts.shape[0], int(seq_len), H, W, bank.frames.device, True, second_order=True,
+                                   param_tangent=with_params)
         bank.check_plan(plan)
         dh0, dc0 = self._tangent_state(plan, state_tangent)
         with torch.no_grad():
             pred, seq = plan.forward_bank(bank.frames, starts, hidden_state)
+            if with_params:
+                plan.set_param_tangent(*self.param_direction(param_direction or {}))
             dpred, dseq, _ = plan.forward_tangent_bank(dbank, dh0, dc0)
         loss, u, du = self._loss_seeds(loss_fn, pred, seq, dpred, dseq)
         new = lambda: torch.zeros((N, bank.channels, H, W), dtype=torch.float32, device=bank.frames.device)
         gf, hf = new(), new()
         gs, hs = plan.backward_second_order_bank(u, du, gf, hf, state=plan.check_state(hidden_state))
+        pr = self._param_results(plan, param_direction, wrt_params)
+        if pr is not None:
+            return loss, (gf, gs, pr[0]), (hf, hs, pr[1])
         return loss, (gf, gs), (hf, hs)
 
     def release_workspaces(self):
