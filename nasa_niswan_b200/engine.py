@@ -60,6 +60,7 @@ class Plan:
         self.generation = 0          # bumped by every forward and every backward: BPTT consumes the saved activations
         self._weight_keys = [None] * (self.L + 1)
         self._keep = None            # tensors the queued kernels still read (frame bank, window indices)
+        self._tkeep = None           # the tangent frames of the last forward_tangent_bank (the params call reads them)
         self._stateful = False       # the last forward was given an initial state (it stays in the workspace)
 
     def __del__(self):
@@ -192,7 +193,7 @@ class Plan:
             raise TypeError("bf16 inputs need precision='bf16' (a tf32 plan would lose input precision)")
         x = x.detach().contiguous()
         self._initial_state(state)
-        self._keep = None                   # no frame bank behind this forward
+        self._keep = self._tkeep = None     # no frame bank behind this forward
         pred, seq = self._outputs()
         with _lib.on_device(self.device):
             _lib.check(self.lib.nint_forward_ex(self._h, _ptr(x), _lib.X_BF16 if x.dtype == torch.bfloat16 else _lib.X_FP32,
@@ -217,6 +218,7 @@ class Plan:
             _lib.check(self.lib.nint_forward_bank(self._h, _ptr(frames), frames.shape[0], _ptr(win_start), _ptr(pred),
                                                   _ptr(seq), self._stream()), "nint_forward_bank")
         self._keep = (frames, win_start)    # the backward kernels read both again
+        self._tkeep = None
         self.generation += 1
         return pred, seq
 
@@ -413,7 +415,8 @@ class Plan:
     def forward_tangent_bank(self, dframes: torch.Tensor, dh0=None, dc0=None):
         """forward_tangent after `forward_bank`: dframes [N,H,W,c_pad] are the tangent frames in the bank's layout with
         the constant-1 lane 0 (FrameBank.tangent / tangent_from_fields), N the bank's; the windows are those of the
-        forward."""
+        forward.  The plan keeps a reference to dframes until the next forward: backward_second_order_params reads
+        them again."""
         if self._keep is None:
             raise RuntimeError("forward_tangent_bank: the last forward did not read a frame bank (forward_bank)")
         frames = self._keep[0]
@@ -428,6 +431,7 @@ class Plan:
                                                           self._ptr_table(dc0), _ptr(dpred), _ptr(dseq),
                                                           self._ptr_table(dh_T), self._ptr_table(dc_T), self._stream()),
                        "nint_forward_tangent_bank")
+        self._tkeep = dframes    # backward_second_order_params' wgrad reads them again through the plan's tensor maps
         return dpred, dseq, list(zip(dh_T, dc_T))
 
     # ---- second-order adjoint (plans made with training=True, second_order=True)
